@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the B-mode renderer hot path (BASELINE.json metric: frames/s and Gsamples/s, forward+backward).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--poses P]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--poses P] [--dump-outputs DIR]
 
 Workload (SURVEY.md 8d config 3, the batched pose sweep, with config 2's loss): P probe
 poses per GPU x 128 rays x 512 samples over one synthetic MRI-shaped 256^3 impedance
@@ -22,6 +22,9 @@ Besides the headline (weak scaling: 1024 poses PER GPU) the line carries, at eve
   `nccl_parity`  a small scene rendered rank-sharded: gathered frames and all-reduced weight gradients against the full
                  batch computed on rank 0 alone;
   `config5`      (N = 1) the 512^3 / 512 x 2048 stress case on >= 1024 poses spread over the sphere.
+Every timed loop of these records runs `--steps` steps.  `--dump-outputs DIR` writes what the last timed headline step
+returned (loss.npy, grad_sources.npy, grad_directions.npy; with N ranks, every rank's shard concatenated in rank order,
+one loss per rank); the scene and poses are seeded, so two builds given the same arguments can be compared output for output.
 `--impl reference` times the UNMODIFIED reference (oracle/_ref archive or /root/reference) on the host cores: all 128 rays of
 a pose at the first 128 samples, forward + backward, plus one full config-1 frame (forward).
 """
@@ -178,6 +181,37 @@ def timed_steps(fn, warmup, steps, barrier):
     return e0.elapsed_time(e1) / steps
 
 
+DUMP_BYTES = 60 * 1000 ** 2      # keeps a dump, .npy headers included, under 64 MB
+
+
+def dump_outputs(out_dir, outputs):
+    """Write the tensors a caller of the timed step receives as ``out_dir/<name>.npy`` (float32; float64 stays float64), so
+    that two builds can be compared output for output.  If they exceed DUMP_BYTES in all, every array keeps the same fixed, seeded
+    sample of rows along its first (pose) axis."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    for name, t in outputs.items():
+        t = t.detach()
+        arrays[name] = (t if t.dtype == torch.float64 else t.float()).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES and a.ndim > 0:
+            keep = max(1, a.shape[0] * DUMP_BYTES // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
+def gather_ranks(t, world):
+    """Every rank's tensor of the same shape, concatenated along dim 0 in rank order (a collective: all ranks call it)."""
+    if world == 1:
+        return t
+    import torch.distributed as dist
+    parts = [torch.empty_like(t) for _ in range(world)]
+    dist.all_gather(parts, t.contiguous())
+    return torch.cat(parts)
+
+
 def max_over_ranks(values, dev, world):
     import torch.distributed as dist
     t = torch.tensor(values, dtype=torch.float64, device=dev)
@@ -186,7 +220,7 @@ def max_over_ranks(values, dev, world):
     return t.tolist()
 
 
-def strong_scaling_record(dev, rank, world, barrier, layout):
+def strong_scaling_record(dev, rank, world, barrier, layout, steps):
     """BASELINE config 3 as worded: 1024 poses IN TOTAL, sharded over the ranks (each rank: its contiguous block)."""
     from diffus_b200 import PreparedVolume, ops, render_frames
     from diffus_b200 import distributed as D
@@ -203,11 +237,11 @@ def strong_scaling_record(dev, rank, world, barrier, layout):
 
     def eager():
         ops.render_mse_impl(pv.volume, pv.bricks, dims, src, dirs, target, N_SAMPLES, 0, ALPHA, SAMPLER_TRILINEAR, False, False, True, False)
-    ms_eager = timed_steps(eager, 5, 200, barrier)
+    ms_eager = timed_steps(eager, 5, steps, barrier)
     g = GraphedPoseStep(pv, target, N_RAYS, N_SAMPLES, ALPHA)
     g.sources.copy_(src)
     g.directions.copy_(dirs)
-    ms_graph = timed_steps(g.graph.replay, 5, 200, barrier)
+    ms_graph = timed_steps(g.graph.replay, 5, steps, barrier)
     ms_eager, ms_graph = max_over_ranks([ms_eager, ms_graph], dev, world)
     return {"what": "config 3 strong scaling: 1024 poses in total, contiguous pose blocks per rank, fused fwd+MSE+bwd step, no collective "
                     "on the path; max over ranks of the CUDA-event time",
@@ -215,7 +249,7 @@ def strong_scaling_record(dev, rank, world, barrier, layout):
             "frames_per_s_op_calls": total / (ms_eager * 1e-3), "frames_per_s_cuda_graph": total / (ms_graph * 1e-3)}
 
 
-def config4_record(dev, rank, world, barrier):
+def config4_record(dev, rank, world, barrier, steps):
     """BASELINE config 4: MLP over a T2-shaped 256^3 volume -> 4096 frames per step IN TOTAL (sharded) -> MSE ->
     weight gradients -> NCCL all-reduce -> Adam, everything inside the timed region (FusedTrainer.step)."""
     from diffus_b200 import ImpedanceEstimator, PreparedVolume, render_frames
@@ -255,10 +289,10 @@ def config4_record(dev, rank, world, barrier):
             last[0] = tr.step(s, d, tgt, N_SAMPLES, ALPHA, n_total=n_total)      # (a view of the trainer's persistent loss slot)
         step()
         loss_first = float(last[0])                      # read back before the next step overwrites the slot; untimed
-        ms = timed_steps(step, 3, 10, barrier)
+        ms = timed_steps(step, 3, steps, barrier)
         (ms,) = max_over_ranks([ms], dev, world)
         out[sampler] = {"ms_per_step": ms, "frames_per_s": total / (ms * 1e-3), "gsamples_per_s": n_total / (ms * 1e-3) / 1e9,
-                        "loss_first": loss_first, "loss_last": float(last[0]), "adam_steps": 14}
+                        "loss_first": loss_first, "loss_last": float(last[0]), "adam_steps": 1 + 3 + steps}
         del tr, tgt
     return out
 
@@ -313,7 +347,7 @@ def nccl_parity_record(dev, rank, world):
     return rec
 
 
-def config5_record(dev, poses, layout):
+def config5_record(dev, poses, layout, steps):
     """BASELINE config 5 on one GPU: 512^3 volume (512 MiB: four times the L2), 512 rays x 2048 samples, `poses` poses spread
     over the sphere, fused fwd + MSE + bwd (pose gradients).  BASELINE's 4096 poses are `4096 / poses` such launches."""
     from diffus_b200 import PreparedVolume, ops, render_frames
@@ -329,7 +363,7 @@ def config5_record(dev, poses, layout):
 
     def step():
         ops.render_mse_impl(pv.volume, pv.bricks, dims, s, d, tgt, S, 0, ALPHA, SAMPLER_TRILINEAR, False, False, True, False)
-    ms = timed_steps(step, 2, 5, torch.cuda.synchronize)
+    ms = timed_steps(step, 2, steps, torch.cuda.synchronize)
     samples = poses * R * S
     peak, _ = load_peaks()
     gs = samples / (ms * 1e-3) / 1e9
@@ -481,13 +515,18 @@ def run_ours(args):
     frames_per_s = world * P / (ms_per_step * 1e-3)
     e2e_frames_per_s = world * P / (e2e_ms_total / K * 1e-3)
     loss_value, loss_e2e = float(loss), (float(out_pin[-1]) if args.e2e == "fan" else float(out_loss))
+    if args.dump_outputs:
+        # the last timed step's tensors (render_mse_impl allocates fresh outputs on every call); every rank's shard
+        outs = {name: gather_ranks(t, world) for name, t in (("loss", loss), ("grad_sources", gs), ("grad_directions", gd))}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outs)
 
     # ---- the other records: every rank takes part (collectives inside), rank 0 reports; a failure never costs the headline ----
     del target, fstep, gstep
     extras = {}
     if not args.no_extras:
-        for name, fn in (("strong", lambda: strong_scaling_record(dev, rank, world, barrier, args.layout)),
-                         ("config4", lambda: config4_record(dev, rank, world, barrier)),
+        for name, fn in (("strong", lambda: strong_scaling_record(dev, rank, world, barrier, args.layout, K)),
+                         ("config4", lambda: config4_record(dev, rank, world, barrier, K)),
                          ("nccl_parity", lambda: nccl_parity_record(dev, rank, world))):
             try:
                 extras[name] = fn()
@@ -496,7 +535,7 @@ def run_ours(args):
             torch.cuda.empty_cache()
         if world == 1 and args.config5_poses > 0:
             try:
-                extras["config5"] = config5_record(dev, args.config5_poses, args.layout)
+                extras["config5"] = config5_record(dev, args.config5_poses, args.layout, K)
             except Exception as exc:                        # noqa: BLE001
                 extras["config5"] = {"error": f"{type(exc).__name__}: {exc}"}
             torch.cuda.empty_cache()
@@ -709,7 +748,13 @@ def main():
     ap.add_argument("--config5-poses", type=int, default=1024, help="poses of the 512^3 stress record (N = 1 only; 0 = skip)")
     ap.add_argument("--no-cpu-config1", action="store_true", help="reference arm: skip the full config-1 frame (~75 s on 8 cores)")
     ap.add_argument("--e2e", default="fan", choices=["fan", "graph", "eager"], help="public API used by the end-to-end loop")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and pose gradients of the last timed step (all ranks', in rank order) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:
