@@ -9,8 +9,9 @@ from .cone import generate_cone_directions
 from .impedance import ImpedanceEstimator
 from .ops import fan_directions
 from .renderer import (PreparedVolume, UltrasoundRenderer, compute_echo_traces, compute_gaussian_pulse, gaussian_pulse, custom_nearest_sampler, differentiable_splat,
-                       propagate_full_rays_batched, render_frames, render_mse_loss, rotate_around_apex)
+                       propagate_full_rays_batched, render_frames, render_gauss_newton, render_mse_loss, rotate_around_apex)
+from .pose_recovery import apply_fan_twist, apply_pose_twist, recover_poses
 
-__all__ = ["UltrasoundRenderer", "render_frames", "render_mse_loss", "PreparedVolume", "compute_echo_traces", "compute_gaussian_pulse", "gaussian_pulse",
+__all__ = ["UltrasoundRenderer", "render_frames", "render_mse_loss", "render_gauss_newton", "PreparedVolume", "compute_echo_traces", "compute_gaussian_pulse", "gaussian_pulse",
            "propagate_full_rays_batched", "custom_nearest_sampler", "differentiable_splat", "rotate_around_apex", "generate_cone_directions",
-           "fan_directions", "ImpedanceEstimator"]
+           "fan_directions", "ImpedanceEstimator", "apply_pose_twist", "apply_fan_twist", "recover_poses"]

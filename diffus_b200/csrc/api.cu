@@ -174,6 +174,28 @@ BwdWorkspace bwd_workspace(const DiffusRenderBwdArgs* b, void* base) {
 
 int32_t cuda_rc(cudaError_t e) { return e == cudaSuccess ? DIFFUS_OK : (int32_t)e; }
 
+// Gauss-Newton workspace: [fwd workspace | median tangent (P*6) | per-ray partials (P*R*32)]
+struct GnWorkspace {
+    FwdWorkspace fwd;
+    float* med_tan;
+    float* partial;
+    int64_t bytes;
+};
+GnWorkspace gn_workspace(const DiffusGaussNewtonArgs* g, void* base) {
+    GnWorkspace w{};
+    const DiffusRenderArgs* a = &g->fwd;
+    w.fwd = fwd_workspace(a, base);
+    int64_t off = w.fwd.bytes;
+    if (a->start > 0) {
+        w.med_tan = (float*)((char*)base + off);
+        off += align_up(a->n_poses * 24, 256);
+    }
+    w.partial = (float*)((char*)base + off);
+    off += align_up(a->n_poses * a->n_rays * 128, 256);
+    w.bytes = off;
+    return w;
+}
+
 }  // namespace
 
 extern "C" {
@@ -285,6 +307,36 @@ int32_t diffus_render_backward(const DiffusRenderBwdArgs* b, void* stream) {
         if (ce != cudaSuccess) return (int32_t)ce;
     }
     return DIFFUS_OK;
+}
+
+int64_t diffus_render_gauss_newton_workspace_bytes(const DiffusGaussNewtonArgs* g) {
+    if (!g) return 0;
+    return gn_workspace(g, nullptr).bytes;
+}
+
+int32_t diffus_render_gauss_newton(const DiffusGaussNewtonArgs* g, void* stream) {
+    if (!g) return DIFFUS_E_NULL;
+    const DiffusRenderArgs* a = &g->fwd;
+    int32_t e = check_render(a, false);
+    if (e) return e;
+    if (!g->target || !g->loss || !g->jtr || !g->jtj) return DIFFUS_E_NULL;
+    if (a->sampler != DIFFUS_SAMPLER_TRILINEAR || a->pose_dtype != DIFFUS_POSE_F32) return DIFFUS_E_UNSUPPORTED;
+    GnWorkspace w = gn_workspace(g, g->workspace);
+    if (!g->workspace || g->workspace_bytes < w.bytes) return DIFFUS_E_WORKSPACE;
+    cudaStream_t st = (cudaStream_t)stream;
+    RenderParams p = pack(a);
+    p.frame = nullptr;
+    p.seg_prefix = nullptr;
+    p.target = g->target;
+    cudaError_t ce;
+    if (a->start > 0) {
+        ce = launch_first_refl_median(p, a->sampler, a->volume.layout, 0, w.fwd.median, w.fwd.tie_count, st);
+        if (ce != cudaSuccess) return (int32_t)ce;
+        p.median = w.fwd.median;
+        ce = launch_gn_median_tangent(p, a->volume.layout, w.fwd.tie_count, w.med_tan, st);
+        if (ce != cudaSuccess) return (int32_t)ce;
+    }
+    return cuda_rc(launch_render_gn(p, a->volume.layout, w.med_tan, w.partial, g->loss, g->jtr, g->jtj, st));
 }
 
 int32_t diffus_ray_indices(const DiffusRenderArgs* a, int64_t* x, int64_t* y, int64_t* z, void* stream) {

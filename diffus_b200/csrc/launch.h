@@ -138,6 +138,12 @@ cudaError_t launch_to_quads(const float* linear, const int32_t dim[3], float* qu
 cudaError_t launch_gather_probe(const float* buf, int64_t n_floats, int reads, int64_t n_threads, uint32_t seed, float* sink,
                                 cudaStream_t st);
 
+// gn_kernels.cu: the Gauss-Newton system of each pose (trilinear sampler, float32 poses); partial holds 32 floats per ray,
+// med_tan 6 floats per pose (start > 0 only)
+cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, const int32_t* tie_count, float* med_tan, cudaStream_t st);
+cudaError_t launch_render_gn(const RenderParams& p, int layout, const float* med_tan, float* partial, float* loss, float* jtr,
+                             float* jtj, cudaStream_t st);
+
 // splat_kernels.cu
 int64_t splat_workspace_bytes(int H, int W);
 cudaError_t launch_splat_fwd(const float* c0, const float* c1, const float* c2, const float* val, int64_t n, int H, int W,

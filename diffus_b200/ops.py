@@ -489,6 +489,54 @@ class RenderMSELoss(torch.autograd.Function):
 
 
 # ---------------------------------------------------------------------------------------
+# Gauss-Newton system of each pose: one forward-mode render pass
+# ---------------------------------------------------------------------------------------
+def render_gauss_newton_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: List[int], sources: torch.Tensor,
+                             directions: torch.Tensor, target: torch.Tensor, n_samples: int, start: int, alpha: float,
+                             loss_out: Optional[torch.Tensor] = None, jtj_out: Optional[torch.Tensor] = None,
+                             jtr_out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Per pose p, with res = frame - target and J = d frame / d xi for a rigid twist xi = (v, w) of the pose about its source:
+    ``loss[p] = sum res^2``, ``JtJ[p] = J^T J`` (6x6), ``Jtr[p] = J^T res`` (6).  Trilinear sampler, float32 poses.
+
+    Two launches (+ two for the median when ``start > 0``).  ``*_out``: caller-provided output buffers (static tensors of a
+    CUDA graph), else fresh tensors."""
+    dev = _require_cuda(volume, bricks, sources, directions, target)
+    _check_inputs(volume, bricks, dims, sources, directions)
+    lib = _lib.load()
+    g = _lib.DiffusGaussNewtonArgs()
+    with _on_device(dev):
+        P, R = _fill_render_args(g.fwd, volume, bricks, dims, sources, directions, n_samples, start, alpha, SAMPLER_TRILINEAR,
+                                 False)
+        sout = n_samples - start
+        if tuple(target.shape) != (P, R, sout) or target.dtype != torch.float32 or not target.is_contiguous():
+            raise _lib.DiffusError(f"target must be contiguous float32 {(P, R, sout)}")
+        loss = _out_buffer(loss_out, (P,), dev, "loss_out")
+        jtj = _out_buffer(jtj_out, (P, 6, 6), dev, "jtj_out")
+        jtr = _out_buffer(jtr_out, (P, 6), dev, "jtr_out")
+        g.target, g.loss, g.jtr, g.jtj = target.data_ptr(), loss.data_ptr(), jtr.data_ptr(), jtj.data_ptr()
+        wbytes = lib.diffus_render_gauss_newton_workspace_bytes(C.byref(g))
+        ws = torch.empty((max(wbytes, 1),), dtype=torch.uint8, device=dev)
+        g.workspace, g.workspace_bytes = ws.data_ptr(), wbytes
+        _lib.check(lib.diffus_render_gauss_newton(C.byref(g), _stream(dev)), "diffus_render_gauss_newton")
+        _count(2 + (2 if start > 0 else 0))
+    return loss.view(P), jtj.view(P, 6, 6), jtr.view(P, 6)
+
+
+@torch.library.custom_op("diffus::render_gn", mutates_args=())
+def render_gn(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: List[int], sources: torch.Tensor,
+              directions: torch.Tensor, target: torch.Tensor, n_samples: int, start: int,
+              alpha: float) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    return render_gauss_newton_impl(volume, bricks, dims, sources, directions, target, n_samples, start, alpha)
+
+
+@render_gn.register_fake
+def _(volume, bricks, dims, sources, directions, target, n_samples, start, alpha):
+    P = sources.shape[0]
+    return (volume.new_empty((P,), dtype=torch.float32), volume.new_empty((P, 6, 6), dtype=torch.float32),
+            volume.new_empty((P, 6), dtype=torch.float32))
+
+
+# ---------------------------------------------------------------------------------------
 # indices / raw values
 # ---------------------------------------------------------------------------------------
 def ray_indices(dims, sources, directions, n_samples, start, product_f32=False):

@@ -161,6 +161,37 @@ def render_mse_loss(volume, sources: torch.Tensor, directions: torch.Tensor, tar
     return (loss, frame) if return_frame else loss
 
 
+def render_gauss_newton(volume, sources: torch.Tensor, directions: torch.Tensor, target: torch.Tensor, num_samples: int,
+                        attenuation_coeff: float = 0.5, start=0, *, sampler: str = "trilinear"):
+    """Gauss-Newton system of every pose's frame residual in one forward-mode render pass.
+
+    A pose update is the twist ``xi = (v, w)``: ``sources + v`` and the directions rotated by ``Rot(w)`` about the source
+    (:func:`diffus_b200.pose_recovery.apply_pose_twist`).  With ``res = frame - target`` and ``J = d frame / d xi`` at
+    ``xi = 0``, returns per pose ``loss (P,) = sum res^2``, ``JtJ (P,6,6) = J^T J`` and ``Jtr (P,6) = J^T res``.  ``2 Jtr / n``
+    is the gradient of :func:`render_mse_loss` (mean over n elements) in twist coordinates.  ``sources`` (P,3) and
+    ``directions`` (P,R,3) or (R,3) are float32 (float64 poses are not supported); ``volume`` is a (D,H,W) CUDA tensor or a
+    :class:`PreparedVolume`.  Only the trilinear sampler has a pose derivative.  The outputs are NOT differentiable: they
+    are what a Gauss-Newton / Levenberg-Marquardt step consumes (:func:`diffus_b200.pose_recovery.recover_poses`).
+    """
+    if _sampler_id(sampler) != SAMPLER_TRILINEAR:
+        raise DiffusError("render_gauss_newton needs sampler='trilinear' (the nearest sampler has no pose derivative)")
+    bricks = None
+    if isinstance(volume, PreparedVolume):
+        bricks, volume = volume.bricks, volume.volume
+    src = torch.as_tensor(sources, device=volume.device)
+    dirs = torch.as_tensor(directions, device=volume.device)
+    if src.dtype != torch.float32 or dirs.dtype != torch.float32:
+        raise DiffusError("render_gauss_newton takes float32 sources and directions")
+    if src.dim() == 1:
+        src = src.unsqueeze(0)
+    vol32 = (volume if volume.dtype == torch.float32 else volume.float()).detach().contiguous()
+    tgt = target.detach().to(torch.float32).contiguous()
+    if tgt.dim() == 2:
+        tgt = tgt.unsqueeze(0)
+    return ops.render_gauss_newton_impl(vol32, bricks, list(volume.shape), src.detach().contiguous(), dirs.detach().contiguous(),
+                                        tgt, int(num_samples), _resolve_start(start, num_samples), float(attenuation_coeff))
+
+
 def _resolve_start(start, num_samples: int) -> int:
     """``src/renderer.py:237-240``: a float start is a fraction of ``num_samples``."""
     if type(start) is float:

@@ -139,6 +139,26 @@ int64_t diffus_render_bwd_workspace_bytes(const DiffusRenderBwdArgs* args);
 int32_t diffus_render_bwd_needs_prefix(const DiffusRenderBwdArgs* args);
 int32_t diffus_render_backward(const DiffusRenderBwdArgs* args, void* stream);
 
+/* Gauss-Newton system of each pose in one forward-mode pass: with res = frame - target and J the derivative of the frame
+ * w.r.t. a rigid twist xi = (v, w) of the pose about its source (sources + v, directions rotated by Rot(w)),
+ *   loss[p] = sum res^2,   jtr[p] (6) = J^T res,   jtj[p] (6x6, full symmetric) = J^T J
+ * over the R x (S-start) elements of pose p.  (2/n) jtr is the gradient of the mean-squared loss over n elements in twist
+ * coordinates.  start > 0: the median-replaced coefficient's tangent is the mean of the tangents of the rays tied with the
+ * median.  Trilinear sampler and float32 poses only (the nearest sampler has no pose derivative): anything else returns
+ * DIFFUS_E_UNSUPPORTED.  Outputs are overwritten; the result is bit-identical from run to run (fixed-order sums). */
+typedef struct DiffusGaussNewtonArgs {
+    DiffusRenderArgs fwd;       /* the render; fwd.frame, fwd.seg_prefix and fwd.workspace are unused */
+    const float* target;        /* (P,R,S-start)                                             */
+    float* loss;                /* (P)                                                       */
+    float* jtr;                 /* (P,6)                                                     */
+    float* jtj;                 /* (P,6,6)                                                   */
+    void* workspace;            /* diffus_render_gauss_newton_workspace_bytes() bytes        */
+    int64_t workspace_bytes;
+} DiffusGaussNewtonArgs;
+
+int64_t diffus_render_gauss_newton_workspace_bytes(const DiffusGaussNewtonArgs* args);
+int32_t diffus_render_gauss_newton(const DiffusGaussNewtonArgs* args, void* stream);
+
 /* Clamped nearest-voxel indices of every ray point: the x, y, z int64 outputs of
  * custom_nearest_sampler (src/renderer.py:754-756, :816-819), cropped like
  * plot_beam_frame's return (:275).  Outputs are (P,R,S-start) int64. */
