@@ -48,16 +48,12 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if not force and not _stale():
         return LIB
     nvcc = _nvcc()
-    flags = list(NVCC_FLAGS)
-    flags += os.environ.get("DIFFUS_NVCC_EXTRA", "").split()     # kernel-development A/B switches (-DDIFFUS_TEX_GB=4 ...)
-    if os.environ.get("DIFFUS_DEV_MINIMAL") == "1":      # kernel-development shortcut (csrc/launch.h): benchmark kernels only
-        flags.append("-DDIFFUS_DEV_MINIMAL")
     os.makedirs(BUILD, exist_ok=True)
 
     def compile_one(item):
         src, extra, objname = item
         obj = os.path.join(BUILD, objname)
-        cmd = [nvcc, *flags, *extra, "-c", os.path.join(CSRC, src), "-o", obj]
+        cmd = [nvcc, *NVCC_FLAGS, *extra, "-c", os.path.join(CSRC, src), "-o", obj]
         r = subprocess.run(cmd, capture_output=True, text=True)
         with open(obj + ".log", "w") as f:
             f.write(" ".join(cmd) + "\n" + r.stdout + r.stderr)
@@ -74,38 +70,6 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if r.returncode != 0:
         raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")
     return LIB
-
-
-def build_variant(name: str, extra_flags, objects) -> str:
-    """Kernel-development aid: ``variants/libdiffus_<name>.so`` = the shipped objects with ``objects`` (names out of SOURCES)
-    recompiled with ``extra_flags``.  Pointed at by DIFFUS_B200_LIB for A/B runs on the GPU box; never the shipped library."""
-    build()
-    nvcc = _nvcc()
-    vdir = os.path.join(BUILD, name)
-    os.makedirs(vdir, exist_ok=True)
-    os.makedirs(os.path.join(HERE, "variants"), exist_ok=True)
-    objs = []
-
-    def one(item):
-        src, extra, objname = item
-        if objname not in objects:
-            return os.path.join(BUILD, objname)
-        obj = os.path.join(vdir, objname)
-        cmd = [nvcc, *NVCC_FLAGS, *extra, *extra_flags, "-c", os.path.join(CSRC, src), "-o", obj]
-        r = subprocess.run(cmd, capture_output=True, text=True)
-        with open(obj + ".log", "w") as f:
-            f.write(" ".join(cmd) + "\n" + r.stdout + r.stderr)
-        if r.returncode != 0:
-            raise RuntimeError(f"nvcc failed on {src}:\n{r.stdout}\n{r.stderr}")
-        return obj
-
-    with ThreadPoolExecutor(max_workers=4) as ex:
-        objs = list(ex.map(one, SOURCES))
-    lib = os.path.join(HERE, "variants", f"libdiffus_{name}.so")
-    r = subprocess.run([nvcc, "-shared", "-o", lib, *objs, "-gencode", "arch=compute_100a,code=sm_100a"], capture_output=True, text=True)
-    if r.returncode != 0:
-        raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")
-    return lib
 
 
 if __name__ == "__main__":

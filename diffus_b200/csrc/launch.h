@@ -1,6 +1,5 @@
 // Host-side launcher declarations (internal to the shared library).
 #pragma once
-#include <cstdlib>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -16,19 +15,14 @@ namespace diffus {
         constexpr bool P64_ = (Pv);                                        \
         __VA_ARGS__;                                                       \
     }
-// The cases of one layout.  -DDIFFUS_DEV_MINIMAL instantiates only the benchmark's kernels (trilinear, float32 pose,
-// brick / quad) -- a build-time shortcut for looking at one kernel's SASS, never used for the shipped library.
-// -DDIFFUS_LAYOUT_SLICE=n keeps one layout only: render_kernels.cu is compiled once per layout, in parallel (build.py).
-#ifdef DIFFUS_DEV_MINIMAL
-#define DIFFUS_LAYOUT_CASES(Lv, ...) DIFFUS_DISPATCH_CASE(DIFFUS_SAMPLER_TRILINEAR, Lv, false, __VA_ARGS__)
-#else
+// The cases of one layout.  -DDIFFUS_LAYOUT_SLICE=n keeps one layout only: render_kernels.cu is compiled once per layout,
+// in parallel (build.py).
 #define DIFFUS_LAYOUT_CASES(Lv, ...)                                        \
     DIFFUS_DISPATCH_CASE(DIFFUS_SAMPLER_NEAREST, Lv, false, __VA_ARGS__)    \
     DIFFUS_DISPATCH_CASE(DIFFUS_SAMPLER_NEAREST, Lv, true, __VA_ARGS__)     \
     DIFFUS_DISPATCH_CASE(DIFFUS_SAMPLER_TRILINEAR, Lv, false, __VA_ARGS__)  \
     DIFFUS_DISPATCH_CASE(DIFFUS_SAMPLER_TRILINEAR, Lv, true, __VA_ARGS__)
-#endif
-#if (!defined(DIFFUS_LAYOUT_SLICE) || DIFFUS_LAYOUT_SLICE == 0) && !defined(DIFFUS_DEV_MINIMAL)
+#if !defined(DIFFUS_LAYOUT_SLICE) || DIFFUS_LAYOUT_SLICE == 0
 #define DIFFUS_DISPATCH_L0(...) DIFFUS_LAYOUT_CASES(DIFFUS_LAYOUT_LINEAR, __VA_ARGS__)
 #else
 #define DIFFUS_DISPATCH_L0(...)
@@ -76,19 +70,14 @@ static inline cudaError_t ensure_smem(K kernel, size_t smem, int ctas_per_sm = 0
         pct = (int)(pick * 100 / 228);
         if (pct > 100) pct = 100;
     }
-    if (ctas_per_sm > 0) {                                   // kernel-development override: DIFFUS_CARVEOUT_PCT=<percent>
-        static const int forced = [] { const char* e = getenv("DIFFUS_CARVEOUT_PCT"); return e ? atoi(e) : 0; }();
-        if (forced > 0) pct = forced;
-    }
     return prepare_kernel((const void*)kernel, pct);
 }
 
 // Rays of two to four 512-column passes (513..2048 columns) with a pose gradient and no volume gradient go through the COOP form
 // of render_bwd_kernel (one ray per CTA, one pass per warp): it needs no forward pre-pass for the 512-column prefixes, so
-// DiffusRenderArgs.seg_prefix may be NULL for them.  DIFFUS_COOP=0 (kernel development) switches back to the multi-pass kernel.
+// DiffusRenderArgs.seg_prefix may be NULL for them.
 inline bool render_bwd_is_coop(int Sout, int64_t total_rays, int sampler, bool pose64, bool pose_grad, bool vol_grad) {
-    static const bool enabled = [] { const char* e = getenv("DIFFUS_COOP"); return !e || atoi(e) != 0; }();
-    return enabled && sampler == DIFFUS_SAMPLER_TRILINEAR && !pose64 && pose_grad && !vol_grad && Sout > PREFIX_STRIDE &&
+    return sampler == DIFFUS_SAMPLER_TRILINEAR && !pose64 && pose_grad && !vol_grad && Sout > PREFIX_STRIDE &&
            Sout <= 4 * PREFIX_STRIDE && total_rays <= 0x7fffffffLL;      // (one CTA per ray)
 }
 

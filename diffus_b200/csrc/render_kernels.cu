@@ -56,46 +56,10 @@ __device__ __forceinline__ M2 forward_chunk(const float r[G::CHUNK], M2 carry, f
 //               diff = frame - target, ebar = grad_scale * diff * att, accumulates diff^2
 //               and (optionally) stores the frame
 constexpr int LOSS_GRAD = 0, LOSS_MSE = 1;
-#ifndef DIFFUS_H_ROLLED
-#define DIFFUS_H_ROLLED 0    // 1: the sub-segment loop of the reverse sweep is not unrolled (half the sweep code, one more branch)
-#endif
-#ifndef DIFFUS_GATHER_PIPE
-#define DIFFUS_GATHER_PIPE 0   // 1: fused backward, TEXTURE layout: two batches of gathers in flight (software pipeline)
-#endif
-#ifndef DIFFUS_WIDE_SWEEP
-#define DIFFUS_WIDE_SWEEP 1    // one-pass pose-gradient kernels: single 512-column reverse sweep (see WideGeo)
-#endif
-#ifndef DIFFUS_WIDE_MULTIPASS
-#define DIFFUS_WIDE_MULTIPASS 0    // rays longer than one pass (config 5) as WIDE segments: 612 bytes of spills at 128 registers -- off
-#endif
-#ifndef DIFFUS_WIDE_VOLGRAD
-#define DIFFUS_WIDE_VOLGRAD 1     // the WIDE sweep for the fused volume-gradient kernels (config 4) too
-#endif
-#ifndef DIFFUS_CARVEOUT
-#define DIFFUS_CARVEOUT 1         // the same for the forward and the other backward kernels (resident warps from their launch bounds)
-#endif
-#ifndef DIFFUS_LANE_MAJOR_TARGET
-#define DIFFUS_LANE_MAJOR_TARGET 0   // 1: WIDE fused pose kernel stages the target / e-bar row lane-major (four 16-byte cp.async per lane,
-                                     // float4 accesses in the sweeps: 132 fewer instructions per ray).  Measured: bit-identical, 0.560 vs 0.536 ms.
-#endif
-#ifndef DIFFUS_WIDE_CARVEOUT
-#define DIFFUS_WIDE_CARVEOUT 1    // WIDE kernels: shared-memory carveout sized to their 4 resident CTAs (more L1 / texture cache)
-#endif
-#ifndef DIFFUS_WIDE_CTAS
-#define DIFFUS_WIDE_CTAS 4      // resident 4-warp CTA equivalents per SM of the WIDE kernels (4: 128 registers, 5: 96 and spills)
-#endif
-#ifndef DIFFUS_WIDE_WPB
-#define DIFFUS_WIDE_WPB 4       // rays (warps) per CTA of the WIDE kernels on large batches
-#endif
-#ifndef DIFFUS_FWD_GB
-#define DIFFUS_FWD_GB 1      // tiles per gather batch of the forward kernel (trilinear)
-#endif
-#ifndef DIFFUS_TEX_GB
-#define DIFFUS_TEX_GB 2      // tiles of tld4 gathers in flight per warp in the fused backward (TEXTURE layout)
-#endif
-#ifndef DIFFUS_TEX_GB_WIDE
-#define DIFFUS_TEX_GB_WIDE 4 // the same in the WIDE kernels (128 registers; the multi-pass kernel spills 620 bytes with 4: config 5 14.4 -> 15.8 ms)
-#endif
+constexpr int WIDE_CTAS = 4;     // resident 4-warp CTA equivalents per SM of the WIDE kernels (4: 128 registers, 5: 96 and spills)
+constexpr int FWD_GB = 1;        // tiles per gather batch of the forward kernel (trilinear)
+constexpr int TEX_GB = 2;        // tiles of tld4 gathers in flight per warp in the fused backward (TEXTURE layout)
+constexpr int TEX_GB_WIDE = 4;   // the same in the WIDE kernels (128 registers; the multi-pass kernel spills 620 bytes with 4: config 5 14.4 -> 15.8 ms)
 constexpr int BWD_DZ_STRIDE = FwdGeo::OBUF;   // floats between the per-axis rows of the spatial-gradient buffer
 
 // What the render kernels add to the plain echo backward: the impedances around the lane's columns, so that the
@@ -139,14 +103,11 @@ __device__ __forceinline__ M2 xch_load(const float* x) { return m2_make(x[0], x[
 //   vin         adjoint flowing into the segment's last column from later segments
 //   ncol_lane   number of existing columns in this lane's chunk (may be <= 0 or > CHUNK)
 // returns the adjoint flowing out of the segment's first column (into the previous segment)
-//   LM          (LOSS_MSE, no STORE_ZBAR) `gbuf` is this lane's OWN row of CHUNK floats, 16-byte aligned (lane-major staging of
-//               the target, see render_bwd_kernel): target and e-bar move as float4 -- 12 instead of 48 shared-memory
-//               instructions per lane and ray
-//   COOP        the segment is one of the passes of a ray, each walked by one warp of the CTA (ZMODE only): `vin` is
+//   COOP       the segment is one of the passes of a ray, each walked by one warp of the CTA (ZMODE only): `vin` is
 //               ignored -- the passes exchange their affine maps (and, for the last column's d loss / d Z, the weight of the
 //               next pass's first column) through zt->xch.  Every warp of the CTA must run the SAME instantiation:
 //               the function holds two __syncthreads().
-template <class G_, int LOSS, bool ZMODE = false, bool POSE_GRAD = false, bool STORE_ZBAR = false, bool FULL = false, bool LM = false,
+template <class G_, int LOSS, bool ZMODE = false, bool POSE_GRAD = false, bool STORE_ZBAR = false, bool FULL = false,
           bool COOP = false>
 __device__ __forceinline__ M2 backward_chunk(const float r[G_::CHUNK], const M2& carry, const M2& vin, float* gbuf,
                                              const float* att_lane, float* frame_lane, float grad_scale, int ncol_lane,
@@ -155,10 +116,7 @@ __device__ __forceinline__ M2 backward_chunk(const float r[G_::CHUNK], const M2&
                                              const float* att_scale = nullptr) {
     constexpr int CHUNK = G_::CHUNK;
     static_assert(!COOP || ZMODE, "COOP: render kernels only");
-    static_assert(!LM || (LOSS == LOSS_MSE && !STORE_ZBAR && CHUNK % 4 == 0), "LM: fused MSE without a volume gradient");
-    const int base = LM ? 0 : G_::pad(lane * CHUNK);        // columns lane*CHUNK .. +CHUNK-1 share a 32-column block
-    float4 t4 = make_float4(0.f, 0.f, 0.f, 0.f), g4 = t4;   // LM: four columns of the target / of e-bar at a time
-    auto comp = [](const float4& v, int k) { return k == 0 ? v.x : k == 1 ? v.y : k == 2 ? v.z : v.w; };
+    const int base = G_::pad(lane * CHUNK);        // columns lane*CHUNK .. +CHUNK-1 share a 32-column block
     // chunk product and exclusive prefix: reuse them when the caller already ran this sweep (prefix pass)
     M2 T, P;
     if (known_total) {
@@ -186,8 +144,7 @@ __device__ __forceinline__ M2 backward_chunk(const float r[G_::CHUNK], const M2&
         const float att = att_lane ? (att_scale ? __fmul_rn(att_lane[i], *att_scale) : att_lane[i]) : 1.f;     // (scale: see render_bwd_kernel)
         if (LOSS == LOSS_MSE) {
             float fr = __fmul_rn(nan_to_num(e), att);
-            if (LM && (i & 3) == 0) t4 = *reinterpret_cast<const float4*>(gbuf + i);
-            float diff = fr - (LM ? comp(t4, i & 3) : gbuf[base + i]);
+            float diff = fr - gbuf[base + i];
             if (FULL || i < ncol_lane) {
                 loss_acc += diff * diff;
                 if (frame_lane) frame_lane[i] = fr;      // 8 consecutive floats per lane: whole 32-byte sectors
@@ -197,12 +154,7 @@ __device__ __forceinline__ M2 backward_chunk(const float r[G_::CHUNK], const M2&
             ge = gbuf[base + i] * att;
         }
         if (!finite || (!FULL && i >= ncol_lane)) ge = 0.f;   // columns that do not exist: the table beyond Sout is not filled
-        if (LM) {
-            if ((i & 3) == 0) g4.x = ge; else if ((i & 3) == 1) g4.y = ge; else if ((i & 3) == 2) g4.z = ge; else g4.w = ge;
-            if ((i & 3) == 3) *reinterpret_cast<float4*>(gbuf + i - 3) = g4;
-        } else {
-            gbuf[base + i] = ge;
-        }
+        gbuf[base + i] = ge;
         const float2 dcol = make_float2(ge * inv, -ge * e * inv);   // D = [[0, da], [0, db]];  B += D G^T
         B.c0 = __ffma2_rn(dcol, bcast(G.b()), B.c0);
         B.c1 = __ffma2_rn(dcol, bcast(G.d()), B.c1);
@@ -263,8 +215,7 @@ __device__ __forceinline__ M2 backward_chunk(const float r[G_::CHUNK], const M2&
         const float2 pc1 = __ffma2_rn(Q.c0, bcast(r[i]), Q.c1);      // (b, d) of the prefix through column i
         float inv = fast_rcp(pc1.y);
         float e = echo_of(pc1.x, inv);
-        if (LM && (i & 3) == 3) g4 = *reinterpret_cast<const float4*>(gbuf + i - 3);
-        float ge = LM ? comp(g4, i & 3) : gbuf[base + i];
+        float ge = gbuf[base + i];
         M2 Pbar = V;
         Pbar.c1 = __fadd2_rn(Pbar.c1, make_float2(ge * inv, -ge * e * inv));
         const float2 t0 = __fmul2_rn(Q.c0, Pbar.c0), t1 = __fmul2_rn(Q.c0, Pbar.c1), t2 = __fmul2_rn(Q.c1, Pbar.c0);
@@ -322,12 +273,6 @@ __device__ __forceinline__ void cp_async_stream4(float* smem_dst, const float* g
 __device__ __forceinline__ int64_t pose_of_ray(int64_t ray, const RenderParams& p) {
     if (p.total_rays <= 0xffffffffLL) return (int64_t)((uint32_t)ray / (uint32_t)p.n_rays);
     return ray / p.n_rays;
-}
-
-__device__ __forceinline__ void cp_async_stream16(float* smem_dst, const float* gmem_src, uint64_t policy) {
-    asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)),
-                 "l"(gmem_src), "l"(policy)
-                 : "memory");
 }
 
 // coefficient of the interface owned by column c from the two impedances around it
@@ -414,7 +359,7 @@ __global__ void __launch_bounds__(128, 7) render_fwd_kernel(const RenderParams p
         // batches of tiles: every load of a batch is issued before the first one is combined.  One tile per batch for
         // the trilinear sampler: measured, 28 resident warps (7 CTAs at 72 registers) hide the gather latency better than
         // deeper batches at fewer warps (0.460 vs 0.470 ms per 1024 poses)
-        constexpr int GB = SAMPLER == DIFFUS_SAMPLER_NEAREST ? 8 : DIFFUS_FWD_GB;
+        constexpr int GB = SAMPLER == DIFFUS_SAMPLER_NEAREST ? 8 : FWD_GB;
         const int nt_full = (ncol >> 5) / GB * GB;       // batches of complete tiles run without the per-lane bounds tests
         for (int t0 = 0; t0 < nt_full; t0 += GB) {
             Fetch<SAMPLER, LAYOUT> fe[GB];
@@ -530,27 +475,6 @@ __device__ __forceinline__ void scatter_volume_grad(const RenderParams& p, const
 // (no slot-key sums, no "touched" flags), but a slot misses in some lane of the warp at almost every sample, so the branch
 // bodies run nearly always: config 4 step 5.78 vs 5.10 ms (5.65 with two samples per trip).
 // ---------------------------------------------------------------------------------------
-#ifndef DIFFUS_SCATTER_BRANCHY
-#define DIFFUS_SCATTER_BRANCHY 0   // slot miss handled in one branch region (flush + re-key + zero) instead of per-component selects
-#endif
-#ifndef DIFFUS_EARLY_POSE_LOAD
-#define DIFFUS_EARLY_POSE_LOAD 1   // backward kernels: the ray's pose is loaded before the attenuation table is filled (A/B switch)
-#endif
-#ifndef DIFFUS_WARP_SUM8
-#define DIFFUS_WARP_SUM8 1     // pose-gradient kernels: the ray's seven final sums in one transposing warp reduction (A/B switch)
-#endif
-#ifndef DIFFUS_COOP_NEIGHBOUR_SMEM
-#define DIFFUS_COOP_NEIGHBOUR_SMEM 1   // COOP: the sample before a pass comes from the previous warp's buffer (one more barrier) instead of
-                                       // one more dependent single-lane gather per pass: config 5 9.64 -> 9.42 ms (benchmarks/gpu/r2_call57.sh)
-#endif
-#ifndef DIFFUS_SCATTER_UNROLL
-#define DIFFUS_SCATTER_UNROLL 1    // samples per trip of the trilinear quad-slot loop (2: config 4 step 5.26 vs 5.04 ms, benchmarks/gpu/r2_call56.sh)
-#endif
-#define DIFFUS_PRAGMA_(x) _Pragma(#x)
-#define DIFFUS_PRAGMA_UNROLL(n) DIFFUS_PRAGMA_(unroll n)
-#ifndef DIFFUS_SCATTER_QUADS
-#define DIFFUS_SCATTER_QUADS 1
-#endif
 constexpr uint32_t QUAD_NONE = 0xffffffffu;
 constexpr int SCATTER_RUN = PREFIX_STRIDE / 32;      // consecutive samples per lane in the scatter phase
 
@@ -571,17 +495,6 @@ __device__ __forceinline__ void red_add_v4_if(float* base, uint32_t quad, const 
 // it is flushed (predicated reduction) and the slot restarts from zero.  Branch-free: 4 selects + 4 FMAs for the accumulators.
 __device__ __forceinline__ void quad_slot_fma(float* grad, uint32_t& K, float4& acc, uint32_t key, float a0, float a1, float k0, float k1,
                                               bool nz) {
-#if DIFFUS_SCATTER_BRANCHY
-    if (nz && key != K) {                                   // one (rare) branch region: flush, re-key, restart from zero
-        red_add_v4_if(grad, K, acc, K != QUAD_NONE);
-        K = key;
-        acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    }
-    acc.x = __fmaf_rn(a0, k0, acc.x);                       // a0 = a1 = 0 when !nz: the slot is left as it is
-    acc.y = __fmaf_rn(a0, k1, acc.y);
-    acc.z = __fmaf_rn(a1, k0, acc.z);
-    acc.w = __fmaf_rn(a1, k1, acc.w);
-#else
     const bool miss = nz && key != K;
     red_add_v4_if(grad, K, acc, miss && K != QUAD_NONE);
     K = miss ? key : K;
@@ -589,7 +502,6 @@ __device__ __forceinline__ void quad_slot_fma(float* grad, uint32_t& K, float4& 
     acc.y = __fmaf_rn(a0, k1, miss ? 0.f : acc.y);
     acc.z = __fmaf_rn(a1, k0, miss ? 0.f : acc.z);
     acc.w = __fmaf_rn(a1, k1, miss ? 0.f : acc.w);
-#endif
 }
 
 // (nearest sampler) one parity slot: accumulate `v` under `key`
@@ -643,7 +555,8 @@ __device__ __forceinline__ void scatter_pass_quads(const RenderParams& p, const 
     float4 acc[8];
 #pragma unroll
     for (int s = 0; s < 8; ++s) { K[s] = QUAD_NONE; acc[s] = make_float4(0.f, 0.f, 0.f, 0.f); }
-    DIFFUS_PRAGMA_UNROLL(DIFFUS_SCATTER_UNROLL)
+    // one sample per trip (two: config 4 step 5.26 vs 5.04 ms, benchmarks/gpu/r2_call56.sh)
+#pragma unroll 1
     for (int i = 0; i < SCATTER_RUN; ++i) {
         const int c = col0 + i;
         const float zbar = c < ncol ? gbuf[G::pad(c)] : 0.f;
@@ -695,12 +608,8 @@ __device__ __forceinline__ void scatter_pass_quads(const RenderParams& p, const 
 // WIDE (one-pass rays longer than 256 columns): the reverse sweep walks the pass as ONE 512-column segment, 16 columns per
 // lane with a prefix checkpoint every 4 (Geo<16, 4>), instead of two 256-column sub-segments of 8 columns per lane: one
 // prefix scan and one suffix scan per ray instead of two of each, no prefix pre-pass over the first sub-segment, for 1.5
-// instead of 0.5 recomputed transfer products per column.
+// instead of 0.5 recomputed transfer products per column.  (Rays longer than one pass as WIDE segments: 612 bytes of spills.)
 using WideGeo = Geo<16, 4>;
-constexpr int BWD_LM_STRIDE = WideGeo::CHUNK + 4;                 // lane-major target / e-bar row: 20 floats per lane (80 B: float4 accesses
-                                                                  // of the eight lanes of a quarter warp fall on distinct banks)
-constexpr int BWD_LM_ROW = 32 * BWD_LM_STRIDE;
-constexpr int BWD_SMEM_PER_WARP_LM = (BWD_LM_ROW + BWD_ZBUF + 3 * BWD_DZ + 3) / 4 * 4;   // the lane-major row comes first: 16-byte aligned
 // COOP (rays of 513..2048 columns = two to four passes; config 5 has four): ONE ray per CTA of as many warps as the ray has
 // passes, warp w walks pass w.  The passes of a ray
 // depend on each other only through (i) the forward prefix entering the pass = the product of the earlier passes' transfer
@@ -709,12 +618,11 @@ constexpr int BWD_SMEM_PER_WARP_LM = (BWD_LM_ROW + BWD_ZBUF + 3 * BWD_DZ + 3) / 
 // shared memory (CoopXch; five __syncthreads per ray in all), so the ray is gathered ONCE: no forward pre-pass for the 512-column
 // prefixes (it re-gathered 3 of 4 passes, ~30 % of the config-5 step), no state carried from pass to pass through the gather
 // loop (the single 512-column WIDE sweep fits 128 registers like the one-pass kernel's).
-template <int SAMPLER, int LAYOUT, bool POSE64, bool POSE_GRAD, bool VOL_GRAD, int LOSS, bool ONE_PASS, bool WIDE = false, bool LM = false,
+template <int SAMPLER, int LAYOUT, bool POSE64, bool POSE_GRAD, bool VOL_GRAD, int LOSS, bool ONE_PASS, bool WIDE = false,
           bool COOP = false>
-__global__ void __launch_bounds__((WIDE && !COOP) ? 32 * DIFFUS_WIDE_WPB : 128,
-                                  COOP ? 4 : WIDE ? DIFFUS_WIDE_CTAS * 4 / DIFFUS_WIDE_WPB : ((ONE_PASS && !VOL_GRAD) ? 5 : 4))
+__global__ void __launch_bounds__(128, COOP ? 4 : WIDE ? WIDE_CTAS : ((ONE_PASS && !VOL_GRAD) ? 5 : 4))
 render_bwd_kernel(const RenderParams p) {
-    static_assert(!COOP || (WIDE && !ONE_PASS && !VOL_GRAD && !LM && !POSE64), "COOP: long rays, WIDE sweep, no volume gradient");
+    static_assert(!COOP || (WIDE && !ONE_PASS && !VOL_GRAD && !POSE64), "COOP: long rays, WIDE sweep, no volume gradient");
     using G = typename std::conditional<WIDE, WideGeo, BwdGeo>::type;
     constexpr int BWD_SUB = PREFIX_STRIDE / G::SEG;
     constexpr int SS = PREFIX_STRIDE;        // columns gathered per pass (BWD_SUB sub-segments of G::SEG)
@@ -731,23 +639,15 @@ render_bwd_kernel(const RenderParams p) {
     const int64_t pose = live ? pose_of_ray(ray, p) : 0;
     RaySetup<POSE64> rs;
     float med = 0.f;
-    if (DIFFUS_EARLY_POSE_LOAD && live) {
+    if (live) {
         rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.n_rays, p.dir_pose_stride, p.product_f32);
         if (p.median) med = __ldg(p.median + pose);
     }
     fill_attenuation_padded<G>(att, ONE_PASS ? p.Sout : min(p.Sout, SS), p.alpha);
     if (!live) return;                       // (COOP: the grid is exactly the rays -- no warp leaves before the barriers)
-    if (!DIFFUS_EARLY_POSE_LOAD) {
-        rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.n_rays, p.dir_pose_stride, p.product_f32);
-        if (p.median) med = __ldg(p.median + pose);
-    }
-    static_assert(!LM || (WIDE && ONE_PASS && LOSS == LOSS_MSE && !VOL_GRAD), "LM: the one-pass fused pose kernels");
-    // LM: the target / e-bar row is laid out LANE-major (lane l owns floats [20 l, 20 l + 16)): the chunk phase is its only
-    // reader, so it is staged with four 16-byte cp.async per lane and moved as float4 (132 fewer instructions per ray)
-    float* wbase = smem + p.att_slots_padded + warp * (LM ? BWD_SMEM_PER_WARP_LM : BWD_SMEM_PER_WARP);   // att_slots_padded % 4 == 0
-    float* zbuf = LM ? wbase + BWD_LM_ROW : wbase;
-    float* gbuf = LM ? wbase : zbuf + BWD_ZBUF;    // target / upstream gradient in, d loss / d r out
-    float* dz = LM ? zbuf + BWD_ZBUF : gbuf + BWD_OBUF;    // [3][BWD_DZ] spatial gradient of Z at each sample (padded rows)
+    float* zbuf = smem + p.att_slots_padded + warp * BWD_SMEM_PER_WARP;
+    float* gbuf = zbuf + BWD_ZBUF;           // target / upstream gradient in, d loss / d r out
+    float* dz = gbuf + BWD_OBUF;             // [3][BWD_DZ] spatial gradient of Z at each sample (padded rows)
     const float* gin = (LOSS == LOSS_MSE ? p.target : p.grad_frame) + ray * (int64_t)p.Sout;
     float* fout = (LOSS == LOSS_MSE && p.frame) ? p.frame + ray * (int64_t)p.Sout : nullptr;
     if (lane == 0) zbuf[0] = 0.f;
@@ -771,45 +671,29 @@ render_bwd_kernel(const RenderParams p) {
         const int ntile = (ncol + 31) >> 5;
         const int nsub = (ncol + G::SEG - 1) / G::SEG;
         // The target (or upstream-gradient) row streams from HBM: copy it straight into shared
-        // memory with cp.async at the top of the pass so its latency hides behind the gathers.
+        // memory with cp.async at the top of the pass so its latency hides behind the gathers.  (Staged lane-major and moved
+        // as float4 in the sweeps: 132 fewer instructions per ray, bit-identical, but 0.560 vs 0.536 ms.)
         {
             const int nt = nsub * (G::SEG / 32);
-            if (LM) {
-                const int lc = lane * G::CHUNK;
-                float* dst = gbuf + lane * BWD_LM_STRIDE;
-                const float* src = gin + c0 + lc;
-                if (lc + G::CHUNK <= ncol && (((uintptr_t)src) & 15u) == 0) {        // the usual case: four 16-byte copies
+            // complete tiles: no bounds test.  pad(32 t + lane) = 33 t + lane: both addresses advance by a constant per
+            // tile, so the copies are one instruction each with immediate offsets
+            {
+                float* dst = gbuf + lane;
+                const float* src = gin + c0 + lane;
+                const int nfull = ncol >> 5;
+                if ((ONE_PASS || COOP) && nfull == SS / 32) {
 #pragma unroll
-                    for (int q = 0; q < G::CHUNK / 4; ++q) cp_async_stream16(dst + 4 * q, src + 4 * q, stream_policy);
+                    for (int t = 0; t < SS / 32; ++t) cp_async_stream4(dst + 33 * t, src + 32 * t, stream_policy);
                 } else {
-#pragma unroll
-                    for (int i = 0; i < G::CHUNK; ++i) {
-                        if (lc + i < ncol) cp_async_stream4(dst + i, src + i, stream_policy);
-                        else dst[i] = 0.f;                   // columns that do not exist carry no gradient
-                    }
+                    for (int t = 0; t < nfull; ++t) cp_async_stream4(dst + 33 * t, src + 32 * t, stream_policy);
                 }
-                __pipeline_commit();
-            } else {
-                // complete tiles: no bounds test.  pad(32 t + lane) = 33 t + lane: both addresses advance by a constant per
-                // tile, so the copies are one instruction each with immediate offsets
-                {
-                    float* dst = gbuf + lane;
-                    const float* src = gin + c0 + lane;
-                    const int nfull = ncol >> 5;
-                    if ((ONE_PASS || COOP) && nfull == SS / 32) {
-#pragma unroll
-                        for (int t = 0; t < SS / 32; ++t) cp_async_stream4(dst + 33 * t, src + 32 * t, stream_policy);
-                    } else {
-                        for (int t = 0; t < nfull; ++t) cp_async_stream4(dst + 33 * t, src + 32 * t, stream_policy);
-                    }
-                }
-                for (int t = ncol >> 5; t < nt; ++t) {
-                    int idx = t * 32 + lane;
-                    if (idx < ncol) cp_async_stream4(gbuf + G::pad(idx), gin + c0 + idx, stream_policy);
-                    else gbuf[G::pad(idx)] = 0.f;            // columns that do not exist carry no gradient
-                }
-                __pipeline_commit();
             }
+            for (int t = ncol >> 5; t < nt; ++t) {
+                int idx = t * 32 + lane;
+                if (idx < ncol) cp_async_stream4(gbuf + G::pad(idx), gin + c0 + idx, stream_policy);
+                else gbuf[G::pad(idx)] = 0.f;            // columns that do not exist carry no gradient
+            }
+            __pipeline_commit();
             // gather phase: one pass over the volume for these columns.  (A cp.async ring for the
             // gathers themselves was measured slower than plain loads: LDGSTS issues at a quarter of
             // the LDG rate and adds eight shared-memory reads per sample, DESIGN.md section 4.)
@@ -820,8 +704,9 @@ render_bwd_kernel(const RenderParams p) {
             // spilled and one tile per batch was the fastest: 0.753 / 0.779 / 0.785).
             // TEXTURE (round 2): with the shared-memory carveout sized to the resident CTAs (60 KB of L1 / texture cache instead of 28)
             // deeper batches pay again on the WIDE kernel (128 registers): 1 pipelined / 2 / 2 pipelined / 4 / 4 pipelined / 8 tiles:
-            // 0.564 / 0.573 / 0.555 / 0.542 / 0.562 / 0.586 ms (profiles/r2_carveout.md).
-            constexpr int GB = SAMPLER == DIFFUS_SAMPLER_NEAREST ? 8 : (LAYOUT == DIFFUS_LAYOUT_TEXTURE ? (WIDE ? DIFFUS_TEX_GB_WIDE : DIFFUS_TEX_GB) : ((LAYOUT == DIFFUS_LAYOUT_QUAD && ONE_PASS) ? 4 : 2));
+            // 0.564 / 0.573 / 0.555 / 0.542 / 0.562 / 0.586 ms (profiles/r2_carveout.md; pipelined: the next batch is issued
+            // before the current one is combined).
+            constexpr int GB = SAMPLER == DIFFUS_SAMPLER_NEAREST ? 8 : (LAYOUT == DIFFUS_LAYOUT_TEXTURE ? (WIDE ? TEX_GB_WIDE : TEX_GB) : ((LAYOUT == DIFFUS_LAYOUT_QUAD && ONE_PASS) ? 4 : 2));
             // batches whose tiles are all complete run without the per-lane bounds tests; the tail keeps them
             const int nt_full = (ncol >> 5) / GB * GB;
             auto issue_batch = [&](Fetch<SAMPLER, LAYOUT>(&fe)[GB], int t0) {
@@ -847,29 +732,10 @@ render_bwd_kernel(const RenderParams p) {
                     }
                 }
             };
-            // The gather phase is latency-bound (profiles/r2_fused_kernel_texture.md: the first use of a tld4 result holds
-            // 17 % of all warp time): with texture gathers, which return in order, the next batch is issued BEFORE the
-            // current one is combined, so the combine + shared-memory stores overlap the flight of the next gathers.
-            constexpr bool PIPELINED = DIFFUS_GATHER_PIPE && SAMPLER == DIFFUS_SAMPLER_TRILINEAR && LAYOUT == DIFFUS_LAYOUT_TEXTURE;
-            if (PIPELINED && nt_full > 0 && nt_full % (2 * GB) == 0) {        // (warp-uniform) branch-free steady state
-                Fetch<SAMPLER, LAYOUT> fa[GB], fb[GB];
-                issue_batch(fa, 0);
-                int t0 = 0;
-                for (; t0 + 2 * GB < nt_full; t0 += 2 * GB) {
-                    issue_batch(fb, t0 + GB);
-                    finish_batch(fa, t0);
-                    issue_batch(fa, t0 + 2 * GB);
-                    finish_batch(fb, t0 + GB);
-                }
-                issue_batch(fb, t0 + GB);
-                finish_batch(fa, t0);
-                finish_batch(fb, t0 + GB);
-            } else {
-                for (int t0 = 0; t0 < nt_full; t0 += GB) {
-                    Fetch<SAMPLER, LAYOUT> fe[GB];
-                    issue_batch(fe, t0);
-                    finish_batch(fe, t0);
-                }
+            for (int t0 = 0; t0 < nt_full; t0 += GB) {
+                Fetch<SAMPLER, LAYOUT> fe[GB];
+                issue_batch(fe, t0);
+                finish_batch(fe, t0);
             }
             for (int t0 = nt_full; t0 < nt; t0 += GB) {
                 Fetch<SAMPLER, LAYOUT> fe[GB];
@@ -900,14 +766,14 @@ render_bwd_kernel(const RenderParams p) {
             }
             __pipeline_wait_prior(0);
         }
-        if (COOP && DIFFUS_COOP_NEIGHBOUR_SMEM) {
+        if (COOP) {
             // the sample before the pass's first column is the previous warp's last one: one more barrier instead of one more
-            // (dependent, single-lane) gather per pass
+            // (dependent, single-lane) gather per pass: config 5 9.64 -> 9.42 ms (benchmarks/gpu/r2_call57.sh)
             __syncthreads();
             if (lane == 0 && warp > 0) zbuf[G::pad(0)] = zbuf[G::pad(SS) - BWD_SMEM_PER_WARP];
         }
         if (lane == 0) {
-            if (s > 0 && !(COOP && DIFFUS_COOP_NEIGHBOUR_SMEM)) {                     // left neighbour of the pass's first column
+            if (s > 0 && !COOP) {                     // left neighbour of the pass's first column
                 int k = p.start + c0 - 1;
                 float g[3];
                 zbuf[G::pad(0)] = sample_volume<SAMPLER, LAYOUT, false>(p.vol, rs.coord(0, k), rs.coord(1, k), rs.coord(2, k), g);
@@ -956,11 +822,7 @@ render_bwd_kernel(const RenderParams p) {
         }
         // reverse scan, last sub-segment first; it ends in d loss / d Z per column and the pose accumulators
         zt.w_after = (c0 + ncol < p.Sout) ? carry_w : 0.f;
-#if DIFFUS_H_ROLLED
-#pragma unroll 1
-#else
 #pragma unroll
-#endif
         for (int h = BWD_SUB - 1; h >= 0; --h) {
             if (h < nsub) {
                 const int off = h * G::SEG;
@@ -976,18 +838,18 @@ render_bwd_kernel(const RenderParams p) {
                 zt.kbase = (float)(p.start + c0 + lane_col);
                 zt.rbar1 = (p.first_rbar && s == 0 && h == 0) ? p.first_rbar + ray : nullptr;
                 const M2* kt = (COOP || (h == 0 && have0)) ? &T0 : nullptr;
-                M2 ch = carry[0];                        // (a select, not an indexed read: the loop may be rolled)
+                M2 ch = carry[0];                        // (a select, not an indexed read: carry[h] changes the code and its registers)
                 if (BWD_SUB == 2 && h == 1) ch = carry[BWD_SUB - 1];
                 float* fl = fout ? fout + c0 + lane_col : nullptr;
-                float* gl = LM ? gbuf + lane * BWD_LM_STRIDE : gbuf + G::pad(off);
+                float* gl = gbuf + G::pad(off);
                 const float pass_scale = ONE_PASS ? 1.f : expf(-p.alpha * (float)c0);
                 const float* asc = ONE_PASS ? nullptr : &pass_scale;
                 if (full)
-                    vin = backward_chunk<G, LOSS, true, POSE_GRAD, VOL_GRAD, true, LM, COOP>(
+                    vin = backward_chunk<G, LOSS, true, POSE_GRAD, VOL_GRAD, true, COOP>(
                         r, ch, vin, gl, att + G::pad(ONE_PASS ? c0 + lane_col : lane_col), fl, p.grad_scale, ncol - lane_col,
                         loss_acc, lane, &zt, kt, &E0, asc);
                 else
-                    vin = backward_chunk<G, LOSS, true, POSE_GRAD, VOL_GRAD, false, LM, COOP>(
+                    vin = backward_chunk<G, LOSS, true, POSE_GRAD, VOL_GRAD, false, COOP>(
                         r, ch, vin, gl, att + G::pad(ONE_PASS ? c0 + lane_col : lane_col), fl, p.grad_scale, ncol - lane_col,
                         loss_acc, lane, &zt, kt, &E0, asc);
                 zt.w_after = zt.w_first;
@@ -999,7 +861,7 @@ render_bwd_kernel(const RenderParams p) {
 
         // tile phase, only for the volume gradient: scatter d loss / d Z_c with lane = consecutive sample
         if (VOL_GRAD) {
-            if (DIFFUS_SCATTER_QUADS && GradLayout<LAYOUT>::value == DIFFUS_LAYOUT_BRICK) {
+            if (GradLayout<LAYOUT>::value == DIFFUS_LAYOUT_BRICK) {
                 scatter_pass_quads<SAMPLER, POSE64>(p, rs, gbuf, c0, ncol, lane);       // lane = 16 consecutive samples
             } else {
                 for (int t = 0; t < ntile; ++t) {                                        // lane = consecutive sample
@@ -1031,8 +893,7 @@ render_bwd_kernel(const RenderParams p) {
         }
         return;
     }
-#if DIFFUS_WARP_SUM8
-    if (POSE_GRAD) {              // the ray's seven sums (3 + 3 + loss) in one transposing reduction: 9 shuffles instead of 35
+    if (POSE_GRAD) {             // the ray's seven sums (3 + 3 + loss) in one transposing reduction: 9 shuffles instead of 35
         float v[8] = {zt.acc[0].x, zt.acc[1].x, zt.acc[2].x, zt.acc[0].y, zt.acc[1].y, zt.acc[2].y, loss_acc, 0.f};
         const float t = warp_sum8(v, lane);
         const int j = warp_sum8_index(lane);
@@ -1042,17 +903,6 @@ render_bwd_kernel(const RenderParams p) {
             else if (j == 6 && LOSS == LOSS_MSE && p.loss_partial) p.loss_partial[ray] = t;
         }
         return;
-    }
-#endif
-    if (POSE_GRAD) {
-#pragma unroll
-        for (int a = 0; a < 3; ++a) {
-            float ss = warp_sum(zt.acc[a].x), dd = warp_sum(zt.acc[a].y);
-            if (lane == 0) {
-                p.grad_src_partial[ray * 3 + a] = ss;
-                p.grad_dir[ray * 3 + a] = dd;
-            }
-        }
     }
     if (LOSS == LOSS_MSE && p.loss_partial) {
         float l = warp_sum(loss_acc);
@@ -1274,7 +1124,7 @@ cudaError_t DIFFUS_FWD_NAME(const RenderParams& p_in, int sampler, int layout, i
     int wpb = warps_per_block(p.total_rays);
     size_t smem = ((size_t)p.att_slots + (size_t)wpb * FWD_SMEM_PER_WARP) * sizeof(float);
     unsigned grid = (unsigned)((p.total_rays + wpb - 1) / wpb);
-    DIFFUS_DISPATCH(auto k = render_fwd_kernel<S_, L_, P64_>; cudaError_t e = ensure_smem(k, smem, DIFFUS_CARVEOUT ? 28 / wpb : 0);
+    DIFFUS_DISPATCH(auto k = render_fwd_kernel<S_, L_, P64_>; cudaError_t e = ensure_smem(k, smem, 28 / wpb);
                     if (e != cudaSuccess) return e; k<<<grid, wpb * 32, smem, st>>>(p); return cudaGetLastError())
     return cudaErrorInvalidValue;
 }
@@ -1283,61 +1133,40 @@ template <int S_, int L_, bool P64_, int LOSS>
 static cudaError_t launch_bwd_g(const RenderParams& p, bool pg, bool vg, unsigned grid, int threads, size_t smem,
                                 cudaStream_t st) {
     constexpr bool TRI = S_ == DIFFUS_SAMPLER_TRILINEAR;
-#define DIFFUS_BWD_GO(PG, VG)                                                   \
-    {                                                                           \
-        /* the one-pass specialisation exists for float32 poses only (build time) */ \
-        if (DIFFUS_LANE_MAJOR_TARGET && DIFFUS_WIDE_SWEEP && !P64_ && TRI && PG && !VG && LOSS == LOSS_MSE &&            \
-            p.Sout <= PREFIX_STRIDE && p.Sout > BwdGeo::SEG) {                  \
-            auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, true, true,                                          \
-                                       (DIFFUS_LANE_MAJOR_TARGET && DIFFUS_WIDE_SWEEP && TRI && PG && !VG && LOSS == LOSS_MSE)>; \
-            int wpb_ = threads / 32;                                            \
-            if (wpb_ == 4) wpb_ = DIFFUS_WIDE_WPB;                              \
-            const size_t smem_ = ((size_t)p.att_slots_padded + (size_t)wpb_ * BWD_SMEM_PER_WARP_LM) * sizeof(float); \
-            cudaError_t e = ensure_smem(k, smem_, DIFFUS_WIDE_CTAS * 4 / wpb_); \
-            if (e != cudaSuccess) return e;                                     \
-            k<<<(unsigned)((p.total_rays + wpb_ - 1) / wpb_), wpb_ * 32, smem_, st>>>(p); \
-            return cudaGetLastError();                                          \
-        }                                                                       \
-        if (DIFFUS_WIDE_SWEEP && !P64_ && ((TRI && PG && !VG) || (DIFFUS_WIDE_VOLGRAD && VG && !PG && LOSS == LOSS_MSE)) &&  \
-            p.Sout <= PREFIX_STRIDE && p.Sout > BwdGeo::SEG) {                  \
-            auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, true,       \
-                                       (DIFFUS_WIDE_SWEEP && ((TRI && PG && !VG) || (DIFFUS_WIDE_VOLGRAD && VG && !PG && LOSS == LOSS_MSE)))>; \
-            int wpb_ = threads / 32;                                            \
-            if (wpb_ == 4) wpb_ = DIFFUS_WIDE_WPB;                              \
-            const size_t smem_ = ((size_t)p.att_slots_padded + (size_t)wpb_ * BWD_SMEM_PER_WARP) * sizeof(float); \
-            cudaError_t e = ensure_smem(k, smem_, DIFFUS_WIDE_CARVEOUT ? DIFFUS_WIDE_CTAS * 4 / wpb_ : 0); \
-            if (e != cudaSuccess) return e;                                     \
-            k<<<(unsigned)((p.total_rays + wpb_ - 1) / wpb_), wpb_ * 32, smem_, st>>>(p); \
-            return cudaGetLastError();                                          \
-        }                                                                       \
-        if (!P64_ && p.Sout <= PREFIX_STRIDE) {                                 \
-            auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, true>;      \
-            cudaError_t e = ensure_smem(k, smem, DIFFUS_CARVEOUT ? ((VG) ? 16 : 20) / (threads / 32) : 0); \
-            if (e != cudaSuccess) return e;                                     \
-            k<<<grid, threads, smem, st>>>(p);                                  \
-            return cudaGetLastError();                                          \
-        }                                                                       \
+#define DIFFUS_BWD_GO(PG, VG)                                                                                         \
+    {                                                                                                                 \
+        /* the one-pass specialisations exist for float32 poses only (build time); the WIDE sweep serves the pose */   \
+        /* gradient alone and, under MSE, the volume gradient alone */                                                \
+        constexpr bool WIDE_ = !P64_ && ((TRI && PG && !VG) || (VG && !PG && LOSS == LOSS_MSE));                      \
+        constexpr bool COOP_ = !P64_ && TRI && PG && !VG;                                                             \
+        if (WIDE_ && p.Sout <= PREFIX_STRIDE && p.Sout > BwdGeo::SEG) {                                               \
+            auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, true, WIDE_>;                                     \
+            cudaError_t e = ensure_smem(k, smem, WIDE_CTAS * 4 / (threads / 32));                                     \
+            if (e != cudaSuccess) return e;                                                                           \
+            k<<<grid, threads, smem, st>>>(p);                                                                        \
+            return cudaGetLastError();                                                                                \
+        }                                                                                                             \
+        if (!P64_ && p.Sout <= PREFIX_STRIDE) {                                                                       \
+            auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, true>;                                            \
+            cudaError_t e = ensure_smem(k, smem, ((VG) ? 16 : 20) / (threads / 32));                                  \
+            if (e != cudaSuccess) return e;                                                                           \
+            k<<<grid, threads, smem, st>>>(p);                                                                        \
+            return cudaGetLastError();                                                                                \
+        }                                                                                                             \
         if (render_bwd_is_coop(p.Sout, p.total_rays, S_, P64_, PG, VG)) { /* rays of 2..4 passes (config 5: 4): one ray per CTA, no pre-pass */ \
-            auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, false, (TRI && PG && !VG && !P64_), false, (TRI && PG && !VG && !P64_)>; \
+            auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, false, COOP_, COOP_>;                             \
             const int nw_ = (p.Sout + PREFIX_STRIDE - 1) / PREFIX_STRIDE;       /* 2, 3 or 4 warps: 8, 5 or 4 CTAs per SM */ \
             const size_t smem_ = ((size_t)p.att_slots_padded + (size_t)nw_ * BWD_SMEM_PER_WARP + CoopXch::FLOATS) * sizeof(float); \
-            cudaError_t e = ensure_smem(k, smem_, 16 / nw_);                    \
-            if (e != cudaSuccess) return e;                                     \
-            k<<<(unsigned)p.total_rays, nw_ * 32, smem_, st>>>(p);              \
-            return cudaGetLastError();                                          \
-        }                                                                       \
-        if (DIFFUS_WIDE_MULTIPASS && !P64_ && TRI && PG && !VG && p.Sout > PREFIX_STRIDE) { /* long rays (config 5) */ \
-            auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, false, (DIFFUS_WIDE_MULTIPASS && TRI && PG && !VG)>; \
-            cudaError_t e = ensure_smem(k, smem);                               \
-            if (e != cudaSuccess) return e;                                     \
-            k<<<grid, threads, smem, st>>>(p);                                  \
-            return cudaGetLastError();                                          \
-        }                                                                       \
-        auto k = render_bwd_kernel<S_, L_, P64_, PG, VG, LOSS, false>;          \
-        cudaError_t e = ensure_smem(k, smem, DIFFUS_CARVEOUT ? 16 / (threads / 32) : 0); \
-        if (e != cudaSuccess) return e;                                         \
-        k<<<grid, threads, smem, st>>>(p);                                      \
-        return cudaGetLastError();                                              \
+            cudaError_t e = ensure_smem(k, smem_, 16 / nw_);                                                          \
+            if (e != cudaSuccess) return e;                                                                           \
+            k<<<(unsigned)p.total_rays, nw_ * 32, smem_, st>>>(p);                                                    \
+            return cudaGetLastError();                                                                                \
+        }                                                                                                             \
+        auto k = render_bwd_kernel<S_, L_, P64_, PG, VG, LOSS, false>;                                                \
+        cudaError_t e = ensure_smem(k, smem, 16 / (threads / 32));                                                    \
+        if (e != cudaSuccess) return e;                                                                               \
+        k<<<grid, threads, smem, st>>>(p);                                                                            \
+        return cudaGetLastError();                                                                                    \
     }
     if (!TRI) pg = false;                      // no pose gradient exists (round+long cuts the graph)
     if (pg && vg) DIFFUS_BWD_GO(TRI, true)
