@@ -127,6 +127,7 @@ SIGNATURES = {
     "diffus_ssim_loss_backward": (_i32, [_vp, _vp, _i32, _i32, _i32, _f32, _i32, _vp, _vp, _vp, _i64, _vp]),
     "diffus_quad_elems": (_i64, [_P(_i32 * 3)]),
     "diffus_volume_to_quads": (_i32, [_vp, _P(_i32 * 3), _vp, _vp]),
+    "diffus_volume_gaussian_blur": (_i32, [_vp, _P(_i32 * 3), _f32, _f32, _vp, _vp, _vp]),
 }
 
 _lib = None

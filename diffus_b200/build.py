@@ -22,7 +22,7 @@ SOURCES = [("render_kernels.cu", ["-DDIFFUS_LAYOUT_SLICE=1"], "render_kernels_br
            ("mlp_pwl_kernels.cu", [], "mlp_pwl_kernels.o"),
            ("splat_kernels.cu", [], "splat_kernels.o"), ("preprocess_kernels.cu", [], "preprocess_kernels.o"),
            ("train_kernels.cu", [], "train_kernels.o"), ("loss_kernels.cu", [], "loss_kernels.o"),
-           ("gn_kernels.cu", [], "gn_kernels.o")]
+           ("gn_kernels.cu", [], "gn_kernels.o"), ("smooth_kernels.cu", [], "smooth_kernels.o")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--threads", "2"]
 

@@ -1,5 +1,6 @@
 // extern "C" entry points of libdiffus_b200.so (see include/diffus_b200.h).
 // Argument validation and parameter packing only; kernels live in the other translation units.
+#include <cmath>
 #include <mutex>
 #include <unordered_map>
 #include <unordered_set>
@@ -640,6 +641,25 @@ int32_t diffus_volume_to_quads(const float* linear, const int32_t dim[3], float*
     if (dim[0] < 1 || dim[1] < 1 || dim[2] < 1) return DIFFUS_E_SHAPE;
     if ((uintptr_t)quads & 15) return DIFFUS_E_UNSUPPORTED;
     return cuda_rc(launch_to_quads(linear, dim, quads, (cudaStream_t)stream));
+}
+
+static bool overlap(const float* a, const float* b, int64_t n) {
+    const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b, bytes = (uintptr_t)n * sizeof(float);
+    return x < y + bytes && y < x + bytes;
+}
+
+int32_t diffus_volume_gaussian_blur(const float* src, const int32_t dim[3], float sigma, float truncate, float* dst, float* scratch,
+                                    void* stream) {
+    if (!src || !dim || !dst || !scratch) return DIFFUS_E_NULL;
+    if (dim[0] < 1 || dim[1] < 1 || dim[2] < 1) return DIFFUS_E_SHAPE;
+    if (!std::isfinite(sigma) || sigma < 0.f || !std::isfinite(truncate) || truncate <= 0.f) return DIFFUS_E_SHAPE;
+    if ((double)dim[0] * dim[1] * dim[2] >= (double)((int64_t)1 << 60)) return DIFFUS_E_UNSUPPORTED;   // int64 byte offsets
+    const int64_t n = (int64_t)dim[0] * dim[1] * dim[2];
+    if (overlap(src, dst, n) || overlap(src, scratch, n) || overlap(dst, scratch, n)) return DIFFUS_E_SHAPE;
+    // scipy: an axis with sigma <= 1e-15 is skipped; else radius = int(truncate * sigma + 0.5)
+    const double rr = (double)sigma <= 1e-15 ? 0.0 : (double)truncate * (double)sigma + 0.5;
+    if (rr >= BLUR_MAX_RADIUS + 1) return DIFFUS_E_UNSUPPORTED;
+    return cuda_rc(launch_gaussian_blur(src, dim, sigma, (int)rr, dst, scratch, (cudaStream_t)stream));
 }
 
 // The layered array: width = dim[2] (p2, fastest), height = dim[1], layers = dim[0].

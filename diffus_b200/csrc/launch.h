@@ -133,6 +133,12 @@ cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, const in
 cudaError_t launch_render_gn(const RenderParams& p, int layout, const float* med_tan, float* partial, float* loss, float* jtr,
                              float* jtj, cudaStream_t st);
 
+// smooth_kernels.cu: scipy.ndimage.gaussian_filter(mode='nearest') of a (D,H,W) float32 volume in three separable passes,
+// radius r = int(truncate sigma + 0.5) <= BLUR_MAX_RADIUS (r = 0: a copy); dst and scratch hold D*H*W floats each
+constexpr int BLUR_MAX_RADIUS = 64;
+cudaError_t launch_gaussian_blur(const float* src, const int32_t dim[3], float sigma, int r, float* dst, float* scratch,
+                                 cudaStream_t st);
+
 // splat_kernels.cu
 int64_t splat_workspace_bytes(int H, int W);
 cudaError_t launch_splat_fwd(const float* c0, const float* c1, const float* c2, const float* val, int64_t n, int H, int W,

@@ -849,6 +849,23 @@ def to_quads(volume: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def gaussian_blur_volume(volume: torch.Tensor, sigma: float, truncate: float = 4.0) -> torch.Tensor:
+    """``scipy.ndimage.gaussian_filter(volume, sigma, mode='nearest', truncate=truncate)`` of a (D,H,W) CUDA volume, computed in
+    float32 (three separable passes); a new (D,H,W) float32 tensor.  Not differentiable."""
+    dev = _require_cuda(volume)
+    if volume.dim() != 3:
+        raise _lib.DiffusError("volume must be (D,H,W)")
+    v = volume.detach().contiguous().float()
+    dim = (C.c_int32 * 3)(*v.shape)
+    with _on_device(dev):
+        out = torch.empty_like(v)
+        scratch = torch.empty_like(v)
+        _lib.check(_lib.load().diffus_volume_gaussian_blur(v.data_ptr(), C.byref(dim), float(sigma), float(truncate), out.data_ptr(),
+                                                           scratch.data_ptr(), _stream(dev)), "diffus_volume_gaussian_blur")
+        _count(3 if sigma > 0 else 0)
+    return out
+
+
 def from_bricks(bricks: torch.Tensor, dims) -> torch.Tensor:
     dev = _require_cuda(bricks)
     lib = _lib.load()

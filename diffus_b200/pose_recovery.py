@@ -8,9 +8,12 @@ the CPU).
 """
 from __future__ import annotations
 
+import math
+import numbers
+
 import torch
 
-from .renderer import PreparedVolume
+from .renderer import PreparedVolume, smooth_volume
 
 
 def _rotate(x: torch.Tensor, w: torch.Tensor) -> torch.Tensor:
@@ -78,3 +81,51 @@ def recover_poses(volume, targets: torch.Tensor, sources: torch.Tensor, median: 
         step()
         history[i + 1].copy_(step.loss)
     return (step.sources.clone(), step.median.clone(), step.hint.clone()), history
+
+
+def _schedule(sigmas, iterations):
+    """Validated ``(sigmas, iterations)`` lists of one coarse-to-fine schedule (host only)."""
+    sig = [float(s) for s in sigmas]
+    if not sig or not all(math.isfinite(s) and s >= 0.0 for s in sig):
+        raise ValueError(f"sigmas must be a non-empty sequence of finite values >= 0, got {tuple(sigmas)!r}")
+    its = [iterations] * len(sig) if isinstance(iterations, numbers.Integral) else list(iterations)
+    if len(its) != len(sig):
+        raise ValueError(f"iterations must be an int or one per level ({len(sig)}), got {len(its)}")
+    if not all(isinstance(k, numbers.Integral) and not isinstance(k, bool) and k >= 0 for k in its):
+        raise ValueError(f"iterations must be non-negative ints, got {its!r}")
+    return sig, [int(k) for k in its]
+
+
+def recover_poses_coarse_to_fine(volume, targets: torch.Tensor, sources: torch.Tensor, median: torch.Tensor, hint: torch.Tensor,
+                                 opening_angle: float, n_rays: int, num_samples: int, attenuation_coeff: float = 0.5, start=0, *,
+                                 sigmas=(4.0, 2.0, 1.0, 0.0), iterations=10, damping: float = 1e-3, layout=None):
+    """Levenberg-Marquardt pose recovery from a blurred volume to the sharp one (a Gaussian scale space).
+
+    On a volume with sharp tissue boundaries the frame depends on the pose through one-voxel gradient cells, so a Gauss-Newton
+    step is only valid within about a voxel.  Level l renders from ``smooth_volume(volume, sigmas[l])`` instead, where the
+    basin of the true pose is about sigma wide, and starts from the previous level's poses; the target frames stay as they
+    are.  A sigma of 0 uses ``volume`` as given.  Each level is :func:`recover_poses` with ``iterations`` (an int, or one per
+    level) and a fresh ``damping``; its first history row is the incoming poses' loss on that level's own volume, so no
+    accept / reject compares losses across volumes.  ``layout`` of the blurred levels' :class:`PreparedVolume` defaults to the
+    caller's layout, else ``'texture'``; each level's copy is released before the next is built.
+
+    Returns ``((sources, median, hint), histories)``: one (iterations_l + 1, P) loss history per level.
+    """
+    sig, its = _schedule(sigmas, iterations)
+    if layout is None:
+        layout = volume.layout if isinstance(volume, PreparedVolume) else "texture"
+    base = volume.volume if isinstance(volume, PreparedVolume) else volume
+    poses, histories = (sources, median, hint), []
+    for sigma, k in zip(sig, its):
+        if sigma == 0.0:
+            level = volume
+        else:
+            with torch.no_grad():
+                level = PreparedVolume(smooth_volume(base, sigma), layout)
+        poses, hist = recover_poses(level, targets, *poses, opening_angle, n_rays, num_samples, attenuation_coeff, start,
+                                    iterations=k, damping=damping)
+        histories.append(hist)
+        if level is not volume:
+            level.close()
+        del level
+    return poses, histories

@@ -82,6 +82,14 @@ class PreparedVolume:
         self._texture = None
         self.refresh()
 
+    def close(self) -> None:
+        """Release the packed copy now; the next use rebuilds it.  The TEXTURE layout's CUDA array lives outside torch's
+        allocator and stays allocated until closed, so a caller that builds prepared volumes in a loop closes each one."""
+        if self._texture is not None:
+            self._texture.close()
+            self._texture = None
+        self._bricks, self._version = None, None
+
     def refresh(self) -> "PreparedVolume":
         """Rebuild the packed copy (done automatically when the volume tensor was modified in place)."""
         if self.layout == "texture":
@@ -190,6 +198,20 @@ def render_gauss_newton(volume, sources: torch.Tensor, directions: torch.Tensor,
         tgt = tgt.unsqueeze(0)
     return ops.render_gauss_newton_impl(vol32, bricks, list(volume.shape), src.detach().contiguous(), dirs.detach().contiguous(),
                                         tgt, int(num_samples), _resolve_start(start, num_samples), float(attenuation_coeff))
+
+
+def smooth_volume(volume, sigma: float, truncate: float = 4.0) -> torch.Tensor:
+    """Isotropic Gaussian smoothing of a (D,H,W) volume on the device: ``scipy.ndimage.gaussian_filter(volume, sigma,
+    mode='nearest', truncate=truncate)`` computed in float32, radius ``int(truncate * sigma + 0.5)`` <= 64.  Beyond a face the
+    edge voxel repeats (the renderer's border rule).  ``sigma = 0`` returns an exact copy.
+
+    ``volume`` is a CUDA tensor or a :class:`PreparedVolume` (its ``volume`` is smoothed); returns a new float32 tensor.  Not
+    differentiable: a volume that requires grad, with grad enabled, raises rather than being silently detached.
+    """
+    vol = volume.volume if isinstance(volume, PreparedVolume) else volume
+    if torch.is_grad_enabled() and vol.requires_grad:
+        raise DiffusError("smooth_volume is not differentiable; call it under torch.no_grad() or on a detached volume")
+    return ops.gaussian_blur_volume(vol, sigma, truncate)
 
 
 def _resolve_start(start, num_samples: int) -> int:

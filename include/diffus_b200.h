@@ -345,6 +345,16 @@ int32_t diffus_bricks_to_volume(const float* bricks, const int32_t dim[3], float
 int64_t diffus_quad_elems(const int32_t dim[3]);
 int32_t diffus_volume_to_quads(const float* linear, const int32_t dim[3], float* quads, void* stream);
 
+/* Isotropic Gaussian smoothing of a (D,H,W) float32 volume: scipy.ndimage.gaussian_filter(src, sigma, mode='nearest',
+ * truncate=truncate) -- weights exp(-x^2 / (2 sigma^2)) over x = -r..r, r = int(truncate * sigma + 0.5), normalised to sum 1
+ * in float64 and rounded to float32; taps beyond a face repeat the edge voxel (the renderer's border rule), also when r
+ * exceeds a dimension.  sigma <= 1e-15 (scipy skips the axes) or r = 0 is an exact copy.  Three separable passes in fp32,
+ * p2 src -> dst, p1 dst -> scratch, p0 scratch -> dst; bit-identical from run to run.  dst and scratch hold D*H*W floats
+ * each and may not overlap src or each other.  Returns DIFFUS_E_SHAPE for sigma < 0, truncate <= 0 or either not finite,
+ * DIFFUS_E_UNSUPPORTED for r > 64.  The scale space of coarse-to-fine pose recovery. */
+int32_t diffus_volume_gaussian_blur(const float* src, const int32_t dim[3], float sigma, float truncate, float* dst,
+                                    float* scratch, void* stream);
+
 /* TEXTURE layout.  The ONLY entry points of this library that allocate and free device memory (a CUDA array of
  * dim[0] layers x dim[1] x dim[2] float32 texels and a texture object): create once per volume, update after the
  * LINEAR tensor changed (one device-to-device copy enqueued on `stream`), destroy when done.  `*texture_object` is what
