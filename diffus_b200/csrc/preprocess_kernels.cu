@@ -54,9 +54,12 @@ __global__ void zscore_kernel(const float* __restrict__ v, int64_t n, const ZSta
     const double cnt = (double)st->count;
     const double mean = st->sum / cnt;
     const double var = (st->sumsq - cnt * mean * mean) / (cnt - 1.0);      // unbiased, like torch.std
-    const float meanf = (float)mean, scale = 1.f / ((float)sqrt(fmax(var, 0.0)) + 1e-8f);
+    // Rounding can take the one-pass variance just below 0: clamp it, but let a NaN through (one masked voxel gives 0 / 0,
+    // torch's std of a single value).  The mean is subtracted in double: rounded to float32 it would be off by up to
+    // ulp(mean) / 2, 1e-4 of the std when mean / std is 1e4 (a bright, low-contrast MRI).
+    const double scale = 1.0 / (sqrt(var < 0.0 ? 0.0 : var) + 1e-8);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-        out[i] = (v[i] - meanf) * scale;
+        out[i] = (float)(((double)v[i] - mean) * scale);
 }
 
 static unsigned grid_for(int64_t n) { return (unsigned)max((int64_t)1, min((int64_t)148 * 16, (n + 255) / 256)); }

@@ -399,7 +399,7 @@ def compute_impedance_volume(volume, params, threshold=50):
 # ----------------------------------------------------------------------------------------
 
 
-def splat(x, y, z, intensities, H=256, W=256, sigma=2.0, last_wins=True):
+def splat(x, y, z, intensities, H=256, W=256, sigma=2.0, last_wins=True, dtype=torch.float32):
     """``differentiable_splat`` (``src/renderer.py:694-737``).
 
     Pick the two axes of largest coordinate variance (descending); round+clamp to pixels;
@@ -411,6 +411,9 @@ def splat(x, y, z, intensities, H=256, W=256, sigma=2.0, last_wins=True):
     both win, depending on thread chunking).  ``last_wins=True`` pins the sequential
     reading -- the sample with the highest flat index survives -- while keeping torch's
     backward, in which every duplicate receives its pixel's gradient.
+
+    ``dtype`` is the precision of the image arithmetic (scatter, blur, ratio): float32 as in the reference, float64 for a
+    reference value.  The pixel indices are rounded from float32 coordinates either way, as in the reference.
     """
     import torch.nn.functional as F
     coords = [x, y, z]
@@ -418,8 +421,8 @@ def splat(x, y, z, intensities, H=256, W=256, sigma=2.0, last_wins=True):
     a0, a1 = sorted(range(3), key=lambda i: -variances[i])[:2]
     c0 = coords[a0].to(torch.float32)
     c1 = coords[a1].to(torch.float32)
-    val = intensities.to(torch.float32)
-    img = torch.zeros((1, 1, H, W))
+    val = intensities.to(dtype)
+    img = torch.zeros((1, 1, H, W), dtype=dtype)
     wgt = torch.zeros_like(img)
     i0 = torch.clamp(c0.round().long(), 0, W - 1)
     i1 = torch.clamp(c1.round().long(), 0, H - 1)
@@ -432,7 +435,7 @@ def splat(x, y, z, intensities, H=256, W=256, sigma=2.0, last_wins=True):
     img[0, 0, i1, i0] += val
     wgt[0, 0, i1, i0] += 1
     size = int(6 * sigma) | 1
-    t = torch.arange(size) - size // 2
+    t = (torch.arange(size) - size // 2).to(dtype)
     k1 = torch.exp(-0.5 * (t / sigma) ** 2)
     k1 = k1 / k1.sum()
     k2 = (k1[:, None] @ k1[None, :])[None, None]
