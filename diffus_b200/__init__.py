@@ -7,13 +7,13 @@ first op call loads ``libdiffus_b200.so`` and fails loudly if it has not been bu
 """
 from .cone import generate_cone_directions
 from .impedance import ImpedanceEstimator
-from .ops import fan_directions
+from .ops import fan_directions, probe_rays
 from .renderer import (PreparedVolume, UltrasoundRenderer, compute_echo_traces, compute_gaussian_pulse, gaussian_pulse, custom_nearest_sampler, differentiable_splat,
                        propagate_full_rays_batched, render_frames, render_gauss_newton, render_mse_loss, rotate_around_apex,
                        smooth_volume)
-from .pose_recovery import apply_fan_twist, apply_pose_twist, recover_poses, recover_poses_coarse_to_fine
+from .pose_recovery import apply_fan_twist, apply_pose_twist, apply_probe_twist, recover_poses, recover_poses_coarse_to_fine
 
 __all__ = ["UltrasoundRenderer", "render_frames", "render_mse_loss", "render_gauss_newton", "PreparedVolume", "compute_echo_traces", "compute_gaussian_pulse", "gaussian_pulse",
            "propagate_full_rays_batched", "custom_nearest_sampler", "differentiable_splat", "rotate_around_apex", "generate_cone_directions",
            "fan_directions", "ImpedanceEstimator", "apply_pose_twist", "apply_fan_twist", "recover_poses", "smooth_volume",
-           "recover_poses_coarse_to_fine"]
+           "recover_poses_coarse_to_fine", "probe_rays", "apply_probe_twist"]

@@ -14,7 +14,8 @@ ABI_VERSION = 1
 
 SAMPLER_NEAREST, SAMPLER_TRILINEAR = 0, 1
 LAYOUT_LINEAR, LAYOUT_BRICK, LAYOUT_QUAD, LAYOUT_TEXTURE = 0, 1, 2, 3
-POSE_F32, POSE_F64 = 0, 1
+POSE_F32, POSE_F64, POSE_F32_PER_RAY = 0, 1, 2
+PROBE_CONVEX, PROBE_LINEAR = 0, 1
 MLP_NPARAMS = 1153
 
 
@@ -108,6 +109,8 @@ SIGNATURES = {
     "diffus_bricks_to_volume": (_i32, [_vp, _P(_i32 * 3), _vp, _vp]),
     "diffus_fan_directions": (_i32, [_vp, _vp, _i64, _i64, C.c_double, _vp, _vp]),
     "diffus_fan_directions_backward": (_i32, [_vp, _vp, _vp, _i64, _i64, C.c_double, _vp, _vp, _vp]),
+    "diffus_probe_rays": (_i32, [_i32, _vp, _vp, _vp, _i64, _i64, _f64, _f64, _f64, _vp, _vp, _vp]),
+    "diffus_probe_rays_backward": (_i32, [_i32, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _f64, _f64, _f64, _vp, _vp, _vp, _vp]),
     "diffus_gather_probe": (_i32, [_vp, _i64, _i32, _i64, C.c_uint32, _vp, _vp]),
     "diffus_volume_texture_create": (_i32, [_vp, _P(_i32 * 3), _P(C.c_uint64), _P(C.c_uint64), _vp]),
     "diffus_volume_texture_update": (_i32, [C.c_uint64, _vp, _P(_i32 * 3), _vp]),

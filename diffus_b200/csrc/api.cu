@@ -52,13 +52,16 @@ int32_t check_volume(const DiffusVolume& v) {
     return DIFFUS_OK;
 }
 
+bool pose_dtype_ok(int32_t t) { return t == DIFFUS_POSE_F32 || t == DIFFUS_POSE_F64 || t == DIFFUS_POSE_F32_PER_RAY; }
+bool per_ray(const DiffusRenderArgs* a) { return a->pose_dtype == DIFFUS_POSE_F32_PER_RAY; }
+
 int32_t check_render(const DiffusRenderArgs* a, bool need_frame) {
     if (!a) return DIFFUS_E_NULL;
     int32_t e = check_volume(a->volume);
     if (e) return e;
     if (!a->sources || !a->directions) return DIFFUS_E_NULL;
     if (need_frame && !a->frame) return DIFFUS_E_NULL;
-    if (a->pose_dtype != DIFFUS_POSE_F32 && a->pose_dtype != DIFFUS_POSE_F64) return DIFFUS_E_ENUM;
+    if (!pose_dtype_ok(a->pose_dtype)) return DIFFUS_E_ENUM;
     if (a->sampler != DIFFUS_SAMPLER_NEAREST && a->sampler != DIFFUS_SAMPLER_TRILINEAR) return DIFFUS_E_ENUM;
     if (a->n_poses < 1 || a->n_rays < 1 || a->n_samples < 2) return DIFFUS_E_SHAPE;
     if (a->n_samples > 32768) return DIFFUS_E_UNSUPPORTED;           // attenuation table lives in shared memory
@@ -96,6 +99,8 @@ RenderParams pack(const DiffusRenderArgs* a) {
     p.sources = a->sources;
     p.directions = a->directions;
     p.dir_pose_stride = a->dir_pose_stride;
+    p.src_pose_stride = per_ray(a) ? a->n_rays * 3 : 3;
+    p.src_ray_stride = per_ray(a) ? 3 : 0;
     p.product_f32 = a->product_f32;
     p.n_poses = a->n_poses;
     p.n_rays = a->n_rays;
@@ -134,7 +139,8 @@ FwdWorkspace fwd_workspace(const DiffusRenderArgs* a, void* base) {
     return w;
 }
 
-// backward workspace: [fwd workspace | source partials (P*R*3) | direction scratch (P*R*3) | first_rbar (P*R)]
+// backward workspace: [fwd workspace | source partials (P*R*3) | direction scratch (P*R*3) | first_rbar (P*R)]; with per-ray
+// origins the kernels write grad_sources itself, so there are no source partials when it is given
 struct BwdWorkspace {
     FwdWorkspace fwd;
     float* src_partial;
@@ -152,8 +158,12 @@ BwdWorkspace bwd_workspace(const DiffusRenderBwdArgs* b, void* base) {
     int64_t rays = a->n_poses * a->n_rays;
     bool pose_grad = a->sampler == DIFFUS_SAMPLER_TRILINEAR && (b->grad_sources || b->grad_directions);
     if (pose_grad) {
-        w.src_partial = (float*)((char*)base + off);
-        off += align_up(rays * 12, 256);
+        if (per_ray(a) && b->grad_sources) {
+            w.src_partial = b->grad_sources;
+        } else {
+            w.src_partial = (float*)((char*)base + off);
+            off += align_up(rays * 12, 256);
+        }
         if (!b->grad_directions) {
             w.dir_scratch = (float*)((char*)base + off);
             off += align_up(rays * 12, 256);
@@ -175,10 +185,11 @@ BwdWorkspace bwd_workspace(const DiffusRenderBwdArgs* b, void* base) {
 
 int32_t cuda_rc(cudaError_t e) { return e == cudaSuccess ? DIFFUS_OK : (int32_t)e; }
 
-// Gauss-Newton workspace: [fwd workspace | median tangent (P*6) | per-ray partials (P*R*32)]
+// Gauss-Newton workspace: [fwd workspace | median tangent (P*6) | per-ray partials (P*R*32) | pivots (P*3 doubles, per-ray origins)]
 struct GnWorkspace {
     FwdWorkspace fwd;
     float* med_tan;
+    double* pivot;
     float* partial;
     int64_t bytes;
 };
@@ -193,6 +204,10 @@ GnWorkspace gn_workspace(const DiffusGaussNewtonArgs* g, void* base) {
     }
     w.partial = (float*)((char*)base + off);
     off += align_up(a->n_poses * a->n_rays * 128, 256);
+    if (per_ray(a)) {
+        w.pivot = (double*)((char*)base + off);
+        off += align_up(a->n_poses * 24, 256);
+    }
     w.bytes = off;
     return w;
 }
@@ -245,7 +260,7 @@ int64_t diffus_render_bwd_workspace_bytes(const DiffusRenderBwdArgs* b) {
 int32_t diffus_render_bwd_needs_prefix(const DiffusRenderBwdArgs* b) {
     if (!b) return DIFFUS_E_NULL;
     const DiffusRenderArgs* a = &b->fwd;
-    if (a->pose_dtype != DIFFUS_POSE_F32 && a->pose_dtype != DIFFUS_POSE_F64) return DIFFUS_E_ENUM;
+    if (!pose_dtype_ok(a->pose_dtype)) return DIFFUS_E_ENUM;
     if (a->sampler != DIFFUS_SAMPLER_NEAREST && a->sampler != DIFFUS_SAMPLER_TRILINEAR) return DIFFUS_E_ENUM;
     if (a->n_poses < 1 || a->n_rays < 1 || a->n_samples < 2 || a->start < 0 || a->start > a->n_samples - 2) return DIFFUS_E_SHAPE;
     const int sout = (int)(a->n_samples - a->start);
@@ -294,12 +309,14 @@ int32_t diffus_render_backward(const DiffusRenderBwdArgs* b, void* stream) {
         ce = launch_median_backward(p, a->sampler, a->volume.layout, pose64, w.fwd.tie_count, pose_grad, vol_grad, st);
         if (ce != cudaSuccess) return (int32_t)ce;
     }
-    if (pose_grad && b->grad_sources && w.loss_partial && reduce_rays_and_sum_fits(a->n_poses * a->n_rays)) {
+    // per-ray origins: the kernels wrote grad_sources themselves, there is nothing to fold over the rays
+    const bool fold_sources = pose_grad && b->grad_sources && !per_ray(a);
+    if (fold_sources && w.loss_partial && reduce_rays_and_sum_fits(a->n_poses * a->n_rays)) {
         // the fused pose step: both reductions in one launch
         return cuda_rc(launch_reduce_rays_and_sum(w.src_partial, a->n_poses, a->n_rays, b->grad_sources, w.loss_partial,
                                                   a->n_poses * a->n_rays, b->loss_scale, b->loss, st));
     }
-    if (pose_grad && b->grad_sources) {
+    if (fold_sources) {
         ce = launch_reduce_rays(w.src_partial, a->n_poses, a->n_rays, b->grad_sources, st);
         if (ce != cudaSuccess) return (int32_t)ce;
     }
@@ -321,7 +338,7 @@ int32_t diffus_render_gauss_newton(const DiffusGaussNewtonArgs* g, void* stream)
     int32_t e = check_render(a, false);
     if (e) return e;
     if (!g->target || !g->loss || !g->jtr || !g->jtj) return DIFFUS_E_NULL;
-    if (a->sampler != DIFFUS_SAMPLER_TRILINEAR || a->pose_dtype != DIFFUS_POSE_F32) return DIFFUS_E_UNSUPPORTED;
+    if (a->sampler != DIFFUS_SAMPLER_TRILINEAR || a->pose_dtype == DIFFUS_POSE_F64) return DIFFUS_E_UNSUPPORTED;
     GnWorkspace w = gn_workspace(g, g->workspace);
     if (!g->workspace || g->workspace_bytes < w.bytes) return DIFFUS_E_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
@@ -330,14 +347,18 @@ int32_t diffus_render_gauss_newton(const DiffusGaussNewtonArgs* g, void* stream)
     p.seg_prefix = nullptr;
     p.target = g->target;
     cudaError_t ce;
+    if (w.pivot) {
+        ce = launch_gn_pivot((const float*)a->sources, a->n_poses, a->n_rays, w.pivot, st);
+        if (ce != cudaSuccess) return (int32_t)ce;
+    }
     if (a->start > 0) {
         ce = launch_first_refl_median(p, a->sampler, a->volume.layout, 0, w.fwd.median, w.fwd.tie_count, st);
         if (ce != cudaSuccess) return (int32_t)ce;
         p.median = w.fwd.median;
-        ce = launch_gn_median_tangent(p, a->volume.layout, w.fwd.tie_count, w.med_tan, st);
+        ce = launch_gn_median_tangent(p, a->volume.layout, w.fwd.tie_count, w.pivot, w.med_tan, st);
         if (ce != cudaSuccess) return (int32_t)ce;
     }
-    return cuda_rc(launch_render_gn(p, a->volume.layout, w.med_tan, w.partial, g->loss, g->jtr, g->jtj, st));
+    return cuda_rc(launch_render_gn(p, a->volume.layout, w.med_tan, w.pivot, w.partial, g->loss, g->jtr, g->jtj, st));
 }
 
 int32_t diffus_ray_indices(const DiffusRenderArgs* a, int64_t* x, int64_t* y, int64_t* z, void* stream) {
@@ -380,19 +401,20 @@ int32_t diffus_trace_values_backward(const DiffusRenderArgs* a, const float* gra
     const bool pose_grad = a->sampler == DIFFUS_SAMPLER_TRILINEAR && (grad_sources || grad_directions);
     if (!pose_grad && !grad_volume) return DIFFUS_OK;
     if (pose_grad && (!grad_sources || !grad_directions)) return DIFFUS_E_NULL;
-    const int64_t need = pose_grad ? align_up(a->n_poses * a->n_rays * 12, 256) : 0;
+    // per-ray origins: the kernel writes grad_sources itself
+    const int64_t need = pose_grad && !per_ray(a) ? align_up(a->n_poses * a->n_rays * 12, 256) : 0;
     if (need > 0 && (!workspace || workspace_bytes < need)) return DIFFUS_E_WORKSPACE;
     RenderParams p = pack(a);
     p.start = 0;
     p.Sout = p.S;
     p.grad_volume = grad_volume;
-    p.grad_src_partial = (float*)workspace;
+    p.grad_src_partial = per_ray(a) ? grad_sources : (float*)workspace;
     p.grad_dir = grad_directions;
     cudaStream_t st = (cudaStream_t)stream;
     cudaError_t ce = launch_trace_values_bwd(p, a->sampler, a->volume.layout, a->pose_dtype == DIFFUS_POSE_F64, grad_values,
                                              pose_grad, grad_volume != nullptr, st);
     if (ce != cudaSuccess) return (int32_t)ce;
-    if (pose_grad) return cuda_rc(launch_reduce_rays(p.grad_src_partial, a->n_poses, a->n_rays, grad_sources, st));
+    if (pose_grad && !per_ray(a)) return cuda_rc(launch_reduce_rays(p.grad_src_partial, a->n_poses, a->n_rays, grad_sources, st));
     return DIFFUS_OK;
 }
 
@@ -746,6 +768,38 @@ int32_t diffus_fan_directions_backward(const float* median, const float* hint, c
     if (n_poses < 1 || n_rays < 1 || n_poses >= ((int64_t)1 << 31)) return DIFFUS_E_SHAPE;
     return cuda_rc(launch_fan_directions_bwd(median, hint, grad_directions, n_poses, n_rays, opening_angle, grad_median, grad_hint,
                                              (cudaStream_t)stream));
+}
+
+static int32_t check_probe(int32_t kind, int64_t n_poses, int64_t n_rays, double opening_angle, double radius, double width) {
+    if (n_poses < 1 || n_rays < 1 || n_poses >= ((int64_t)1 << 31) || n_poses * n_rays >= ((int64_t)1 << 31)) return DIFFUS_E_SHAPE;
+    if (kind == DIFFUS_PROBE_CONVEX) {
+        if (!std::isfinite(opening_angle) || !std::isfinite(radius) || radius < 0.0) return DIFFUS_E_SHAPE;
+    } else if (kind == DIFFUS_PROBE_LINEAR) {
+        if (!std::isfinite(width) || width <= 0.0) return DIFFUS_E_SHAPE;
+    } else {
+        return DIFFUS_E_ENUM;
+    }
+    return DIFFUS_OK;
+}
+
+int32_t diffus_probe_rays(int32_t kind, const float* centre, const float* median, const float* hint, int64_t n_poses, int64_t n_rays,
+                          double opening_angle, double radius, double width, float* origins, float* directions, void* stream) {
+    if (!centre || !median || !hint || !origins || !directions) return DIFFUS_E_NULL;
+    int32_t e = check_probe(kind, n_poses, n_rays, opening_angle, radius, width);
+    if (e) return e;
+    return cuda_rc(launch_probe_rays(kind, centre, median, hint, n_poses, n_rays, opening_angle, radius, width, origins, directions,
+                                     (cudaStream_t)stream));
+}
+
+int32_t diffus_probe_rays_backward(int32_t kind, const float* centre, const float* median, const float* hint, const float* grad_origins,
+                                   const float* grad_directions, int64_t n_poses, int64_t n_rays, double opening_angle, double radius,
+                                   double width, float* grad_centre, float* grad_median, float* grad_hint, void* stream) {
+    if (!centre || !median || !hint || !grad_origins || !grad_directions || !grad_centre || !grad_median || !grad_hint)
+        return DIFFUS_E_NULL;
+    int32_t e = check_probe(kind, n_poses, n_rays, opening_angle, radius, width);
+    if (e) return e;
+    return cuda_rc(launch_probe_rays_bwd(kind, centre, median, hint, grad_origins, grad_directions, n_poses, n_rays, opening_angle,
+                                         radius, width, grad_centre, grad_median, grad_hint, (cudaStream_t)stream));
 }
 
 }  // extern "C"

@@ -33,7 +33,7 @@ __global__ void first_refl_median_kernel(const RenderParams p, float* __restrict
     __syncthreads();
     for (int ray = threadIdx.x; ray < R; ray += blockDim.x) {
         RaySetup<POSE64> rs;
-        rs.load(p.sources, p.directions, pose, ray, p.n_rays, p.dir_pose_stride, p.product_f32);
+        rs.load(p.sources, p.directions, pose, ray, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, p.product_f32);
         float g[3];
         int k = p.start;
         float z0 = sample_volume<SAMPLER, LAYOUT, false>(p.vol, rs.coord(0, k), rs.coord(1, k), rs.coord(2, k), g);
@@ -106,7 +106,7 @@ __global__ void median_backward_kernel(const RenderParams p, const int32_t* __re
     for (int64_t m = lane; m < p.n_rays; m += 32) {
         const int64_t ray = pose * p.n_rays + m;
         RaySetup<POSE64> rs;
-        rs.load(p.sources, p.directions, pose, m, p.n_rays, p.dir_pose_stride, p.product_f32);
+        rs.load(p.sources, p.directions, pose, m, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, p.product_f32);
         float g0[3], g1[3];
         float z0 = sample_volume<SAMPLER, LAYOUT, POSE_GRAD>(p.vol, rs.coord(0, k), rs.coord(1, k), rs.coord(2, k), g0);
         float z1 = sample_volume<SAMPLER, LAYOUT, POSE_GRAD>(p.vol, rs.coord(0, k + 1), rs.coord(1, k + 1), rs.coord(2, k + 1), g1);
@@ -168,7 +168,7 @@ __global__ void ray_indices_kernel(const RenderParams p, int64_t* __restrict__ x
         int c = (int)(t - ray * p.Sout);
         int64_t pose = ray / p.n_rays;
         RaySetup<POSE64> rs;
-        rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.n_rays, p.dir_pose_stride, p.product_f32);
+        rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, p.product_f32);
         int k = p.start + c;
         x[t] = nearest_index(rs.coord(0, k), p.vol.D);
         y[t] = nearest_index(rs.coord(1, k), p.vol.H);
@@ -192,7 +192,7 @@ __global__ void trace_values_kernel(const RenderParams p, float* __restrict__ ou
         int k = (int)(t - ray * p.S);
         int64_t pose = ray / p.n_rays;
         RaySetup<POSE64> rs;
-        rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.n_rays, p.dir_pose_stride, p.product_f32);
+        rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, p.product_f32);
         float g[3];
         out[t] = sample_volume<SAMPLER, LAYOUT, false>(p.vol, rs.coord(0, k), rs.coord(1, k), rs.coord(2, k), g);
     }
@@ -241,7 +241,7 @@ __global__ void trace_values_bwd_kernel(const RenderParams p, const float* __res
     if (ray >= p.total_rays) return;
     const int64_t pose = ray / p.n_rays;
     RaySetup<POSE64> rs;
-    rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.n_rays, p.dir_pose_stride, p.product_f32);
+    rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, p.product_f32);
     float acc_s[3] = {0.f, 0.f, 0.f}, acc_d[3] = {0.f, 0.f, 0.f};
     for (int k = lane; k < p.S; k += 32) {
         float g = __ldg(gval + ray * (int64_t)p.S + k);
@@ -474,6 +474,30 @@ __device__ __forceinline__ double fan_angle(int64_t i, int64_t n_rays, double an
     return (i == n_rays - 1) ? hi : (double)i * ((hi - lo) / (double)(n_rays - 1)) + lo;
 }
 
+// d loss / d m^ and d loss / d u^ (as independent vectors) -> d loss / d median and d loss / d hint (3 floats each, overwritten)
+// through the normalisations and the Gram-Schmidt step of fan_frame
+__device__ __forceinline__ void fan_frame_bwd(const float* median, const float* hint, int64_t pose, const double gm[3],
+                                              const double gu[3], float* grad_median, float* grad_hint) {
+    const FanFrame f = fan_frame(median + pose * 3, hint + pose * 3);
+    // u^ = u / |u|
+    double gud = gu[0] * f.u[0] + gu[1] * f.u[1] + gu[2] * f.u[2], gv[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) gv[a] = (gu[a] - gud * f.u[a]) / f.nu;              // d loss / d u
+    // u = h - (h.m^) m^
+    const double gvm = gv[0] * f.m[0] + gv[1] * f.m[1] + gv[2] * f.m[2];
+    double gmt[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        const double h = (double)hint[pose * 3 + a];
+        grad_hint[pose * 3 + a] = (float)(gv[a] - gvm * f.m[a]);
+        gmt[a] = gm[a] - f.hm * gv[a] - gvm * h;                                        // total d loss / d m^
+    }
+    // m^ = m / |m|
+    const double gmd = gmt[0] * f.m[0] + gmt[1] * f.m[1] + gmt[2] * f.m[2];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) grad_median[pose * 3 + a] = (float)((gmt[a] - gmd * f.m[a]) / f.nm);
+}
+
 __global__ void fan_directions_kernel(const float* __restrict__ median, const float* __restrict__ hint, int64_t n_poses,
                                       int64_t n_rays, double angle, float* __restrict__ out) {
     const int64_t pose = blockIdx.x;
@@ -508,24 +532,7 @@ __global__ void fan_directions_bwd_kernel(const float* __restrict__ median, cons
             gu[a] += __shfl_xor_sync(FULL, gu[a], d);
         }
     if (lane != 0) return;
-    const FanFrame f = fan_frame(median + pose * 3, hint + pose * 3);
-    // u^ = u / |u|
-    double gud = gu[0] * f.u[0] + gu[1] * f.u[1] + gu[2] * f.u[2], gv[3];
-#pragma unroll
-    for (int a = 0; a < 3; ++a) gv[a] = (gu[a] - gud * f.u[a]) / f.nu;              // d loss / d u
-    // u = h - (h.m^) m^
-    const double gvm = gv[0] * f.m[0] + gv[1] * f.m[1] + gv[2] * f.m[2];
-    double gmt[3];
-#pragma unroll
-    for (int a = 0; a < 3; ++a) {
-        const double h = (double)hint[pose * 3 + a];
-        grad_hint[pose * 3 + a] = (float)(gv[a] - gvm * f.m[a]);
-        gmt[a] = gm[a] - f.hm * gv[a] - gvm * h;                                        // total d loss / d m^
-    }
-    // m^ = m / |m|
-    const double gmd = gmt[0] * f.m[0] + gmt[1] * f.m[1] + gmt[2] * f.m[2];
-#pragma unroll
-    for (int a = 0; a < 3; ++a) grad_median[pose * 3 + a] = (float)((gmt[a] - gmd * f.m[a]) / f.nm);
+    fan_frame_bwd(median, hint, pose, gm, gu, grad_median, grad_hint);
 }
 
 cudaError_t launch_fan_directions(const float* median, const float* hint, int64_t n_poses, int64_t n_rays, double angle,
@@ -538,6 +545,102 @@ cudaError_t launch_fan_directions_bwd(const float* median, const float* hint, co
                                       int64_t n_rays, double angle, float* grad_median, float* grad_hint, cudaStream_t st) {
     fan_directions_bwd_kernel<<<(unsigned)n_poses, 32, 0, st>>>(median, hint, grad_dirs, n_poses, n_rays, angle, grad_median,
                                                                 grad_hint);
+    return cudaGetLastError();
+}
+
+
+// ---------------------------------------------------------------------------------------
+// array probes from pose PARAMETERS (centre, median, hint; m^ and u^ as in the fan above), one origin per ray:
+//   convex (opening angle, radius rho >= 0): d_i = cos a_i m^ + sin a_i u^ exactly as fan_directions_kernel forms it, and
+//          origin_i = c + rho d_i on the arc, in double -- rho = 0 gives the sector probe's rays bit for bit;
+//   linear (width w > 0): d_i = m^ for every ray, origin_i = c + t_i u^ with t_i spread over [-w/2, w/2] by fan_angle's rule.
+// The backward maps d loss / d origins and d loss / d directions (P,R,3 each) to d loss / d centre, median and hint (P,3 each).
+// ---------------------------------------------------------------------------------------
+__global__ void probe_rays_kernel(int kind, const float* __restrict__ centre, const float* __restrict__ median,
+                                  const float* __restrict__ hint, int64_t n_rays, double angle, double radius, double width,
+                                  float* __restrict__ origins, float* __restrict__ dirs) {
+    const int64_t pose = blockIdx.x;
+    const FanFrame f = fan_frame(median + pose * 3, hint + pose * 3);
+    const double c[3] = {(double)centre[pose * 3], (double)centre[pose * 3 + 1], (double)centre[pose * 3 + 2]};
+    for (int64_t i = threadIdx.x; i < n_rays; i += blockDim.x) {
+        float* o = origins + (pose * n_rays + i) * 3;
+        float* d = dirs + (pose * n_rays + i) * 3;
+        if (kind == DIFFUS_PROBE_CONVEX) {
+            double sa, ca;
+            sincos(fan_angle(i, n_rays, angle), &sa, &ca);
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                const double w = ca * f.m[a] + sa * f.u[a];
+                d[a] = (float)w;
+                o[a] = (float)(c[a] + radius * w);
+            }
+        } else {
+            const double t = fan_angle(i, n_rays, width);
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                d[a] = (float)f.m[a];
+                o[a] = (float)(c[a] + t * f.u[a]);
+            }
+        }
+    }
+}
+
+__global__ void probe_rays_bwd_kernel(int kind, const float* __restrict__ median, const float* __restrict__ hint,
+                                      const float* __restrict__ grad_origins, const float* __restrict__ grad_dirs, int64_t n_rays,
+                                      double angle, double radius, double width, float* __restrict__ grad_centre,
+                                      float* __restrict__ grad_median, float* __restrict__ grad_hint) {
+    const int64_t pose = blockIdx.x;                       // one warp per pose
+    const int lane = threadIdx.x;
+    double gc[3] = {0, 0, 0}, gm[3] = {0, 0, 0}, gu[3] = {0, 0, 0};
+    for (int64_t i = lane; i < n_rays; i += 32) {
+        const float* go = grad_origins + (pose * n_rays + i) * 3;
+        const float* gd = grad_dirs + (pose * n_rays + i) * 3;
+        if (kind == DIFFUS_PROBE_CONVEX) {
+            double sa, ca;
+            sincos(fan_angle(i, n_rays, angle), &sa, &ca);
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                const double g = (double)gd[a] + radius * (double)go[a];      // d_i and the arc point both follow the fan ray
+                gm[a] += ca * g;
+                gu[a] += sa * g;
+                gc[a] += (double)go[a];
+            }
+        } else {
+            const double t = fan_angle(i, n_rays, width);
+#pragma unroll
+            for (int a = 0; a < 3; ++a) {
+                gm[a] += (double)gd[a];
+                gu[a] += t * (double)go[a];
+                gc[a] += (double)go[a];
+            }
+        }
+    }
+#pragma unroll
+    for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) {
+            gc[a] += __shfl_xor_sync(FULL, gc[a], d);
+            gm[a] += __shfl_xor_sync(FULL, gm[a], d);
+            gu[a] += __shfl_xor_sync(FULL, gu[a], d);
+        }
+    if (lane != 0) return;
+#pragma unroll
+    for (int a = 0; a < 3; ++a) grad_centre[pose * 3 + a] = (float)gc[a];
+    fan_frame_bwd(median, hint, pose, gm, gu, grad_median, grad_hint);
+}
+
+cudaError_t launch_probe_rays(int kind, const float* centre, const float* median, const float* hint, int64_t n_poses, int64_t n_rays,
+                              double angle, double radius, double width, float* origins, float* dirs, cudaStream_t st) {
+    probe_rays_kernel<<<(unsigned)n_poses, 128, 0, st>>>(kind, centre, median, hint, n_rays, angle, radius, width, origins, dirs);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_probe_rays_bwd(int kind, const float* centre, const float* median, const float* hint, const float* grad_origins,
+                                  const float* grad_dirs, int64_t n_poses, int64_t n_rays, double angle, double radius, double width,
+                                  float* grad_centre, float* grad_median, float* grad_hint, cudaStream_t st) {
+    (void)centre;                                          // the centre enters the origins linearly
+    probe_rays_bwd_kernel<<<(unsigned)n_poses, 32, 0, st>>>(kind, median, hint, grad_origins, grad_dirs, n_rays, angle, radius, width,
+                                                            grad_centre, grad_median, grad_hint);
     return cudaGetLastError();
 }
 

@@ -229,12 +229,14 @@ __device__ __forceinline__ float echo_of(float pb, float inv_pd) { return __fmul
 template <bool POSE64>
 struct RaySetup;
 
+// Float32 poses: the ray's origin is at src + pose * src_pose_stride + ray * src_ray_stride -- (3, 0) for one source per pose,
+// (3R, 3) for one origin per ray (DIFFUS_POSE_F32_PER_RAY: linear and convex array probes).
 template <>
 struct RaySetup<false> {
     float s[3], d[3];
     __device__ __forceinline__ void load(const void* src, const void* dir, int64_t pose, int64_t ray,
-                                         int64_t n_rays, int64_t dir_pose_stride, int) {
-        const float* sp = (const float*)src + pose * 3;
+                                         int64_t src_pose_stride, int64_t src_ray_stride, int64_t dir_pose_stride, int) {
+        const float* sp = (const float*)src + pose * src_pose_stride + ray * src_ray_stride;
         const float* dp = (const float*)dir + pose * dir_pose_stride + ray * 3;
 #pragma unroll
         for (int a = 0; a < 3; ++a) { s[a] = __ldg(sp + a); d[a] = __ldg(dp + a); }
@@ -249,7 +251,7 @@ struct RaySetup<true> {
     double s[3], d[3];
     int product_f32;
     __device__ __forceinline__ void load(const void* src, const void* dir, int64_t pose, int64_t ray,
-                                         int64_t n_rays, int64_t dir_pose_stride, int prod_f32) {
+                                         int64_t, int64_t, int64_t dir_pose_stride, int prod_f32) {
         const double* sp = (const double*)src + pose * 3;
         const double* dp = (const double*)dir + pose * dir_pose_stride + ray * 3;
 #pragma unroll
@@ -435,6 +437,8 @@ struct RenderParams {
     const void* sources;
     const void* directions;
     int64_t dir_pose_stride;
+    int64_t src_pose_stride;    // float32 origins: (3, 0) per pose, (3R, 3) per ray; float64 poses are always per pose
+    int64_t src_ray_stride;
     int product_f32;
     int64_t n_poses, n_rays, total_rays;
     int S, start, Sout;
@@ -448,7 +452,7 @@ struct RenderParams {
     // backward
     const float* grad_frame;
     float* grad_volume;
-    float* grad_src_partial;    // (total_rays, 3)
+    float* grad_src_partial;    // (total_rays, 3); per-ray origins: the caller's grad_sources itself
     float* grad_dir;            // (total_rays, 3)
     float* first_rbar;          // (total_rays) d loss / d (median-replaced r_1), start > 0
     // fused MSE loss (target != null): d loss / d frame = grad_scale * (frame - target)

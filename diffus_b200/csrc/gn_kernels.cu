@@ -2,7 +2,9 @@
 //
 // A pose update is the twist xi = (v, w) about the current pose, rotating about the source: p_k(xi) = (s + v) + k Rot(w) d_i,
 // so every sample's impedance has the tangent dZ_k / dxi = (grad Z_k, k (d_i x grad Z_k)) -- the spatial gradient the trilinear
-// gather already forms for the pose-gradient kernels.  The transfer-matrix prefix is carried as a DUAL pair (P, Pdot_1..6):
+// gather already forms for the pose-gradient kernels.  With one origin s_i per ray (array probes) the probe turns about its
+// pivot c, the float64 mean of the pose's origins: p_k(xi) = c + v + Rot(w) (s_i - c + k d_i), tangent (grad Z_k,
+// (o_i + k d_i) x grad Z_k) with the lever o_i = s_i - c (the PER_RAY instantiations; the per-pose ones are unchanged).  The transfer-matrix prefix is carried as a DUAL pair (P, Pdot_1..6):
 // (P, Pdot) (M, Mdot) = (P M, Pdot M + P Mdot) is associative, so the march keeps the structure of the forward kernel --
 // lane-local chunk products, one warp scan, a second sweep -- with no reverse sweep and no prefix pre-pass.  Per column
 //     rdot  = ((Zdot_c - Zdot_{c-1}) - r (Zdot_{c-1} + Zdot_c)) / (Z_{c-1} + Z_c)      (d of (Z_c - Z_{c-1}) / (Z_{c-1} + Z_c))
@@ -87,12 +89,27 @@ __device__ __forceinline__ D2 d2_load(const float* s) {
     return x;
 }
 
-// the lane's sample tangent (grad Z, k (d x grad Z))
-__device__ __forceinline__ void sample_tangent(const float d[3], const float g[3], float kf, float t[6]) {
+// the lane's sample tangent (grad Z, k (d x grad Z)); PER_RAY: (grad Z, (o + k d) x grad Z) with the ray's lever o
+template <bool PER_RAY>
+__device__ __forceinline__ void sample_tangent(const float d[3], const float o[3], const float g[3], float kf, float t[6]) {
     t[0] = g[0]; t[1] = g[1]; t[2] = g[2];
-    t[3] = kf * (d[1] * g[2] - d[2] * g[1]);
-    t[4] = kf * (d[2] * g[0] - d[0] * g[2]);
-    t[5] = kf * (d[0] * g[1] - d[1] * g[0]);
+    if (PER_RAY) {
+        const float a0 = fmaf(kf, d[0], o[0]), a1 = fmaf(kf, d[1], o[1]), a2 = fmaf(kf, d[2], o[2]);
+        t[3] = a1 * g[2] - a2 * g[1];
+        t[4] = a2 * g[0] - a0 * g[2];
+        t[5] = a0 * g[1] - a1 * g[0];
+    } else {
+        t[3] = kf * (d[1] * g[2] - d[2] * g[1]);
+        t[4] = kf * (d[2] * g[0] - d[0] * g[2]);
+        t[5] = kf * (d[0] * g[1] - d[1] * g[0]);
+    }
+}
+
+// the ray's lever o = s_i - c about its pose's pivot (float64 difference, one rounding)
+template <bool PER_RAY>
+__device__ __forceinline__ void ray_lever(const RaySetup<false>& rs, const double* __restrict__ pivot, int64_t pose, float o[3]) {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) o[a] = PER_RAY ? (float)((double)rs.s[a] - __ldg(pivot + pose * 3 + a)) : 0.f;
 }
 
 __device__ __forceinline__ int64_t gn_pose_of_ray(int64_t ray, const RenderParams& p) {
@@ -104,9 +121,9 @@ __device__ __forceinline__ int64_t gn_pose_of_ray(int64_t ray, const RenderParam
 // the neighbour's by one shuffle, and the column's r, rdot, attenuation and target parked in shared memory.  Chunk phase (lane =
 // 16 consecutive columns): the dual chunk product, one warp scan, the second sweep forming e, J and the accumulators.  The dual
 // prefix entering the next pass goes through shared memory, so it is not live during the gathers.
-template <int LAYOUT>
+template <int LAYOUT, bool PER_RAY>
 __global__ void __launch_bounds__(128) render_gn_kernel(const RenderParams p, const float* __restrict__ med_tan,
-                                                        float* __restrict__ partial) {
+                                                        const double* __restrict__ pivot, float* __restrict__ partial) {
     using G = FwdGeo;
     constexpr int CH = G::CHUNK;
     extern __shared__ __align__(16) float smem[];
@@ -117,7 +134,9 @@ __global__ void __launch_bounds__(128) render_gn_kernel(const RenderParams p, co
     float* carry_s = rows + GN_ROWS * GN_ROW;
     const int64_t pose = gn_pose_of_ray(ray, p);
     RaySetup<false> rs;
-    rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.n_rays, p.dir_pose_stride, 0);
+    rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, 0);
+    float lever[3];
+    ray_lever<PER_RAY>(rs, pivot, pose, lever);
     const bool has_med = p.median != nullptr;
     const float med = has_med ? __ldg(p.median + pose) : 0.f;
     float mt[6];
@@ -155,7 +174,7 @@ __global__ void __launch_bounds__(128) render_gn_kernel(const RenderParams p, co
                 float z = 0.f;
                 if (ok) z = fe[u].template finish<true>(g);
                 float tz[6];
-                sample_tangent(rs.d, g, (float)(p.start + c), tz);
+                sample_tangent<PER_RAY>(rs.d, lever, g, (float)(p.start + c), tz);
                 float zp = __shfl_up_sync(FULL, z, 1);
                 float tp[6];
 #pragma unroll
@@ -293,8 +312,9 @@ __global__ void __launch_bounds__(128) gn_reduce_kernel(const float* __restrict_
 // mean of the tangents of the rays tied with it (tie_count from first_refl_median_kernel; a NaN median has no tangent).  The
 // coefficient is formed exactly like first_refl_median_kernel does (same expression, IEEE division), so the ties it counted are
 // the ties found here.  One warp per pose.
-template <int LAYOUT>
-__global__ void gn_median_tangent_kernel(const RenderParams p, const int32_t* __restrict__ tie_count, float* __restrict__ med_tan) {
+template <int LAYOUT, bool PER_RAY>
+__global__ void gn_median_tangent_kernel(const RenderParams p, const int32_t* __restrict__ tie_count, const double* __restrict__ pivot,
+                                         float* __restrict__ med_tan) {
     const int64_t pose = blockIdx.x;
     const int lane = threadIdx.x;
     const float med = p.median[pose];
@@ -303,15 +323,16 @@ __global__ void gn_median_tangent_kernel(const RenderParams p, const int32_t* __
     float acc[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     for (int64_t m = lane; m < p.n_rays && ties > 0; m += 32) {
         RaySetup<false> rs;
-        rs.load(p.sources, p.directions, pose, m, p.n_rays, p.dir_pose_stride, 0);
+        rs.load(p.sources, p.directions, pose, m, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, 0);
         float g0[3], g1[3];
         const float z0 = sample_volume<DIFFUS_SAMPLER_TRILINEAR, LAYOUT, true>(p.vol, rs.coord(0, k), rs.coord(1, k), rs.coord(2, k), g0);
         const float z1 = sample_volume<DIFFUS_SAMPLER_TRILINEAR, LAYOUT, true>(p.vol, rs.coord(0, k + 1), rs.coord(1, k + 1),
                                                                                rs.coord(2, k + 1), g1);
         if (!((z1 - z0) / (z0 + z1) == med)) continue;
-        float t0[6], t1[6];
-        sample_tangent(rs.d, g0, (float)k, t0);
-        sample_tangent(rs.d, g1, (float)(k + 1), t1);
+        float lever[3], t0[6], t1[6];
+        ray_lever<PER_RAY>(rs, pivot, pose, lever);
+        sample_tangent<PER_RAY>(rs.d, lever, g0, (float)k, t0);
+        sample_tangent<PER_RAY>(rs.d, lever, g1, (float)(k + 1), t1);
         const float sum = z0 + z1;
         const float w = 2.f / (sum * sum);
 #pragma unroll
@@ -322,6 +343,31 @@ __global__ void gn_median_tangent_kernel(const RenderParams p, const int32_t* __
         const float s = warp_sum(acc[j]);
         if (lane == 0) med_tan[pose * 6 + j] = ties > 0 ? s / (float)ties : 0.f;
     }
+}
+
+// Per-ray origins: the pivot of each pose, the mean of its R origins in double (lane-strided sums, then a butterfly: the same
+// order on every run).  One warp per pose.
+__global__ void __launch_bounds__(128) gn_pivot_kernel(const float* __restrict__ src, int64_t n_poses, int64_t n_rays,
+                                                       double* __restrict__ pivot) {
+    const int lane = threadIdx.x & 31;
+    const int64_t pose = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (pose >= n_poses) return;
+    const float* s = src + pose * n_rays * 3;
+    double a[3] = {0.0, 0.0, 0.0};
+    for (int64_t r = lane; r < n_rays; r += 32)
+#pragma unroll
+        for (int j = 0; j < 3; ++j) a[j] += (double)__ldg(s + r * 3 + j);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) a[j] += __shfl_xor_sync(FULL, a[j], d);
+        if (lane == 0) pivot[pose * 3 + j] = a[j] / (double)n_rays;
+    }
+}
+
+cudaError_t launch_gn_pivot(const float* sources, int64_t n_poses, int64_t n_rays, double* pivot, cudaStream_t st) {
+    gn_pivot_kernel<<<(unsigned)((n_poses + 3) / 4), 128, 0, st>>>(sources, n_poses, n_rays, pivot);
+    return cudaGetLastError();
 }
 
 static int gn_warps_per_block(int64_t total_rays) {
@@ -338,19 +384,31 @@ static int gn_warps_per_block(int64_t total_rays) {
         case DIFFUS_LAYOUT_TEXTURE: { constexpr int L_ = DIFFUS_LAYOUT_TEXTURE; __VA_ARGS__; } \
     }
 
-cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, const int32_t* tie_count, float* med_tan, cudaStream_t st) {
-    DIFFUS_GN_LAYOUTS(gn_median_tangent_kernel<L_><<<(unsigned)p.n_poses, 32, 0, st>>>(p, tie_count, med_tan); return cudaGetLastError())
+cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, const int32_t* tie_count, const double* pivot, float* med_tan,
+                                     cudaStream_t st) {
+    if (pivot) {
+        DIFFUS_GN_LAYOUTS(gn_median_tangent_kernel<L_, true><<<(unsigned)p.n_poses, 32, 0, st>>>(p, tie_count, pivot, med_tan);
+                          return cudaGetLastError())
+    } else {
+        DIFFUS_GN_LAYOUTS(gn_median_tangent_kernel<L_, false><<<(unsigned)p.n_poses, 32, 0, st>>>(p, tie_count, pivot, med_tan);
+                          return cudaGetLastError())
+    }
     return cudaErrorInvalidValue;
 }
 
-cudaError_t launch_render_gn(const RenderParams& p, int layout, const float* med_tan, float* partial, float* loss, float* jtr,
-                             float* jtj, cudaStream_t st) {
+cudaError_t launch_render_gn(const RenderParams& p, int layout, const float* med_tan, const double* pivot, float* partial, float* loss,
+                             float* jtr, float* jtj, cudaStream_t st) {
     const int wpb = gn_warps_per_block(p.total_rays);
     const size_t smem = (size_t)wpb * GN_SMEM_PER_WARP * sizeof(float);
     const unsigned grid = (unsigned)((p.total_rays + wpb - 1) / wpb);
     cudaError_t e = cudaErrorInvalidValue;
-    DIFFUS_GN_LAYOUTS(auto k = render_gn_kernel<L_>; e = ensure_smem(k, smem); if (e != cudaSuccess) return e;
-                      k<<<grid, wpb * 32, smem, st>>>(p, med_tan, partial); e = cudaGetLastError(); break)
+    if (pivot) {
+        DIFFUS_GN_LAYOUTS(auto k = render_gn_kernel<L_, true>; e = ensure_smem(k, smem); if (e != cudaSuccess) return e;
+                          k<<<grid, wpb * 32, smem, st>>>(p, med_tan, pivot, partial); e = cudaGetLastError(); break)
+    } else {
+        DIFFUS_GN_LAYOUTS(auto k = render_gn_kernel<L_, false>; e = ensure_smem(k, smem); if (e != cudaSuccess) return e;
+                          k<<<grid, wpb * 32, smem, st>>>(p, med_tan, pivot, partial); e = cudaGetLastError(); break)
+    }
     if (e != cudaSuccess) return e;
     gn_reduce_kernel<<<(unsigned)p.n_poses, 128, 0, st>>>(partial, p.n_rays, loss, jtr, jtj);
     return cudaGetLastError();

@@ -121,6 +121,11 @@ cudaError_t launch_fan_directions(const float* median, const float* hint, int64_
                                   float* out, cudaStream_t st);
 cudaError_t launch_fan_directions_bwd(const float* median, const float* hint, const float* grad_dirs, int64_t n_poses,
                                       int64_t n_rays, double angle, float* grad_median, float* grad_hint, cudaStream_t st);
+cudaError_t launch_probe_rays(int kind, const float* centre, const float* median, const float* hint, int64_t n_poses, int64_t n_rays,
+                              double angle, double radius, double width, float* origins, float* dirs, cudaStream_t st);
+cudaError_t launch_probe_rays_bwd(int kind, const float* centre, const float* median, const float* hint, const float* grad_origins,
+                                  const float* grad_dirs, int64_t n_poses, int64_t n_rays, double angle, double radius, double width,
+                                  float* grad_centre, float* grad_median, float* grad_hint, cudaStream_t st);
 cudaError_t launch_to_bricks(const float* linear, const int32_t dim[3], float* bricks, cudaStream_t st);
 cudaError_t launch_from_bricks(const float* bricks, const int32_t dim[3], float* linear, cudaStream_t st);
 cudaError_t launch_to_quads(const float* linear, const int32_t dim[3], float* quads, cudaStream_t st);
@@ -128,10 +133,13 @@ cudaError_t launch_gather_probe(const float* buf, int64_t n_floats, int reads, i
                                 cudaStream_t st);
 
 // gn_kernels.cu: the Gauss-Newton system of each pose (trilinear sampler, float32 poses); partial holds 32 floats per ray,
-// med_tan 6 floats per pose (start > 0 only)
-cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, const int32_t* tie_count, float* med_tan, cudaStream_t st);
-cudaError_t launch_render_gn(const RenderParams& p, int layout, const float* med_tan, float* partial, float* loss, float* jtr,
-                             float* jtj, cudaStream_t st);
+// med_tan 6 floats per pose (start > 0 only).  pivot (3 doubles per pose, from launch_gn_pivot) is given for per-ray origins
+// only, and selects the instantiations that rotate about it; NULL = one source per pose.
+cudaError_t launch_gn_pivot(const float* sources, int64_t n_poses, int64_t n_rays, double* pivot, cudaStream_t st);
+cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, const int32_t* tie_count, const double* pivot, float* med_tan,
+                                     cudaStream_t st);
+cudaError_t launch_render_gn(const RenderParams& p, int layout, const float* med_tan, const double* pivot, float* partial, float* loss,
+                             float* jtr, float* jtj, cudaStream_t st);
 
 // smooth_kernels.cu: scipy.ndimage.gaussian_filter(mode='nearest') of a (D,H,W) float32 volume in three separable passes,
 // radius r = int(truncate sigma + 0.5) <= BLUR_MAX_RADIUS (r = 0: a copy); dst and scratch hold D*H*W floats each

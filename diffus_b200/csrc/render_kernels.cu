@@ -343,7 +343,7 @@ __global__ void __launch_bounds__(128, 7) render_fwd_kernel(const RenderParams p
     float* obuf = zbuf + G::ZBUF;
     const int64_t pose = pose_of_ray(ray, p);
     RaySetup<POSE64> rs;
-    rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.n_rays, p.dir_pose_stride, p.product_f32);
+    rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, p.product_f32);
     const float med = p.median ? __ldg(p.median + pose) : 0.f;
     float* out = p.frame + ray * (int64_t)p.Sout;
     if (lane == 0) zbuf[0] = 0.f;
@@ -640,7 +640,7 @@ render_bwd_kernel(const RenderParams p) {
     RaySetup<POSE64> rs;
     float med = 0.f;
     if (live) {
-        rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.n_rays, p.dir_pose_stride, p.product_f32);
+        rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, p.product_f32);
         if (p.median) med = __ldg(p.median + pose);
     }
     fill_attenuation_padded<G>(att, ONE_PASS ? p.Sout : min(p.Sout, SS), p.alpha);

@@ -63,10 +63,16 @@ class GraphedFanPoseStep:
     The fans are generated on the device (``ops.fan_directions``) and the gradient w.r.t. the (P,R,3) directions is
     folded back onto the two (P,3) orientation vectors inside the graph, so a step moves 9 floats per pose in each
     direction instead of 3 + 3R.  Outputs are static tensors that the next call overwrites.
+
+    ``probe='convex'`` (``radius``) or ``'linear'`` (``width``): array probes, whose ``sources`` are the probe centres.  The
+    graph then generates the per-ray origins and directions (``ops.probe_rays_fwd``), runs the fused step with one origin per
+    ray and folds the (P,R,3) gradients back onto centre, median and hint (``ops.probe_rays_bwd``).
     """
 
     def __init__(self, volume, targets: torch.Tensor, n_rays: int, num_samples: int, opening_angle: float,
-                 attenuation_coeff: float = 0.5, start=0):
+                 attenuation_coeff: float = 0.5, start=0, *, probe: str = "sector", radius=None, width=None):
+        from .pose_recovery import probe_keywords
+        probe, radius, width = probe_keywords(probe, radius, width)
         if isinstance(volume, PreparedVolume):
             bricks, vol = volume.bricks, volume.volume
         else:
@@ -88,6 +94,15 @@ class GraphedFanPoseStep:
         o_gs, o_gm, o_gh, o_loss = self.out[:3 * P], self.out[3 * P:6 * P], self.out[6 * P:9 * P], self.out[9 * P:]
 
         def step():
+            if probe != "sector":
+                kid, angle, rho, w = ops.probe_args(probe, opening_angle, radius, width)
+                org, dirs = ops.probe_rays_fwd(kid, self.sources, self.median, self.hint, n_rays, angle, rho, w)
+                _, _, _, go, gd = ops.render_mse_impl(vol, bricks, list(vol.shape), org, dirs, tgt, int(num_samples), start_i,
+                                                      float(attenuation_coeff), SAMPLER_TRILINEAR, False, False, True, False,
+                                                      loss_out=o_loss)
+                ops.probe_rays_bwd(kid, self.sources, self.median, self.hint, go, gd, n_rays, angle, rho, w, grad_centre_out=o_gs,
+                                   grad_median_out=o_gm, grad_hint_out=o_gh)
+                return
             dirs = ops.fan_directions_fwd(self.median, self.hint, opening_angle, n_rays)
             _, _, _, _, gd = ops.render_mse_impl(vol, bricks, list(vol.shape), self.sources, dirs, tgt, int(num_samples),
                                                  start_i, float(attenuation_coeff), SAMPLER_TRILINEAR, False, False, True,
@@ -155,13 +170,21 @@ class GraphedFanGaussNewtonStep:
     the twist to the fan parameters, generates the candidate fans, renders their Gauss-Newton systems
     (``ops.render_gauss_newton_impl``) and accepts or rejects each pose on its own loss.  Call :meth:`reset` before the first
     replay.
+
+    ``probe='convex'`` (``radius``) or ``'linear'`` (``width``): array probes with ``sources`` their centres.  The systems are
+    rendered from the rays of ``ops.probe_rays_fwd`` with one origin per ray, and the step is applied to the parameters by
+    ``apply_probe_twist`` about the pivot of the current origins -- the point the kernel's twist turns about.
     """
 
     LAM_DOWN, LAM_UP, LAM_MIN, LAM_MAX = 1.0 / 3.0, 4.0, 1e-9, 1e9
 
     def __init__(self, volume, targets: torch.Tensor, n_rays: int, num_samples: int, opening_angle: float,
-                 attenuation_coeff: float = 0.5, start=0):
-        from .pose_recovery import apply_fan_twist
+                 attenuation_coeff: float = 0.5, start=0, *, probe: str = "sector", radius=None, width=None):
+        from .pose_recovery import apply_fan_twist, apply_probe_twist, probe_keywords, probe_pivot
+        probe, radius, width = probe_keywords(probe, radius, width)
+        array = probe != "sector"
+        if array:
+            kid, angle, rho, wid = ops.probe_args(probe, opening_angle, radius, width)
         if isinstance(volume, PreparedVolume):
             bricks, vol = volume.bricks, volume.volume
         else:
@@ -183,8 +206,11 @@ class GraphedFanGaussNewtonStep:
         self.lam = torch.ones((P,), dtype=torch.float64, device=dev)
 
         def system(poses, loss, jtj, jtr):
-            dirs = ops.fan_directions_fwd(poses[1], poses[2], opening_angle, n_rays)
-            ops.render_gauss_newton_impl(vol, bricks, list(vol.shape), poses[0], dirs, tgt, int(num_samples), start_i,
+            if array:
+                src, dirs = ops.probe_rays_fwd(kid, poses[0], poses[1], poses[2], n_rays, angle, rho, wid)
+            else:
+                src, dirs = poses[0], ops.fan_directions_fwd(poses[1], poses[2], opening_angle, n_rays)
+            ops.render_gauss_newton_impl(vol, bricks, list(vol.shape), src, dirs, tgt, int(num_samples), start_i,
                                          float(attenuation_coeff), loss_out=loss, jtj_out=jtj, jtr_out=jtr)
 
         def step():
@@ -195,7 +221,11 @@ class GraphedFanGaussNewtonStep:
             delta, ok = _solve_spd6(a, -self.jtr.double())
             ok = ok & torch.isfinite(delta).all(-1)
             delta = torch.where(ok[:, None], delta, torch.zeros_like(delta)).float()
-            s, m, h = apply_fan_twist(self.sources, self.median, self.hint, delta)
+            if array:
+                org, _ = ops.probe_rays_fwd(kid, self.sources, self.median, self.hint, n_rays, angle, rho, wid)
+                s, m, h = apply_probe_twist(self.sources, self.median, self.hint, delta, probe_pivot(org))
+            else:
+                s, m, h = apply_fan_twist(self.sources, self.median, self.hint, delta)
             self.cand[0].copy_(s)
             self.cand[1].copy_(m)
             self.cand[2].copy_(h)

@@ -7,12 +7,14 @@ require CUDA tensors and raise otherwise -- there is no CPU path.
 from __future__ import annotations
 
 import ctypes as C
+import math
 from typing import List, Optional, Tuple
 
 import torch
 
 from . import _lib
-from ._lib import (LAYOUT_BRICK, LAYOUT_LINEAR, LAYOUT_QUAD, LAYOUT_TEXTURE, MLP_NPARAMS, POSE_F32, POSE_F64, SAMPLER_NEAREST,
+from ._lib import (LAYOUT_BRICK, LAYOUT_LINEAR, LAYOUT_QUAD, LAYOUT_TEXTURE, MLP_NPARAMS, POSE_F32, POSE_F32_PER_RAY, POSE_F64,
+                   PROBE_CONVEX, PROBE_LINEAR, SAMPLER_NEAREST,
                    SAMPLER_TRILINEAR, DiffusRenderArgs, DiffusRenderBwdArgs)
 
 SEG = 512  # PREFIX_STRIDE of csrc/common.cuh: the forward saves a 2x2 prefix every SEG columns
@@ -169,7 +171,7 @@ def _fill_render_args(a: DiffusRenderArgs, volume, bricks, dims, sources, direct
     a.volume.layout = layout
     a.sources = sources.data_ptr()
     a.directions = directions.data_ptr()
-    a.pose_dtype = POSE_F64 if sources.dtype == torch.float64 else POSE_F32
+    a.pose_dtype = _pose_tag(sources, directions)
     a.product_f32 = int(product_f32)
     P = sources.shape[0]
     R = directions.shape[-2]
@@ -179,13 +181,25 @@ def _fill_render_args(a: DiffusRenderArgs, volume, bricks, dims, sources, direct
     return P, R
 
 
+def _pose_tag(sources, directions) -> int:
+    """(P,3) sources: one source per pose; (P,R,3): one origin per ray (array probes, float32 only)."""
+    if sources.dim() == 3:
+        if sources.dtype != torch.float32:
+            raise _lib.DiffusError("per-ray sources (P,R,3) must be float32: there is no float64 per-ray form")
+        if sources.shape[1] != directions.shape[-2] or sources.shape[2] != 3 or not sources.is_contiguous():
+            raise _lib.DiffusError("per-ray sources must be contiguous (P,R,3) with R the rays of the directions")
+        return POSE_F32_PER_RAY
+    return POSE_F64 if sources.dtype == torch.float64 else POSE_F32
+
+
 def _check_inputs(volume, bricks, dims, sources, directions):
     if volume.dtype != torch.float32 or not volume.is_contiguous():
         raise _lib.DiffusError("volume must be a contiguous float32 tensor")
     if sources.dtype not in (torch.float32, torch.float64) or sources.dtype != directions.dtype:
         raise _lib.DiffusError("sources/directions must both be float32 or both float64")
-    if sources.dim() != 2 or sources.shape[1] != 3 or not sources.is_contiguous():
-        raise _lib.DiffusError("sources must be contiguous (P,3)")
+    if sources.dim() not in (2, 3) or sources.shape[-1] != 3 or not sources.is_contiguous():
+        raise _lib.DiffusError("sources must be contiguous (P,3), or (P,R,3) for one origin per ray")
+    _pose_tag(sources, directions)
     if directions.shape[-1] != 3 or directions.dim() not in (2, 3) or not directions.is_contiguous():
         raise _lib.DiffusError("directions must be contiguous (R,3) or (P,R,3)")
     if directions.dim() == 3 and directions.shape[0] != sources.shape[0]:
@@ -262,7 +276,7 @@ def render_bwd_impl(grad_frame: torch.Tensor, volume: torch.Tensor, bricks: Opti
         gshape = _grad_volume_shape(bricks, dims)
         gvol = torch.zeros(gshape, dtype=torch.float32, device=dev) if need_volume else \
             torch.empty((0,), dtype=torch.float32, device=dev)
-        gsrc = torch.empty((P, 3) if need_pose else (0,), dtype=torch.float32, device=dev)
+        gsrc = torch.empty(tuple(sources.shape) if need_pose else (0,), dtype=torch.float32, device=dev)
         gdir = torch.empty((P, R, 3) if need_pose else (0,), dtype=torch.float32, device=dev)
         b.fwd.seg_prefix = _ptr(prefix)
         b.grad_frame = grad_frame.data_ptr()
@@ -273,7 +287,8 @@ def render_bwd_impl(grad_frame: torch.Tensor, volume: torch.Tensor, bricks: Opti
         b.workspace, b.workspace_bytes = ws.data_ptr(), wbytes
         b.fwd.workspace, b.fwd.workspace_bytes = None, 0
         _lib.check(lib.diffus_render_backward(C.byref(b), _stream(dev)), "diffus_render_backward")
-        _count((1 if (need_volume or need_pose) else 0) + (2 if start > 0 else 0) + (1 if need_pose else 0))
+        fold = need_pose and sources.dim() == 2           # per-ray origins: no reduction over the rays
+        _count((1 if (need_volume or need_pose) else 0) + (2 if start > 0 else 0) + (1 if fold else 0))
         if need_volume and use_bricks:
             gvol = from_bricks(gvol, dims)
     return gvol, gsrc, gdir
@@ -293,7 +308,7 @@ def _(grad_frame, volume, bricks, dims, sources, directions, prefix, n_samples, 
     P, R = sources.shape[0], directions.shape[-2]
     need_pose = need_pose and sampler == SAMPLER_TRILINEAR
     gvol = volume.new_empty(tuple(dims) if need_volume else (0,), dtype=torch.float32)
-    gsrc = volume.new_empty((P, 3) if need_pose else (0,), dtype=torch.float32)
+    gsrc = volume.new_empty(tuple(sources.shape) if need_pose else (0,), dtype=torch.float32)
     gdir = volume.new_empty((P, R, 3) if need_pose else (0,), dtype=torch.float32)
     return gvol, gsrc, gdir
 
@@ -385,7 +400,7 @@ def render_mse_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: 
     gradients are then this shard's share of the global mean, so that a SUM all-reduce over ranks gives exactly the
     single-process result even for ragged shards.  ``grad_volume_out`` (a zero-filled buffer in the gradient layout) and
     ``loss_out`` (1 float) let a training loop hand in persistent buffers instead of fresh allocations; ``grad_sources_out``
-    (3P floats) likewise for d loss / d sources (a slice of a CUDA graph's static output block).
+    (3P floats, 3PR for per-ray sources) likewise for d loss / d sources (a slice of a CUDA graph's static output block).
     """
     dev = _require_cuda(volume, bricks, sources, directions, target)
     _check_inputs(volume, bricks, dims, sources, directions)
@@ -411,7 +426,7 @@ def render_mse_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: 
             gvol = grad_volume_out
         else:
             gvol = torch.zeros(gshape, dtype=torch.float32, device=dev) if need_volume else empty()
-        gsrc = _out_buffer(grad_sources_out, (P, 3), dev, "grad_sources_out") if need_pose else empty()
+        gsrc = _out_buffer(grad_sources_out, tuple(sources.shape), dev, "grad_sources_out") if need_pose else empty()
         gdir = torch.empty((P, R, 3), dtype=torch.float32, device=dev) if need_pose else empty()
         b.grad_frame = None
         b.grad_volume, b.grad_sources, b.grad_directions = _ptr(gvol), _ptr(gsrc), _ptr(gdir)
@@ -430,7 +445,7 @@ def render_mse_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: 
         b.workspace, b.workspace_bytes = ws.data_ptr(), wbytes
         _lib.check(lib.diffus_render_backward(C.byref(b), _stream(dev)), "diffus_render_backward (fused MSE)")
         # fused kernel + loss reduction (+ the d/dsources reduction: the same launch as the loss up to 2^18 rays) (+ median)
-        _count(2 + (2 if start > 0 else 0) + (1 if need_pose and P * R > (1 << 18) else 0))
+        _count(2 + (2 if start > 0 else 0) + (1 if need_pose and sources.dim() == 2 and P * R > (1 << 18) else 0))
         if need_volume and use_bricks and not keep_brick_grad:
             gvol = from_bricks(gvol, dims)
     return loss, frame, gvol, gsrc, gdir
@@ -454,7 +469,7 @@ def _(volume, bricks, dims, sources, directions, target, n_samples, start, alpha
     return (volume.new_empty((1,), dtype=torch.float32),
             volume.new_empty((P, R, n_samples - start), dtype=torch.float32) if want_frame else e(),
             volume.new_empty(tuple(dims), dtype=torch.float32) if need_volume else e(),
-            volume.new_empty((P, 3), dtype=torch.float32) if need_pose else e(),
+            volume.new_empty(tuple(sources.shape), dtype=torch.float32) if need_pose else e(),
             volume.new_empty((P, R, 3), dtype=torch.float32) if need_pose else e())
 
 
@@ -495,7 +510,8 @@ def render_gauss_newton_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor
                              directions: torch.Tensor, target: torch.Tensor, n_samples: int, start: int, alpha: float,
                              loss_out: Optional[torch.Tensor] = None, jtj_out: Optional[torch.Tensor] = None,
                              jtr_out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-    """Per pose p, with res = frame - target and J = d frame / d xi for a rigid twist xi = (v, w) of the pose about its source:
+    """Per pose p, with res = frame - target and J = d frame / d xi for a rigid twist xi = (v, w) of the pose about its source
+    (per-ray sources (P,R,3): about the pose's pivot, the float64 mean of its origins):
     ``loss[p] = sum res^2``, ``JtJ[p] = J^T J`` (6x6), ``Jtr[p] = J^T res`` (6).  Trilinear sampler, float32 poses.
 
     Two launches (+ two for the median when ``start > 0``).  ``*_out``: caller-provided output buffers (static tensors of a
@@ -518,7 +534,7 @@ def render_gauss_newton_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor
         ws = torch.empty((max(wbytes, 1),), dtype=torch.uint8, device=dev)
         g.workspace, g.workspace_bytes = ws.data_ptr(), wbytes
         _lib.check(lib.diffus_render_gauss_newton(C.byref(g), _stream(dev)), "diffus_render_gauss_newton")
-        _count(2 + (2 if start > 0 else 0))
+        _count(2 + (2 if start > 0 else 0) + (1 if sources.dim() == 3 else 0))
     return loss.view(P), jtj.view(P, 6, 6), jtr.view(P, 6)
 
 
@@ -603,13 +619,13 @@ def trace_values_bwd(grad_values, volume, bricks, dims, sources, directions, n_s
         g = grad_values.contiguous().float()
         gvol = torch.zeros(_grad_volume_shape(bricks, dims), dtype=torch.float32, device=dev) \
             if need_volume else None
-        gsrc = torch.empty((P, 3), dtype=torch.float32, device=dev) if need_pose else None
+        gsrc = torch.empty(tuple(sources.shape), dtype=torch.float32, device=dev) if need_pose else None
         gdir = torch.empty((P, R, 3), dtype=torch.float32, device=dev) if need_pose else None
         ws = torch.empty((max(P * R * 12 + 256, 256),), dtype=torch.uint8, device=dev)
         _lib.check(lib.diffus_trace_values_backward(C.byref(a), g.data_ptr(), _ptr(gvol), _ptr(gsrc), _ptr(gdir),
                                                     ws.data_ptr(), ws.numel(), _stream(dev)),
                    "diffus_trace_values_backward")
-        _count(1 + (1 if need_pose else 0))
+        _count(1 + (1 if need_pose and sources.dim() == 2 else 0))
         if need_volume and use_bricks:
             gvol = from_bricks(gvol, dims)
     return gvol, gsrc, gdir
@@ -785,6 +801,116 @@ def fan_directions(median: torch.Tensor, normal_hint: torch.Tensor, opening_angl
     (P,3) in-plane hints -> (P,R,3) float32 unit directions ``cos(a) m^ + sin(a) u^`` -- ``generate_cone_directions``
     (reference ``src/cone.py:242-259``) generalised from the z = 0 plane to the plane spanned by median and hint."""
     return FanDirectionsFunction.apply(median, normal_hint, opening_angle, n_rays)
+
+
+_PROBE_KINDS = {"convex": PROBE_CONVEX, "linear": PROBE_LINEAR}
+
+
+def probe_kind(kind: str) -> int:
+    try:
+        return _PROBE_KINDS[kind]
+    except KeyError:
+        raise ValueError(f"unknown probe kind {kind!r}; expected 'convex' or 'linear'") from None
+
+
+def _probe_params(median, hint):
+    m, h = median.detach().float().contiguous(), hint.detach().float().contiguous()
+    if m.dim() != 2 or m.shape[1] != 3 or h.shape != m.shape:
+        raise _lib.DiffusError("centre, median and hint must all be (P,3)")
+    return m, h
+
+
+def probe_rays_fwd(kind: int, centre: torch.Tensor, median: torch.Tensor, hint: torch.Tensor, n_rays: int, opening_angle: float,
+                   radius: float, width: float, origins_out: Optional[torch.Tensor] = None,
+                   directions_out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """(P,R,3) origins and directions of convex / linear array probes (``include/diffus_b200.h``: ``diffus_probe_rays``)."""
+    dev = _require_cuda(centre, median, hint)
+    lib = _lib.load()
+    m, h = _probe_params(median, hint)
+    c = centre.detach().float().contiguous()
+    if c.shape != m.shape:
+        raise _lib.DiffusError("centre, median and hint must all be (P,3)")
+    P = m.shape[0]
+    with _on_device(dev):
+        o = _out_buffer(origins_out, (P, n_rays, 3), dev, "origins_out")
+        d = _out_buffer(directions_out, (P, n_rays, 3), dev, "directions_out")
+        _lib.check(lib.diffus_probe_rays(kind, c.data_ptr(), m.data_ptr(), h.data_ptr(), P, n_rays, float(opening_angle),
+                                         float(radius), float(width), o.data_ptr(), d.data_ptr(), _stream(dev)),
+                   "diffus_probe_rays")
+        _count(1)
+    return o.view(P, n_rays, 3), d.view(P, n_rays, 3)
+
+
+def probe_rays_bwd(kind: int, centre: torch.Tensor, median: torch.Tensor, hint: torch.Tensor, grad_origins: torch.Tensor,
+                   grad_directions: torch.Tensor, n_rays: int, opening_angle: float, radius: float, width: float,
+                   grad_centre_out: Optional[torch.Tensor] = None, grad_median_out: Optional[torch.Tensor] = None,
+                   grad_hint_out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    dev = _require_cuda(centre, median, hint, grad_origins, grad_directions)
+    lib = _lib.load()
+    m, h = _probe_params(median, hint)
+    c = centre.detach().float().contiguous()
+    P = m.shape[0]
+    go, gd = grad_origins.float().contiguous(), grad_directions.float().contiguous()
+    if go.numel() != P * n_rays * 3 or gd.numel() != P * n_rays * 3:
+        raise _lib.DiffusError(f"grad_origins and grad_directions must be {(P, n_rays, 3)}")
+    with _on_device(dev):
+        gc = _out_buffer(grad_centre_out, (P, 3), dev, "grad_centre_out")
+        gm = _out_buffer(grad_median_out, (P, 3), dev, "grad_median_out")
+        gh = _out_buffer(grad_hint_out, (P, 3), dev, "grad_hint_out")
+        _lib.check(lib.diffus_probe_rays_backward(kind, c.data_ptr(), m.data_ptr(), h.data_ptr(), go.data_ptr(), gd.data_ptr(), P,
+                                                  n_rays, float(opening_angle), float(radius), float(width), gc.data_ptr(),
+                                                  gm.data_ptr(), gh.data_ptr(), _stream(dev)), "diffus_probe_rays_backward")
+        _count(1)
+    return gc, gm, gh
+
+
+class ProbeRaysFunction(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, kind, centre, median, hint, n_rays, opening_angle, radius, width):
+        ctx.save_for_backward(centre, median, hint)
+        ctx.args = (int(kind), int(n_rays), float(opening_angle), float(radius), float(width))
+        return probe_rays_fwd(kind, centre, median, hint, n_rays, opening_angle, radius, width)
+
+    @staticmethod
+    def backward(ctx, g_origins, g_dirs):
+        centre, median, hint = ctx.saved_tensors
+        kind, n_rays, angle, radius, width = ctx.args
+        if g_origins is None:
+            g_origins = torch.zeros((centre.shape[0], n_rays, 3), dtype=torch.float32, device=centre.device)
+        if g_dirs is None:
+            g_dirs = torch.zeros((centre.shape[0], n_rays, 3), dtype=torch.float32, device=centre.device)
+        gc, gm, gh = probe_rays_bwd(kind, centre, median, hint, g_origins, g_dirs, n_rays, angle, radius, width)
+        return None, gc.to(centre.dtype), gm.to(median.dtype), gh.to(hint.dtype), None, None, None, None
+
+
+def probe_args(kind: str, opening_angle, radius, width) -> Tuple[int, float, float, float]:
+    """Host-side check of the keywords of one probe kind -> ``(kind id, opening_angle, radius, width)`` for the kernels."""
+    kid = probe_kind(kind)
+    if kid == PROBE_CONVEX:
+        if opening_angle is None:
+            raise ValueError("a convex probe needs opening_angle")
+        if not (math.isfinite(float(radius)) and float(radius) >= 0.0):
+            raise ValueError(f"a convex probe needs a finite radius >= 0, got {radius!r}")
+        return kid, float(opening_angle), float(radius), 0.0
+    if width is None or not (math.isfinite(float(width)) and float(width) > 0.0):
+        raise ValueError(f"a linear probe needs a finite width > 0, got {width!r}")
+    return kid, 0.0, 0.0, float(width)
+
+
+def probe_rays(kind: str, centre: torch.Tensor, median: torch.Tensor, hint: torch.Tensor, n_rays: int, *, opening_angle=None,
+               radius: float = 0.0, width=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Rays of linear and convex array probes from their pose parameters, on the device and differentiable.
+
+    ``centre``, ``median`` and ``hint`` are (P,3); ``m^ = median / |median|`` and ``u^`` is the hint made orthogonal to it and
+    normalised (as in :func:`fan_directions`).  Returns ``(origins, directions)``, both (P,R,3) float32, to be rendered with
+    the origins as per-ray ``sources``:
+
+    * ``'convex'`` (``opening_angle``, ``radius`` rho >= 0): ray i leaves ``centre + rho d_i`` along ``d_i = cos a_i m^ +
+      sin a_i u^``, ``a = linspace(-angle/2, angle/2, R)``.  With rho = 0 it is the sector probe of :func:`fan_directions`.
+    * ``'linear'`` (``width`` w > 0): ray i leaves ``centre + t_i u^`` along ``m^``, ``t = linspace(-w/2, w/2, R)``.
+    """
+    kid, angle, rho, w = probe_args(kind, opening_angle, radius, width)
+    return ProbeRaysFunction.apply(kid, centre, median, hint, int(n_rays), angle, rho, w)
 
 
 def gather_probe(buffer_mib: int = 64, reads_per_thread: int = 64, n_threads: int = 148 * 8 * 256, repeats: int = 5,

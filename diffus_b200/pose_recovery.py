@@ -3,8 +3,10 @@
 A pose update is the rigid twist ``xi = (v, w)`` about the current pose, rotating about the source:
 ``p_k(xi) = (s + v) + k Rot(w) d_i``.  :func:`apply_pose_twist` applies it to explicit sources / directions and
 :func:`apply_fan_twist` to the pose parameters of a fan (source, median direction, in-plane hint), which the fan generator
-turns back into the rotated fan.  The functions are plain torch and run on any device (the test oracle differentiates them on
-the CPU).
+turns back into the rotated fan.  Array probes (one origin per ray, :func:`diffus_b200.probe_rays`) turn about their PIVOT
+``c``, the float64 mean of a pose's origins: ``p_k(xi) = c + v + Rot(w) (s_i - c + k d_i)``; :func:`apply_pose_twist` takes their
+(P,R,3) origins and :func:`apply_probe_twist` their parameters.  The functions are plain torch and run on any device (the test
+oracle differentiates them on the CPU).
 """
 from __future__ import annotations
 
@@ -30,11 +32,21 @@ def _rotate(x: torch.Tensor, w: torch.Tensor) -> torch.Tensor:
     return x + a * wx + b * torch.linalg.cross(w, wx, dim=-1)
 
 
+def probe_pivot(origins: torch.Tensor) -> torch.Tensor:
+    """The pivot of array-probe poses: the float64 mean of each pose's (P,R,3) origins -> (P,3) float64."""
+    return origins.to(torch.float64).mean(-2)
+
+
 def apply_pose_twist(sources: torch.Tensor, directions: torch.Tensor, delta: torch.Tensor):
     """``(sources + v, Rot(w) directions)`` for ``delta`` (P,6) = (v, w): sources (P,3), directions (P,R,3) or a shared (R,3)
-    fan, which becomes (P,R,3)."""
+    fan, which becomes (P,R,3).  Per-ray sources (P,R,3) turn about their pivot ``c`` (:func:`probe_pivot`):
+    ``c + v + Rot(w) (s_i - c)``, evaluated in float64 and returned in the sources' dtype."""
     v, w = delta[..., :3], delta[..., 3:]
     dirs = directions if directions.dim() == 3 else directions.unsqueeze(0).expand(sources.shape[0], -1, -1)
+    if sources.dim() == 3:
+        c = probe_pivot(sources).unsqueeze(-2)
+        s = c + v.unsqueeze(-2).to(torch.float64) + _rotate(sources.to(torch.float64) - c, w.unsqueeze(-2).to(torch.float64))
+        return s.to(sources.dtype), _rotate(dirs, w.unsqueeze(-2))
     return sources + v, _rotate(dirs, w.unsqueeze(-2))
 
 
@@ -43,6 +55,43 @@ def apply_fan_twist(sources: torch.Tensor, median: torch.Tensor, hint: torch.Ten
     parameters is the rotated fan (:func:`diffus_b200.fan_directions` is rotation-equivariant)."""
     v, w = delta[..., :3], delta[..., 3:]
     return sources + v, _rotate(median, w), _rotate(hint, w)
+
+
+def apply_probe_twist(centre: torch.Tensor, median: torch.Tensor, hint: torch.Tensor, delta: torch.Tensor, pivot: torch.Tensor):
+    """The twist about ``pivot`` (P,3) on array-probe parameters: ``(pivot + v + Rot(w) (centre - pivot), Rot(w) median,
+    Rot(w) hint)``.  The rays of the twisted parameters are the twisted rays (:func:`diffus_b200.probe_rays` places the origins
+    rigidly in the frame of median and hint), so with the pivot of the current origins this is :func:`apply_pose_twist` on
+    them.  The centre is formed in float64 and returned in its own dtype."""
+    v, w = delta[..., :3], delta[..., 3:]
+    c = pivot.to(torch.float64)
+    centre2 = (c + v.to(torch.float64) + _rotate(centre.to(torch.float64) - c, w.to(torch.float64))).to(centre.dtype)
+    return centre2, _rotate(median, w), _rotate(hint, w)
+
+
+PROBES = ("sector", "convex", "linear")
+
+
+def probe_keywords(probe: str, radius, width):
+    """Validated ``(probe, radius, width)`` of the pose-recovery drivers (host only): ``'sector'`` takes neither keyword,
+    ``'convex'`` a finite radius >= 0 and ``'linear'`` a finite width > 0."""
+    if probe not in PROBES:
+        raise ValueError(f"probe must be one of {PROBES}, got {probe!r}")
+    if probe == "sector":
+        if radius not in (None, 0, 0.0) or width is not None:
+            raise ValueError("radius and width only apply to probe='convex' and probe='linear'")
+        return probe, 0.0, None
+    if probe == "convex":
+        if width is not None:
+            raise ValueError("a convex probe takes radius, not width")
+        rho = 0.0 if radius is None else float(radius)
+        if not (math.isfinite(rho) and rho >= 0.0):
+            raise ValueError(f"a convex probe needs a finite radius >= 0, got {radius!r}")
+        return probe, rho, None
+    if radius not in (None, 0, 0.0):
+        raise ValueError("a linear probe takes width, not radius")
+    if width is None or not (math.isfinite(float(width)) and float(width) > 0.0):
+        raise ValueError(f"a linear probe needs a finite width > 0, got {width!r}")
+    return probe, 0.0, float(width)
 
 
 def fan_frame_angle(median_a, hint_a, median_b, hint_b) -> torch.Tensor:
@@ -59,7 +108,7 @@ def fan_frame_angle(median_a, hint_a, median_b, hint_b) -> torch.Tensor:
 
 def recover_poses(volume, targets: torch.Tensor, sources: torch.Tensor, median: torch.Tensor, hint: torch.Tensor,
                   opening_angle: float, n_rays: int, num_samples: int, attenuation_coeff: float = 0.5, start=0,
-                  iterations: int = 10, damping: float = 1e-3):
+                  iterations: int = 10, damping: float = 1e-3, *, probe: str = "sector", radius=None, width=None):
     """Levenberg-Marquardt pose recovery of a batch of fans against their target frames.
 
     Each pose solves ``(JtJ + lam diag(JtJ) + eps I) delta = -Jtr`` (float64, Marquardt scaling), renders the candidate
@@ -70,9 +119,15 @@ def recover_poses(volume, targets: torch.Tensor, sources: torch.Tensor, median: 
     ``targets`` (P,R,S-start), ``sources`` / ``median`` / ``hint`` (P,3) float32 start poses.  Returns
     ``((sources, median, hint), history)`` with ``history`` the (iterations + 1, P) loss ``sum (frame - target)^2`` of each
     pose before the first and after every iteration.
+
+    ``probe='convex'`` (``radius``) or ``'linear'`` (``width``; ``opening_angle`` is then unused) recovers array probes
+    instead: ``sources`` are their centres and the rays come from :func:`diffus_b200.probe_rays`; the twist turns each probe
+    about its pivot (:func:`apply_probe_twist`).  The default ``'sector'`` is the point-source fan.
     """
+    probe, radius, width = probe_keywords(probe, radius, width)
     from .graphs import GraphedFanGaussNewtonStep
-    step = GraphedFanGaussNewtonStep(volume, targets, n_rays, num_samples, opening_angle, attenuation_coeff, start)
+    step = GraphedFanGaussNewtonStep(volume, targets, n_rays, num_samples, opening_angle, attenuation_coeff, start, probe=probe,
+                                     radius=radius, width=width)
     step.reset(sources, median, hint, damping)
     vol = volume.volume if isinstance(volume, PreparedVolume) else volume
     history = torch.empty((iterations + 1, step.P), dtype=torch.float32, device=vol.device)
@@ -98,7 +153,8 @@ def _schedule(sigmas, iterations):
 
 def recover_poses_coarse_to_fine(volume, targets: torch.Tensor, sources: torch.Tensor, median: torch.Tensor, hint: torch.Tensor,
                                  opening_angle: float, n_rays: int, num_samples: int, attenuation_coeff: float = 0.5, start=0, *,
-                                 sigmas=(4.0, 2.0, 1.0, 0.0), iterations=10, damping: float = 1e-3, layout=None):
+                                 sigmas=(4.0, 2.0, 1.0, 0.0), iterations=10, damping: float = 1e-3, layout=None,
+                                 probe: str = "sector", radius=None, width=None):
     """Levenberg-Marquardt pose recovery from a blurred volume to the sharp one (a Gaussian scale space).
 
     On a volume with sharp tissue boundaries the frame depends on the pose through one-voxel gradient cells, so a Gauss-Newton
@@ -109,9 +165,12 @@ def recover_poses_coarse_to_fine(volume, targets: torch.Tensor, sources: torch.T
     accept / reject compares losses across volumes.  ``layout`` of the blurred levels' :class:`PreparedVolume` defaults to the
     caller's layout, else ``'texture'``; each level's copy is released before the next is built.
 
+    ``probe``, ``radius`` and ``width`` select the probe as in :func:`recover_poses`.
+
     Returns ``((sources, median, hint), histories)``: one (iterations_l + 1, P) loss history per level.
     """
     sig, its = _schedule(sigmas, iterations)
+    probe, radius, width = probe_keywords(probe, radius, width)
     if layout is None:
         layout = volume.layout if isinstance(volume, PreparedVolume) else "texture"
     base = volume.volume if isinstance(volume, PreparedVolume) else volume
@@ -123,7 +182,7 @@ def recover_poses_coarse_to_fine(volume, targets: torch.Tensor, sources: torch.T
             with torch.no_grad():
                 level = PreparedVolume(smooth_volume(base, sigma), layout)
         poses, hist = recover_poses(level, targets, *poses, opening_angle, n_rays, num_samples, attenuation_coeff, start,
-                                    iterations=k, damping=damping)
+                                    iterations=k, damping=damping, probe=probe, radius=radius, width=width)
         histories.append(hist)
         if level is not volume:
             level.close()

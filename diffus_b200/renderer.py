@@ -112,7 +112,8 @@ class PreparedVolume:
 
 def render_frames(volume, sources: torch.Tensor, directions: torch.Tensor, num_samples: int,
                   attenuation_coeff: float = 0.5, start=0, *, sampler: str = "nearest") -> torch.Tensor:
-    """Batched ``plot_beam_frame``: (P,3) sources, (P,R,3) or (R,3) directions -> (P,R,S-start) frames.
+    """Batched ``plot_beam_frame``: (P,3) sources, (P,R,3) or (R,3) directions -> (P,R,S-start) frames.  Float32 sources
+    of shape (P,R,3) give every ray its own origin (linear and convex array probes, :func:`diffus_b200.probe_rays`).
 
     Differentiable w.r.t. ``volume`` and, with ``sampler='trilinear'``, w.r.t. ``sources``
     and ``directions``.  ``volume`` is a (D,H,W) CUDA tensor or a :class:`PreparedVolume`.
@@ -148,7 +149,8 @@ def render_mse_loss(volume, sources: torch.Tensor, directions: torch.Tensor, tar
     with the real frames, back-propagate): the kernel gathers each sample once, evaluates
     the frame, the loss and the reverse scan in shared memory, and hands autograd the
     finished gradients.  Returns the scalar loss (differentiable w.r.t. ``volume`` and, for
-    the trilinear sampler, ``sources`` / ``directions``), plus the frames if asked.
+    the trilinear sampler, ``sources`` / ``directions``), plus the frames if asked.  Per-ray sources (P,R,3) get (P,R,3)
+    gradients.
     """
     bricks = None
     if isinstance(volume, PreparedVolume):
@@ -176,7 +178,9 @@ def render_gauss_newton(volume, sources: torch.Tensor, directions: torch.Tensor,
     A pose update is the twist ``xi = (v, w)``: ``sources + v`` and the directions rotated by ``Rot(w)`` about the source
     (:func:`diffus_b200.pose_recovery.apply_pose_twist`).  With ``res = frame - target`` and ``J = d frame / d xi`` at
     ``xi = 0``, returns per pose ``loss (P,) = sum res^2``, ``JtJ (P,6,6) = J^T J`` and ``Jtr (P,6) = J^T res``.  ``2 Jtr / n``
-    is the gradient of :func:`render_mse_loss` (mean over n elements) in twist coordinates.  ``sources`` (P,3) and
+    is the gradient of :func:`render_mse_loss` (mean over n elements) in twist coordinates.  Per-ray sources (P,R,3) (array
+    probes) turn about the pose's pivot, the float64 mean of its origins (:func:`diffus_b200.pose_recovery.apply_pose_twist`).
+    ``sources`` (P,3) or (P,R,3) and
     ``directions`` (P,R,3) or (R,3) are float32 (float64 poses are not supported); ``volume`` is a (D,H,W) CUDA tensor or a
     :class:`PreparedVolume`.  Only the trilinear sampler has a pose derivative.  The outputs are NOT differentiable: they
     are what a Gauss-Newton / Levenberg-Marquardt step consumes (:func:`diffus_b200.pose_recovery.recover_poses`).

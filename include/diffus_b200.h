@@ -58,6 +58,10 @@ extern "C" {
    src/renderer.py:124, and is cast to float32 at :751) */
 #define DIFFUS_POSE_F32 0 /* sources/directions are float32 arrays                            */
 #define DIFFUS_POSE_F64 1 /* both are float64 arrays; see `product_f32`                        */
+#define DIFFUS_POSE_F32_PER_RAY 2 /* float32; sources are (P,R,3): one origin per ray (linear and convex array probes).
+                                     Ray i of pose p samples sources[p][i] + k * directions[.][i].  Accepted by every entry point
+                                     that takes a DiffusRenderArgs; a library that predates it answers DIFFUS_E_ENUM.  There is no
+                                     float64 per-ray form.                                                                   */
 
 typedef struct DiffusVolume {
     const float* data; /* impedance volume, float32                                          */
@@ -73,7 +77,7 @@ typedef struct DiffusVolume {
  * exp(-alpha k) attenuation (:256-259), for a leading batch of probe poses. */
 typedef struct DiffusRenderArgs {
     DiffusVolume volume;
-    const void* sources;        /* (P,3) float32 or float64 per pose_dtype                   */
+    const void* sources;        /* (P,3) float32 or float64 per pose_dtype; (P,R,3) float32 for DIFFUS_POSE_F32_PER_RAY */
     const void* directions;     /* (P,R,3) or, if dir_pose_stride == 0, (R,3) shared by poses */
     int32_t pose_dtype;         /* DIFFUS_POSE_*                                             */
     int32_t product_f32;        /* POSE_F64 only: directions were float32, so k*dir rounds to
@@ -110,7 +114,7 @@ typedef struct DiffusRenderBwdArgs {
     float* grad_volume;         /* QUAD and TEXTURE volumes: a BRICK buffer.  Otherwise the
                                    same layout as fwd.volume (LINEAR (D,H,W), or diffus_brick_elems()
                                    floats for BRICK), ACCUMULATED into (caller zero-fills)    */
-    float* grad_sources;        /* (P,3) overwritten; trilinear only                         */
+    float* grad_sources;        /* (P,3) overwritten; trilinear only.  DIFFUS_POSE_F32_PER_RAY: (P,R,3), overwritten */
     float* grad_directions;     /* (P,R,3) overwritten; trilinear only (per pose, also when
                                    the directions were shared)                                */
     /* Fused forward + MSE loss + backward (one gather pass): when `target` is not NULL,
@@ -141,6 +145,8 @@ int32_t diffus_render_backward(const DiffusRenderBwdArgs* args, void* stream);
 
 /* Gauss-Newton system of each pose in one forward-mode pass: with res = frame - target and J the derivative of the frame
  * w.r.t. a rigid twist xi = (v, w) of the pose about its source (sources + v, directions rotated by Rot(w)),
+ * or -- DIFFUS_POSE_F32_PER_RAY -- about the pose's PIVOT c_p, the float64 mean of its R origins: a sample moves as
+ *   p_k = c_p + v + Rot(w) (s_i - c_p + k d_i),  i.e. origins c_p + v + Rot(w) (s_i - c_p) and directions Rot(w) d_i,
  *   loss[p] = sum res^2,   jtr[p] (6) = J^T res,   jtj[p] (6x6, full symmetric) = J^T J
  * over the R x (S-start) elements of pose p.  (2/n) jtr is the gradient of the mean-squared loss over n elements in twist
  * coordinates.  start > 0: the median-replaced coefficient's tangent is the mean of the tangents of the rays tied with the
@@ -174,7 +180,8 @@ int32_t diffus_sample_points(const DiffusVolume* volume, const float* points, in
                              float* values, int64_t* x, int64_t* y, int64_t* z, void* stream);
 /* Backward of diffus_trace_values (autograd through the reference's sampler, src/renderer.py:758 / grid_sample): grad_values
  * (P,R,S) -> grad_volume (layout of args->volume, ACCUMULATED), and for the trilinear sampler grad_sources
- * (P,3) + grad_directions (P,R,3) (both or neither).  workspace: P*R*12 bytes (256-aligned) for pose gradients. */
+ * (P,3) + grad_directions (P,R,3) (both or neither).  workspace: P*R*12 bytes (256-aligned) for pose gradients.
+ * DIFFUS_POSE_F32_PER_RAY: grad_sources is (P,R,3) and no workspace is needed. */
 int32_t diffus_trace_values_backward(const DiffusRenderArgs* args, const float* grad_values,
                                      float* grad_volume, float* grad_sources, float* grad_directions,
                                      void* workspace, int64_t workspace_bytes, void* stream);
@@ -204,6 +211,25 @@ int32_t diffus_fan_directions(const float* median, const float* hint, int64_t n_
 int32_t diffus_fan_directions_backward(const float* median, const float* hint, const float* grad_directions,
                                        int64_t n_poses, int64_t n_rays, double opening_angle,
                                        float* grad_median, float* grad_hint, void* stream);
+
+/* Array probes from pose PARAMETERS, one origin per ray (render them with DIFFUS_POSE_F32_PER_RAY).  centre, median, hint
+ * (P,3) float32; m^ and u^ as in diffus_fan_directions; origins and directions out (P,R,3) float32.
+ *   DIFFUS_PROBE_CONVEX (opening_angle, radius rho >= 0): d_i = cos(a_i) m^ + sin(a_i) u^ with a = linspace(-angle/2,
+ *     angle/2, R), formed exactly like diffus_fan_directions, and origin_i = centre + rho d_i (float64, then float32): the
+ *     elements sit on an arc of radius rho and fire along its normals.  rho = 0 is the sector probe, bit for bit.
+ *   DIFFUS_PROBE_LINEAR (width w > 0): d_i = m^ for every ray, origin_i = centre + t_i u^, t = linspace(-w/2, w/2, R).
+ * The backward maps d loss / d origins and d loss / d directions (P,R,3 each) to d loss / d centre, median and hint (P,3
+ * each, overwritten); float64 sums in a fixed order.  DIFFUS_E_SHAPE for a negative or non-finite radius, a width <= 0 or
+ * not finite, a non-finite opening angle (convex), DIFFUS_E_ENUM for an unknown kind. */
+#define DIFFUS_PROBE_CONVEX 0
+#define DIFFUS_PROBE_LINEAR 1
+int32_t diffus_probe_rays(int32_t kind, const float* centre, const float* median, const float* hint, int64_t n_poses,
+                          int64_t n_rays, double opening_angle, double radius, double width, float* origins,
+                          float* directions, void* stream);
+int32_t diffus_probe_rays_backward(int32_t kind, const float* centre, const float* median, const float* hint,
+                                   const float* grad_origins, const float* grad_directions, int64_t n_poses, int64_t n_rays,
+                                   double opening_angle, double radius, double width, float* grad_centre,
+                                   float* grad_median, float* grad_hint, void* stream);
 
 /* ImpedanceEstimator (src/impedance.py:6-17): Linear(1,32)-ReLU-Linear(32,32)-ReLU-Linear(32,1).
  * params is the 1153-float concatenation [W1(32x1) b1(32) W2(32x32 row-major out,in) b2(32)
