@@ -12,7 +12,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspa
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--path", default="piecewise", choices=["cuda_cores", "tensor", "piecewise"])
+    ap.add_argument("--path", default="piecewise", choices=["cuda_cores", "piecewise"])
     ap.add_argument("--n", type=int, default=256 ** 3)
     ap.add_argument("--iters", type=int, default=20)
     args = ap.parse_args()
@@ -25,7 +25,7 @@ def main():
     n = args.n
     x = (mri_phantom(256, "t2") / 1000.0).reshape(-1)[:n].contiguous().to(dev) if n <= 256 ** 3 else torch.rand(n, device=dev) * 3
     g = torch.randn(n, device=dev)
-    path = {"cuda_cores": ops.MLP_PATH_CUDA_CORES, "tensor": ops.MLP_PATH_TENSOR, "piecewise": ops.MLP_PATH_PIECEWISE}[args.path]
+    path = {"cuda_cores": ops.MLP_PATH_CUDA_CORES, "piecewise": ops.MLP_PATH_PIECEWISE}[args.path]
 
     def timed(fn):
         for _ in range(3):

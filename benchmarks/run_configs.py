@@ -133,8 +133,7 @@ def main():
         from diffus_b200.impedance import pack_params
         pk = pack_params(model).detach()
         gz = torch.randn(mri.numel(), device=dev)
-        paths = (("cuda cores", ops.MLP_PATH_CUDA_CORES), ("tcgen05 3xTF32", ops.MLP_PATH_TENSOR),
-                 ("piecewise-linear table", ops.MLP_PATH_PIECEWISE))
+        paths = (("cuda cores", ops.MLP_PATH_CUDA_CORES), ("piecewise-linear table", ops.MLP_PATH_PIECEWISE))
         for name, path in paths:
             with ops.mlp_path(path):
                 t_ms = timed(lambda: ops.mlp_fwd_impl(pk, mri.reshape(-1), None, 1e6, 400.0), args.iters)

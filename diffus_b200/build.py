@@ -18,7 +18,7 @@ SOURCES = [("render_kernels.cu", ["-DDIFFUS_LAYOUT_SLICE=1"], "render_kernels_br
            ("render_kernels.cu", ["-DDIFFUS_LAYOUT_SLICE=2"], "render_kernels_quad.o"),
            ("render_kernels.cu", ["-DDIFFUS_LAYOUT_SLICE=3"], "render_kernels_texture.o"),
            ("aux_kernels.cu", [], "aux_kernels.o"), ("render_kernels.cu", [], "render_kernels.o"),
-           ("api.cu", [], "api.o"), ("mlp_kernels.cu", [], "mlp_kernels.o"), ("mlp_tc_kernels.cu", [], "mlp_tc_kernels.o"),
+           ("api.cu", [], "api.o"), ("mlp_kernels.cu", [], "mlp_kernels.o"),
            ("mlp_pwl_kernels.cu", [], "mlp_pwl_kernels.o"),
            ("splat_kernels.cu", [], "splat_kernels.o"), ("preprocess_kernels.cu", [], "preprocess_kernels.o"),
            ("train_kernels.cu", [], "train_kernels.o"), ("loss_kernels.cu", [], "loss_kernels.o"),

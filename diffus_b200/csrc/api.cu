@@ -438,16 +438,19 @@ int32_t diffus_cone_directions(const double* median, int64_t n_poses, int64_t n_
     return cuda_rc(launch_cone_directions(median, n_poses, n_rays, opening_angle, out, (cudaStream_t)stream));
 }
 
+// value 2 selected a removed tensor-core path: rejected like any unknown value
+static bool mlp_path_valid(int32_t path) {
+    return path == DIFFUS_MLP_PATH_AUTO || path == DIFFUS_MLP_PATH_CUDA_CORES || path == DIFFUS_MLP_PATH_PIECEWISE;
+}
+
 int32_t diffus_mlp_forward_ex(const float* params, const float* x, const uint8_t* mask, int64_t n, float out_scale,
                               float fill, float* out, int32_t path, void* stream) {
     if (!params || !x || !out) return DIFFUS_E_NULL;
     if (n < 1) return DIFFUS_E_SHAPE;
-    if (path < DIFFUS_MLP_PATH_AUTO || path > DIFFUS_MLP_PATH_PIECEWISE) return DIFFUS_E_ENUM;
+    if (!mlp_path_valid(path)) return DIFFUS_E_ENUM;
     // volumes go through the piecewise-linear table; a handful of samples is not worth building it
     if (path == DIFFUS_MLP_PATH_PIECEWISE || (path == DIFFUS_MLP_PATH_AUTO && n >= 1024))
         return cuda_rc(launch_mlp_pwl_fwd(params, x, mask, n, out_scale, fill, out, (cudaStream_t)stream));
-    const bool tensor = path == DIFFUS_MLP_PATH_TENSOR;
-    if (tensor) return cuda_rc(launch_mlp_fwd_tc(params, x, mask, n, out_scale, fill, out, (cudaStream_t)stream));
     return cuda_rc(launch_mlp_fwd(params, x, mask, n, out_scale, fill, out, (cudaStream_t)stream));
 }
 
@@ -463,13 +466,12 @@ int32_t diffus_mlp_backward_ex(const float* params, const float* x, const uint8_
                                void* stream) {
     if (!params || !x || !grad_out || !grad_params) return DIFFUS_E_NULL;
     if (n < 1) return DIFFUS_E_SHAPE;
-    if (path < DIFFUS_MLP_PATH_AUTO || path > DIFFUS_MLP_PATH_PIECEWISE) return DIFFUS_E_ENUM;
+    if (!mlp_path_valid(path)) return DIFFUS_E_ENUM;
     if (!workspace || workspace_bytes < mlp_bwd_workspace_bytes(n)) return DIFFUS_E_WORKSPACE;
     if (((uintptr_t)workspace & 7u) != 0) return DIFFUS_E_WORKSPACE;
     if (path == DIFFUS_MLP_PATH_PIECEWISE || (path == DIFFUS_MLP_PATH_AUTO && n >= 1024))
         return cuda_rc(launch_mlp_pwl_bwd(params, x, mask, grad_out, n, out_scale, grad_params, workspace, (cudaStream_t)stream));
-    const bool tensor = path == DIFFUS_MLP_PATH_TENSOR;
-    return cuda_rc(launch_mlp_bwd(params, x, mask, grad_out, n, out_scale, grad_params, workspace, tensor, (cudaStream_t)stream));
+    return cuda_rc(launch_mlp_bwd(params, x, mask, grad_out, n, out_scale, grad_params, workspace, nullptr, (cudaStream_t)stream));
 }
 
 int32_t diffus_mlp_backward(const float* params, const float* x, const uint8_t* mask, const float* grad_out, int64_t n,

@@ -186,14 +186,10 @@ cudaError_t launch_ssim_bwd(const float* s, const float* y, int H, int W, int K,
 // mlp_kernels.cu
 cudaError_t launch_mlp_fwd(const float* params, const float* x, const uint8_t* mask, int64_t n, float out_scale,
                            float fill, float* out, cudaStream_t st);
-cudaError_t launch_mlp_fwd_tc(const float* params, const float* x, const uint8_t* mask, int64_t n, float out_scale,
-                              float fill, float* out, cudaStream_t st);
 int64_t mlp_bwd_workspace_bytes(int64_t n);
+// gate: NULL, or a device int; the kernels return at once when it reads 0 (the fallback behind the piecewise-linear path)
 cudaError_t launch_mlp_bwd(const float* params, const float* x, const uint8_t* mask, const float* grad_out, int64_t n,
-                           float out_scale, float* grad_params, void* workspace, bool tensor_cores, cudaStream_t st);
-cudaError_t launch_mlp_bwd_gated(const float* params, const float* x, const uint8_t* mask, const float* grad_out, int64_t n,
-                                 float out_scale, float* grad_params, void* workspace, const int* gate, cudaStream_t st);
-int mlp_bwd_tc_blocks(int64_t n);
+                           float out_scale, float* grad_params, void* workspace, const int* gate, cudaStream_t st);
 // mlp_pwl_kernels.cu: the scalar-input MLP as a piecewise-linear table
 int64_t mlp_pwl_bwd_workspace_bytes(int64_t n);
 cudaError_t launch_mlp_pwl_fwd(const float* params, const float* x, const uint8_t* mask, int64_t n, float out_scale, float fill,
@@ -202,7 +198,5 @@ cudaError_t launch_mlp_pwl_dx(const float* params, const float* x, const uint8_t
                               float out_scale, float* grad_x, cudaStream_t st);
 cudaError_t launch_mlp_pwl_bwd(const float* params, const float* x, const uint8_t* mask, const float* grad_out, int64_t n,
                                float out_scale, float* grad_params, void* workspace, cudaStream_t st);
-cudaError_t launch_mlp_bwd_tc(const float* params, const float* x, const uint8_t* mask, const float* grad_out, int64_t n,
-                              float out_scale, float* block_partials, int blocks, cudaStream_t st);
 
 }  // namespace diffus

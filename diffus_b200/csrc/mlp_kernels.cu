@@ -237,37 +237,18 @@ static int mlp_bwd_blocks(int64_t n) {
     return (int)max((int64_t)1, min(want, (int64_t)148 * 4));
 }
 
-static int64_t mlp_bwd_dense_workspace_bytes(int64_t n) {
-    int blocks = max(mlp_bwd_blocks(n), mlp_bwd_tc_blocks(n));
-    return (int64_t)blocks * DIFFUS_MLP_NPARAMS * sizeof(float);
-}
-
 // enough for every path: the piecewise-linear path's tables and partial moments, then the dense block partials (its fallback)
-int64_t mlp_bwd_workspace_bytes(int64_t n) { return mlp_pwl_bwd_workspace_bytes(n) + mlp_bwd_dense_workspace_bytes(n); }
-
-// the CUDA-core kernels behind a device-side gate (run only if *gate != 0)
-cudaError_t launch_mlp_bwd_gated(const float* params, const float* x, const uint8_t* mask, const float* grad_out, int64_t n,
-                                 float out_scale, float* grad_params, void* workspace, const int* gate, cudaStream_t st) {
-    const int blocks = mlp_bwd_blocks(n);
-    mlp_bwd_kernel<<<blocks, BWD_WARPS * 32, 0, st>>>(params, x, mask, grad_out, n, out_scale, (float*)workspace, gate);
-    mlp_bwd_reduce_kernel<<<(DIFFUS_MLP_NPARAMS + 127) / 128, 128, 0, st>>>((const float*)workspace, blocks, grad_params, gate);
-    return cudaGetLastError();
+int64_t mlp_bwd_workspace_bytes(int64_t n) {
+    return mlp_pwl_bwd_workspace_bytes(n) + (int64_t)mlp_bwd_blocks(n) * DIFFUS_MLP_NPARAMS * sizeof(float);
 }
 
 cudaError_t launch_mlp_bwd(const float* params, const float* x, const uint8_t* mask, const float* grad_out, int64_t n,
-                           float out_scale, float* grad_params, void* workspace, bool tensor_cores, cudaStream_t st) {
-    int blocks;
-    cudaError_t e;
-    if (tensor_cores) {
-        blocks = mlp_bwd_tc_blocks(n);
-        e = launch_mlp_bwd_tc(params, x, mask, grad_out, n, out_scale, (float*)workspace, blocks, st);
-    } else {
-        blocks = mlp_bwd_blocks(n);
-        mlp_bwd_kernel<<<blocks, BWD_WARPS * 32, 0, st>>>(params, x, mask, grad_out, n, out_scale, (float*)workspace, nullptr);
-        e = cudaGetLastError();
-    }
+                           float out_scale, float* grad_params, void* workspace, const int* gate, cudaStream_t st) {
+    const int blocks = mlp_bwd_blocks(n);
+    mlp_bwd_kernel<<<blocks, BWD_WARPS * 32, 0, st>>>(params, x, mask, grad_out, n, out_scale, (float*)workspace, gate);
+    cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    mlp_bwd_reduce_kernel<<<(DIFFUS_MLP_NPARAMS + 127) / 128, 128, 0, st>>>((const float*)workspace, blocks, grad_params, nullptr);
+    mlp_bwd_reduce_kernel<<<(DIFFUS_MLP_NPARAMS + 127) / 128, 128, 0, st>>>((const float*)workspace, blocks, grad_params, gate);
     return cudaGetLastError();
 }
 

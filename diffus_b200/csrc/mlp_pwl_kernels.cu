@@ -559,7 +559,7 @@ cudaError_t launch_mlp_pwl_bwd(const float* params, const float* x, const uint8_
     if (e != cudaSuccess) return e;
     // more than PWL_MAXR regions: the layered CUDA-core kernels run instead (they return at once when hdr[1] == 0)
     void* dense_ws = (char*)workspace + mlp_pwl_bwd_workspace_bytes(n);
-    return launch_mlp_bwd_gated(params, x, mask, grad_out, n, out_scale, grad_params, dense_ws, hdr + 1, st);
+    return launch_mlp_bwd(params, x, mask, grad_out, n, out_scale, grad_params, dense_ws, hdr + 1, st);
 }
 
 }  // namespace diffus

@@ -1050,12 +1050,13 @@ class SplatFunction(torch.autograd.Function):
 # ---------------------------------------------------------------------------------------
 # MLP
 # ---------------------------------------------------------------------------------------
-MLP_PATH_AUTO, MLP_PATH_CUDA_CORES, MLP_PATH_TENSOR, MLP_PATH_PIECEWISE = 0, 1, 2, 3
+MLP_PATH_AUTO, MLP_PATH_CUDA_CORES, MLP_PATH_PIECEWISE = 0, 1, 3
 _MLP_PATH = MLP_PATH_AUTO      # tests and benchmarks pin a path through mlp_path(); AUTO = the piecewise-linear table for volumes
 
 
 class mlp_path:
-    """Context manager pinning the MLP forward to the CUDA-core or the tcgen05 kernel (default: automatic)."""
+    """Context manager pinning the MLP forward and weight gradient to the CUDA-core kernels or the piecewise-linear
+    table (default: automatic)."""
 
     def __init__(self, path: int):
         self.path = path

@@ -3,7 +3,7 @@
 
 One step, everything in the brick layout the gathers use (no layout conversions inside the step):
 
-    Z_bricks  = out_scale * MLP(mri_bricks)           tcgen05 kernel, written once
+    Z_bricks  = out_scale * MLP(mri_bricks)           piecewise-linear table, written once
     loss, dZ  = fused render + MSE + backward          dZ scattered with red.add into brick-local lines
     dWeights  = MLP backward from (mri_bricks, dZ)     atomic-free block partials, fixed-order reduction
     all-reduce of the 1 153 weight gradients (+ shared-pose gradients) across ranks, one flat buffer

@@ -241,12 +241,11 @@ int32_t diffus_mlp_forward(const float* params, const float* x, const uint8_t* m
 /* Same with an explicit execution path.  PIECEWISE: a ReLU network of ONE scalar is a piecewise-linear function of it (at most
  * 1088 breakpoints, ~60 in practice); every CTA builds the table of regions in float64 from the 1153 parameters and a voxel
  * costs a binary search and one fused multiply-add -- an HBM-bound pass, no dense contraction left (falls back to the layered
- * evaluation for weights with more than 256 regions).  The layered paths evaluate layer 2 (M x 32 x 32) as fp32 FMAs on the
- * CUDA cores or as a 3xTF32-split tcgen05.mma with the accumulator in TMEM (fp32-grade accuracy; 128-voxel tiles).
+ * evaluation for weights with more than 256 regions).  CUDA_CORES evaluates the layers, layer 2 (M x 32 x 32) as fp32 FMAs.
  * AUTO = PIECEWISE for n >= 1024, CUDA cores below. */
 #define DIFFUS_MLP_PATH_AUTO 0
 #define DIFFUS_MLP_PATH_CUDA_CORES 1
-#define DIFFUS_MLP_PATH_TENSOR 2
+/* 2 is rejected (DIFFUS_E_ENUM): it selected a removed tensor-core path and must not be reused. */
 #define DIFFUS_MLP_PATH_PIECEWISE 3
 int32_t diffus_mlp_forward_ex(const float* params, const float* x, const uint8_t* mask,
                               int64_t n, float out_scale, float fill, float* out, int32_t path,
@@ -261,8 +260,7 @@ int32_t diffus_mlp_backward(const float* params, const float* x, const uint8_t* 
                             void* stream);
 /* Same with an explicit path (DIFFUS_MLP_PATH_*).  PIECEWISE: inside a region d mlp / d params is affine in x, so the pass
  * over the volume only accumulates sum g and sum g x per region (float64 bins, no atomics) and a second small kernel turns
- * the moments into the 1153 gradients.  On the tensor-core path the layer-2 recompute, d/dH1 and the dW2 / db2 reductions
- * over voxels are 3xTF32 tcgen05.mma with TMEM accumulators. */
+ * the moments into the 1153 gradients. */
 int32_t diffus_mlp_backward_ex(const float* params, const float* x, const uint8_t* mask,
                                const float* grad_out, int64_t n, float out_scale,
                                float* grad_params, void* workspace, int64_t workspace_bytes,

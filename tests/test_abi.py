@@ -140,6 +140,8 @@ def test_argument_validation_without_a_device(lib):
     assert lib.diffus_gather_probe(None, 1 << 20, 64, 256, 1, 0x1000, None) == -1
     assert lib.diffus_gather_probe(0x1000, 1 << 20, 60, 256, 1, 0x1000, None) == -2   # reads per thread: multiples of 8
     assert lib.diffus_mlp_backward_ex(0x1000, 0x1000, None, 0x1000, 64, 1.0, 0x1000, 0x1000, 1 << 20, 9, None) == -3
+    assert lib.diffus_mlp_backward_ex(0x1000, 0x1000, None, 0x1000, 64, 1.0, 0x1000, 0x1000, 1 << 20, 2, None) == -3  # removed path
+    assert lib.diffus_mlp_forward_ex(0x1000, 0x1000, None, 64, 1.0, 0.0, 0x1000, 2, None) == -3
     assert lib.diffus_mlp_backward_ex(0x1000, 0x1000, None, 0x1000, 64, 1.0, 0x1000, 0x1000, 16, 3, None) == -4   # piecewise path: workspace too small
     assert lib.diffus_mlp_input_grad(0x1000, None, None, 0x1000, 64, 1.0, 0x1000, None) == -1
     assert lib.diffus_conv1d_rows_forward(0x1000, 4, 60, None, 9, 4, 0x1000, None) == -1
