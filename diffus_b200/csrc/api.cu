@@ -27,7 +27,12 @@ cudaError_t prepare_kernel(const void* kernel, int carveout_pct) {
                              carveout_pct >= 100 ? (int)cudaSharedmemCarveoutMaxShared : carveout_pct);
     if (e != cudaSuccess) return e;
     if (it == done.end()) {
-        e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MAX_DYNAMIC_SMEM);
+        // the opt-in limit covers static + dynamic shared memory: a kernel with static arrays (the median select's
+        // histogram) is refused the whole 227 KB as dynamic memory
+        cudaFuncAttributes fa;
+        e = cudaFuncGetAttributes(&fa, kernel);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(MAX_DYNAMIC_SMEM - fa.sharedSizeBytes));
         if (e != cudaSuccess) return e;
     }
     done[key] = carveout_pct;

@@ -150,9 +150,10 @@ __global__ void median_backward_kernel(const RenderParams p, const int32_t* __re
 cudaError_t launch_median_backward(const RenderParams& p, int sampler, int layout, int pose64,
                                    const int32_t* tie_count, bool pose_grad, bool vol_grad, cudaStream_t st) {
     if (sampler == DIFFUS_SAMPLER_NEAREST) pose_grad = false;
+    if (!pose_grad && !vol_grad) return cudaSuccess;      // loss / frame only: no gradient flows through the median
 #define DIFFUS_MB(PG, VG) median_backward_kernel<S_, L_, P64_, PG, VG><<<(unsigned)p.n_poses, 32, 0, st>>>(p, tie_count)
     DIFFUS_DISPATCH(if (pose_grad && vol_grad) DIFFUS_MB(true, true); else if (pose_grad) DIFFUS_MB(true, false);
-                    else DIFFUS_MB(false, true); return cudaGetLastError())
+                    else if (vol_grad) DIFFUS_MB(false, true); return cudaGetLastError())
 #undef DIFFUS_MB
     return cudaErrorInvalidValue;
 }
@@ -285,10 +286,11 @@ __global__ void trace_values_bwd_kernel(const RenderParams p, const float* __res
 cudaError_t launch_trace_values_bwd(const RenderParams& p, int sampler, int layout, int pose64, const float* gval,
                                     bool pose_grad, bool vol_grad, cudaStream_t st) {
     if (sampler == DIFFUS_SAMPLER_NEAREST) pose_grad = false;
+    if (!pose_grad && !vol_grad) return cudaSuccess;      // nothing requested: nothing to write
     unsigned grid = (unsigned)((p.total_rays + 3) / 4);
 #define DIFFUS_TB(PG, VG) trace_values_bwd_kernel<S_, L_, P64_, PG, VG><<<grid, 128, 0, st>>>(p, gval)
     DIFFUS_DISPATCH(if (pose_grad && vol_grad) DIFFUS_TB(true, true); else if (pose_grad) DIFFUS_TB(true, false);
-                    else DIFFUS_TB(false, true); return cudaGetLastError())
+                    else if (vol_grad) DIFFUS_TB(false, true); return cudaGetLastError())
 #undef DIFFUS_TB
     return cudaErrorInvalidValue;
 }

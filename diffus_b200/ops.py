@@ -444,8 +444,10 @@ def render_mse_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: 
         ws = torch.empty((max(wbytes, 1),), dtype=torch.uint8, device=dev)
         b.workspace, b.workspace_bytes = ws.data_ptr(), wbytes
         _lib.check(lib.diffus_render_backward(C.byref(b), _stream(dev)), "diffus_render_backward (fused MSE)")
-        # fused kernel + loss reduction (+ the d/dsources reduction: the same launch as the loss up to 2^18 rays) (+ median)
-        _count(2 + (2 if start > 0 else 0) + (1 if need_pose and sources.dim() == 2 and P * R > (1 << 18) else 0))
+        # fused kernel + loss reduction (+ the d/dsources reduction: the same launch as the loss up to 2^18 rays) (+ median,
+        # and its backward when a gradient is requested)
+        n_median = (2 if need_volume or need_pose else 1) if start > 0 else 0
+        _count(2 + n_median + (1 if need_pose and sources.dim() == 2 and P * R > (1 << 18) else 0))
         if need_volume and use_bricks and not keep_brick_grad:
             gvol = from_bricks(gvol, dims)
     return loss, frame, gvol, gsrc, gdir
