@@ -72,6 +72,19 @@ class DiffusGaussNewtonArgs(C.Structure):
     ]
 
 
+class DiffusGaussNewtonSweepArgs(C.Structure):
+    _fields_ = [
+        ("fwd", DiffusRenderArgs),
+        ("target", C.c_void_p),
+        ("pivot", C.c_void_p),
+        ("loss", C.c_void_p),
+        ("jtr", C.c_void_p),
+        ("jtj", C.c_void_p),
+        ("workspace", C.c_void_p),
+        ("workspace_bytes", C.c_int64),
+    ]
+
+
 _P = C.POINTER
 _vp, _i32, _i64, _f32, _f64 = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_double
 
@@ -86,6 +99,8 @@ SIGNATURES = {
     "diffus_render_backward": (_i32, [_P(DiffusRenderBwdArgs), _vp]),
     "diffus_render_gauss_newton_workspace_bytes": (_i64, [_P(DiffusGaussNewtonArgs)]),
     "diffus_render_gauss_newton": (_i32, [_P(DiffusGaussNewtonArgs), _vp]),
+    "diffus_render_gauss_newton_sweep_workspace_bytes": (_i64, [_P(DiffusGaussNewtonSweepArgs)]),
+    "diffus_render_gauss_newton_sweep": (_i32, [_P(DiffusGaussNewtonSweepArgs), _vp]),
     "diffus_ray_indices": (_i32, [_P(DiffusRenderArgs), _vp, _vp, _vp, _vp]),
     "diffus_trace_values": (_i32, [_P(DiffusRenderArgs), _vp, _vp]),
     "diffus_sample_points": (_i32, [_P(DiffusVolume), _vp, _i64, _i32, _vp, _vp, _vp, _vp, _vp]),

@@ -217,6 +217,38 @@ GnWorkspace gn_workspace(const DiffusGaussNewtonArgs* g, void* base) {
     return w;
 }
 
+// sweep workspace: [fwd workspace | median tangent (P*6) | per-ray partials (P*R*32) | range sums (32 doubles per range) |
+// pivot (3 doubles, when the caller passes none)]
+struct GnSweepWorkspace {
+    FwdWorkspace fwd;
+    float* med_tan;
+    float* partial;
+    double* range_sum;
+    double* pivot;
+    int64_t bytes;
+};
+GnSweepWorkspace gn_sweep_workspace(const DiffusGaussNewtonSweepArgs* g, void* base) {
+    GnSweepWorkspace w{};
+    const DiffusRenderArgs* a = &g->fwd;
+    const int64_t rays = a->n_poses * a->n_rays;
+    w.fwd = fwd_workspace(a, base);
+    int64_t off = w.fwd.bytes;
+    if (a->start > 0) {
+        w.med_tan = (float*)((char*)base + off);
+        off += align_up(a->n_poses * 24, 256);
+    }
+    w.partial = (float*)((char*)base + off);
+    off += align_up(rays * 128, 256);
+    w.range_sum = (double*)((char*)base + off);
+    off += align_up(gn_sweep_ranges(rays) * 256, 256);
+    if (!g->pivot) {
+        w.pivot = (double*)((char*)base + off);
+        off += 256;
+    }
+    w.bytes = off;
+    return w;
+}
+
 }  // namespace
 
 extern "C" {
@@ -360,10 +392,49 @@ int32_t diffus_render_gauss_newton(const DiffusGaussNewtonArgs* g, void* stream)
         ce = launch_first_refl_median(p, a->sampler, a->volume.layout, 0, w.fwd.median, w.fwd.tie_count, st);
         if (ce != cudaSuccess) return (int32_t)ce;
         p.median = w.fwd.median;
-        ce = launch_gn_median_tangent(p, a->volume.layout, w.fwd.tie_count, w.pivot, w.med_tan, st);
+        ce = launch_gn_median_tangent(p, a->volume.layout, w.pivot ? GN_LEVER_POSE : GN_LEVER_SOURCE, w.fwd.tie_count, w.pivot,
+                                      w.med_tan, st);
         if (ce != cudaSuccess) return (int32_t)ce;
     }
     return cuda_rc(launch_render_gn(p, a->volume.layout, w.med_tan, w.pivot, w.partial, g->loss, g->jtr, g->jtj, st));
+}
+
+int64_t diffus_render_gauss_newton_sweep_workspace_bytes(const DiffusGaussNewtonSweepArgs* g) {
+    if (!g) return 0;
+    return gn_sweep_workspace(g, nullptr).bytes;
+}
+
+int32_t diffus_render_gauss_newton_sweep(const DiffusGaussNewtonSweepArgs* g, void* stream) {
+    if (!g) return DIFFUS_E_NULL;
+    const DiffusRenderArgs* a = &g->fwd;
+    int32_t e = check_render(a, false);
+    if (e) return e;
+    if (!g->target || !g->loss || !g->jtr || !g->jtj) return DIFFUS_E_NULL;
+    if (a->sampler != DIFFUS_SAMPLER_TRILINEAR || a->pose_dtype == DIFFUS_POSE_F64) return DIFFUS_E_UNSUPPORTED;
+    GnSweepWorkspace w = gn_sweep_workspace(g, g->workspace);
+    if (!g->workspace || g->workspace_bytes < w.bytes) return DIFFUS_E_WORKSPACE;
+    cudaStream_t st = (cudaStream_t)stream;
+    RenderParams p = pack(a);
+    p.frame = nullptr;
+    p.seg_prefix = nullptr;
+    p.target = g->target;
+    const double* pivot = g->pivot;
+    cudaError_t ce;
+    if (!pivot) {   // one source per pose stands for its R rays: the mean of the P sources is the mean of all P*R origins
+        const int64_t rows = per_ray(a) ? a->n_poses * a->n_rays : a->n_poses;
+        ce = launch_gn_sweep_pivot((const float*)a->sources, rows, w.range_sum, w.pivot, st);
+        if (ce != cudaSuccess) return (int32_t)ce;
+        pivot = w.pivot;
+    }
+    if (a->start > 0) {
+        ce = launch_first_refl_median(p, a->sampler, a->volume.layout, 0, w.fwd.median, w.fwd.tie_count, st);
+        if (ce != cudaSuccess) return (int32_t)ce;
+        p.median = w.fwd.median;
+        ce = launch_gn_median_tangent(p, a->volume.layout, GN_LEVER_SWEEP, w.fwd.tie_count, pivot, w.med_tan, st);
+        if (ce != cudaSuccess) return (int32_t)ce;
+    }
+    return cuda_rc(launch_render_gn_sweep(p, a->volume.layout, w.med_tan, pivot, w.partial, w.range_sum, g->loss, g->jtr, g->jtj,
+                                          st));
 }
 
 int32_t diffus_ray_indices(const DiffusRenderArgs* a, int64_t* x, int64_t* y, int64_t* z, void* stream) {

@@ -4,7 +4,10 @@
 // so every sample's impedance has the tangent dZ_k / dxi = (grad Z_k, k (d_i x grad Z_k)) -- the spatial gradient the trilinear
 // gather already forms for the pose-gradient kernels.  With one origin s_i per ray (array probes) the probe turns about its
 // pivot c, the float64 mean of the pose's origins: p_k(xi) = c + v + Rot(w) (s_i - c + k d_i), tangent (grad Z_k,
-// (o_i + k d_i) x grad Z_k) with the lever o_i = s_i - c (the PER_RAY instantiations; the per-pose ones are unchanged).  The transfer-matrix prefix is carried as a DUAL pair (P, Pdot_1..6):
+// (o_i + k d_i) x grad Z_k) with the lever o_i = s_i - c (the GN_LEVER_POSE instantiations; the per-pose ones are unchanged).  A
+// tracked sweep shares ONE twist and one pivot c among all poses (GN_LEVER_SWEEP): the lever is o_i = s_i - c with s_i the pose's
+// source or the ray's own origin, and the per-ray partials of every pose are summed into one system (gn_sweep_sum_kernel).
+// The transfer-matrix prefix is carried as a DUAL pair (P, Pdot_1..6):
 // (P, Pdot) (M, Mdot) = (P M, Pdot M + P Mdot) is associative, so the march keeps the structure of the forward kernel --
 // lane-local chunk products, one warp scan, a second sweep -- with no reverse sweep and no prefix pre-pass.  Per column
 //     rdot  = ((Zdot_c - Zdot_{c-1}) - r (Zdot_{c-1} + Zdot_c)) / (Z_{c-1} + Z_c)      (d of (Z_c - Z_{c-1}) / (Z_{c-1} + Z_c))
@@ -89,11 +92,11 @@ __device__ __forceinline__ D2 d2_load(const float* s) {
     return x;
 }
 
-// the lane's sample tangent (grad Z, k (d x grad Z)); PER_RAY: (grad Z, (o + k d) x grad Z) with the ray's lever o
-template <bool PER_RAY>
+// the lane's sample tangent (grad Z, k (d x grad Z)); with a pivot: (grad Z, (o + k d) x grad Z) with the ray's lever o
+template <int LEVER>
 __device__ __forceinline__ void sample_tangent(const float d[3], const float o[3], const float g[3], float kf, float t[6]) {
     t[0] = g[0]; t[1] = g[1]; t[2] = g[2];
-    if (PER_RAY) {
+    if (LEVER != GN_LEVER_SOURCE) {
         const float a0 = fmaf(kf, d[0], o[0]), a1 = fmaf(kf, d[1], o[1]), a2 = fmaf(kf, d[2], o[2]);
         t[3] = a1 * g[2] - a2 * g[1];
         t[4] = a2 * g[0] - a0 * g[2];
@@ -105,11 +108,15 @@ __device__ __forceinline__ void sample_tangent(const float d[3], const float o[3
     }
 }
 
-// the ray's lever o = s_i - c about its pose's pivot (float64 difference, one rounding)
-template <bool PER_RAY>
+// the ray's lever o = s_i - c about its pose's pivot, or about the sweep's one pivot (float64 difference, one rounding)
+template <int LEVER>
 __device__ __forceinline__ void ray_lever(const RaySetup<false>& rs, const double* __restrict__ pivot, int64_t pose, float o[3]) {
 #pragma unroll
-    for (int a = 0; a < 3; ++a) o[a] = PER_RAY ? (float)((double)rs.s[a] - __ldg(pivot + pose * 3 + a)) : 0.f;
+    for (int a = 0; a < 3; ++a) {
+        if (LEVER == GN_LEVER_POSE) o[a] = (float)((double)rs.s[a] - __ldg(pivot + pose * 3 + a));
+        else if (LEVER == GN_LEVER_SWEEP) o[a] = (float)((double)rs.s[a] - __ldg(pivot + a));
+        else o[a] = 0.f;
+    }
 }
 
 __device__ __forceinline__ int64_t gn_pose_of_ray(int64_t ray, const RenderParams& p) {
@@ -121,7 +128,7 @@ __device__ __forceinline__ int64_t gn_pose_of_ray(int64_t ray, const RenderParam
 // the neighbour's by one shuffle, and the column's r, rdot, attenuation and target parked in shared memory.  Chunk phase (lane =
 // 16 consecutive columns): the dual chunk product, one warp scan, the second sweep forming e, J and the accumulators.  The dual
 // prefix entering the next pass goes through shared memory, so it is not live during the gathers.
-template <int LAYOUT, bool PER_RAY>
+template <int LAYOUT, int LEVER>
 __global__ void __launch_bounds__(128) render_gn_kernel(const RenderParams p, const float* __restrict__ med_tan,
                                                         const double* __restrict__ pivot, float* __restrict__ partial) {
     using G = FwdGeo;
@@ -136,7 +143,7 @@ __global__ void __launch_bounds__(128) render_gn_kernel(const RenderParams p, co
     RaySetup<false> rs;
     rs.load(p.sources, p.directions, pose, ray - pose * p.n_rays, p.src_pose_stride, p.src_ray_stride, p.dir_pose_stride, 0);
     float lever[3];
-    ray_lever<PER_RAY>(rs, pivot, pose, lever);
+    ray_lever<LEVER>(rs, pivot, pose, lever);
     const bool has_med = p.median != nullptr;
     const float med = has_med ? __ldg(p.median + pose) : 0.f;
     float mt[6];
@@ -174,7 +181,7 @@ __global__ void __launch_bounds__(128) render_gn_kernel(const RenderParams p, co
                 float z = 0.f;
                 if (ok) z = fe[u].template finish<true>(g);
                 float tz[6];
-                sample_tangent<PER_RAY>(rs.d, lever, g, (float)(p.start + c), tz);
+                sample_tangent<LEVER>(rs.d, lever, g, (float)(p.start + c), tz);
                 float zp = __shfl_up_sync(FULL, z, 1);
                 float tp[6];
 #pragma unroll
@@ -312,7 +319,7 @@ __global__ void __launch_bounds__(128) gn_reduce_kernel(const float* __restrict_
 // mean of the tangents of the rays tied with it (tie_count from first_refl_median_kernel; a NaN median has no tangent).  The
 // coefficient is formed exactly like first_refl_median_kernel does (same expression, IEEE division), so the ties it counted are
 // the ties found here.  One warp per pose.
-template <int LAYOUT, bool PER_RAY>
+template <int LAYOUT, int LEVER>
 __global__ void gn_median_tangent_kernel(const RenderParams p, const int32_t* __restrict__ tie_count, const double* __restrict__ pivot,
                                          float* __restrict__ med_tan) {
     const int64_t pose = blockIdx.x;
@@ -330,9 +337,9 @@ __global__ void gn_median_tangent_kernel(const RenderParams p, const int32_t* __
                                                                                rs.coord(2, k + 1), g1);
         if (!((z1 - z0) / (z0 + z1) == med)) continue;
         float lever[3], t0[6], t1[6];
-        ray_lever<PER_RAY>(rs, pivot, pose, lever);
-        sample_tangent<PER_RAY>(rs.d, lever, g0, (float)k, t0);
-        sample_tangent<PER_RAY>(rs.d, lever, g1, (float)(k + 1), t1);
+        ray_lever<LEVER>(rs, pivot, pose, lever);
+        sample_tangent<LEVER>(rs.d, lever, g0, (float)k, t0);
+        sample_tangent<LEVER>(rs.d, lever, g1, (float)(k + 1), t1);
         const float sum = z0 + z1;
         const float w = 2.f / (sum * sum);
 #pragma unroll
@@ -365,6 +372,102 @@ __global__ void __launch_bounds__(128) gn_pivot_kernel(const float* __restrict__
     }
 }
 
+// Tracked sweeps.  A sum over all P*R rows is split into contiguous ranges whose length follows from the row count alone
+// (gn_sweep_range_rows), each range summed by one CTA in a fixed order, then the range sums by one CTA in a fixed order: no
+// atomics, the same additions in the same order on every run and every device.
+constexpr int SWEEP_THREADS = 256;
+constexpr int64_t SWEEP_MAX_RANGES = 512;
+
+static int64_t gn_sweep_range_rows(int64_t rows) {
+    const int64_t len = (rows + SWEEP_MAX_RANGES - 1) / SWEEP_MAX_RANGES;
+    return len > 64 ? len : 64;
+}
+
+int64_t gn_sweep_ranges(int64_t rows) {
+    const int64_t len = gn_sweep_range_rows(rows);
+    return (rows + len - 1) / len;
+}
+
+// column sums of n rows of 32 values in double: eight row groups of 32 lanes (one lane per column), two chains each, then the
+// groups in a fixed tree.  The result is valid in threads 0..31.
+template <typename T>
+__device__ __forceinline__ double sweep_sum_columns(const T* __restrict__ rows, int64_t n, double (*part)[32]) {
+    const int t = threadIdx.x & 31, grp = threadIdx.x >> 5;
+    const T* src = rows + t;
+    double a0 = 0.0, a1 = 0.0;
+    int64_t r = grp;
+#pragma unroll 4
+    for (; r + 8 < n; r += 16) { a0 += (double)__ldg(src + r * 32); a1 += (double)__ldg(src + (r + 8) * 32); }
+    if (r < n) a0 += (double)__ldg(src + r * 32);
+    part[grp][t] = a0 + a1;
+    __syncthreads();
+    return ((part[0][t] + part[1][t]) + (part[2][t] + part[3][t])) + ((part[4][t] + part[5][t]) + (part[6][t] + part[7][t]));
+}
+
+// stage 1: CTA b sums the 32-float per-ray partials of rays [b len, (b + 1) len)
+__global__ void __launch_bounds__(SWEEP_THREADS) gn_sweep_range_kernel(const float* __restrict__ partial, int64_t n_rows, int64_t len,
+                                                                       double* __restrict__ range_sum) {
+    __shared__ double part[SWEEP_THREADS / 32][32];
+    const int64_t lo = (int64_t)blockIdx.x * len;
+    const double v = sweep_sum_columns(partial + lo * 32, n_rows - lo < len ? n_rows - lo : len, part);
+    if (threadIdx.x < 32) range_sum[(int64_t)blockIdx.x * 32 + threadIdx.x] = v;
+}
+
+// stage 2 (one CTA): the range sums -> loss, Jtr (6) and the symmetric JtJ (6x6), all double
+__global__ void __launch_bounds__(SWEEP_THREADS) gn_sweep_sum_kernel(const double* __restrict__ range_sum, int64_t n_ranges,
+                                                                     double* __restrict__ loss, double* __restrict__ jtr,
+                                                                     double* __restrict__ jtj) {
+    __shared__ double part[SWEEP_THREADS / 32][32];
+    const double v = sweep_sum_columns(range_sum, n_ranges, part);
+    const int t = threadIdx.x;
+    if (t == 0) {
+        loss[0] = v;
+    } else if (t < 7) {
+        jtr[t - 1] = v;
+    } else if (t < 28) {
+        int q = t - 7, a = 0;
+        while (q >= 6 - a) { q -= 6 - a; ++a; }
+        const int b = a + q;
+        jtj[a * 6 + b] = v;
+        jtj[b * 6 + a] = v;
+    }
+}
+
+// The sweep's pivot: the mean of n_rows origins (3 floats each) in double.  Stage 1 (FINAL = false) writes the three sums of
+// rows [b len, (b + 1) len) per CTA, stage 2 (FINAL, one CTA) sums those and divides by `count`.  Thread i takes rows i, i + 256,
+// ...; each warp folds by a butterfly and the eight warps in a fixed tree.
+template <typename T, bool FINAL>
+__global__ void __launch_bounds__(SWEEP_THREADS) gn_sweep_pivot_kernel(const T* __restrict__ rows, int64_t n_rows, int64_t len,
+                                                                       int64_t count, double* __restrict__ out) {
+    __shared__ double part[SWEEP_THREADS / 32][3];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t lo = (int64_t)blockIdx.x * len, hi = lo + len < n_rows ? lo + len : n_rows;
+    double a[3] = {0.0, 0.0, 0.0};
+    for (int64_t r = lo + threadIdx.x; r < hi; r += SWEEP_THREADS)
+#pragma unroll
+        for (int j = 0; j < 3; ++j) a[j] += (double)__ldg(rows + r * 3 + j);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+#pragma unroll
+        for (int d = 16; d > 0; d >>= 1) a[j] += __shfl_xor_sync(FULL, a[j], d);
+        if (lane == 0) part[warp][j] = a[j];
+    }
+    __syncthreads();
+    if (threadIdx.x >= 3) return;
+    const int j = threadIdx.x;
+    const double s = ((part[0][j] + part[1][j]) + (part[2][j] + part[3][j])) + ((part[4][j] + part[5][j]) + (part[6][j] + part[7][j]));
+    out[(int64_t)blockIdx.x * 3 + j] = FINAL ? s / (double)count : s;
+}
+
+cudaError_t launch_gn_sweep_pivot(const float* origins, int64_t n_rows, double* range_ws, double* pivot, cudaStream_t st) {
+    const int64_t len = gn_sweep_range_rows(n_rows), g = (n_rows + len - 1) / len;
+    gn_sweep_pivot_kernel<float, false><<<(unsigned)g, SWEEP_THREADS, 0, st>>>(origins, n_rows, len, n_rows, range_ws);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    gn_sweep_pivot_kernel<double, true><<<1, SWEEP_THREADS, 0, st>>>(range_ws, g, g, n_rows, pivot);
+    return cudaGetLastError();
+}
+
 cudaError_t launch_gn_pivot(const float* sources, int64_t n_poses, int64_t n_rays, double* pivot, cudaStream_t st) {
     gn_pivot_kernel<<<(unsigned)((n_poses + 3) / 4), 128, 0, st>>>(sources, n_poses, n_rays, pivot);
     return cudaGetLastError();
@@ -384,36 +487,52 @@ static int gn_warps_per_block(int64_t total_rays) {
         case DIFFUS_LAYOUT_TEXTURE: { constexpr int L_ = DIFFUS_LAYOUT_TEXTURE; __VA_ARGS__; } \
     }
 
-cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, const int32_t* tie_count, const double* pivot, float* med_tan,
-                                     cudaStream_t st) {
-    if (pivot) {
-        DIFFUS_GN_LAYOUTS(gn_median_tangent_kernel<L_, true><<<(unsigned)p.n_poses, 32, 0, st>>>(p, tie_count, pivot, med_tan);
-                          return cudaGetLastError())
-    } else {
-        DIFFUS_GN_LAYOUTS(gn_median_tangent_kernel<L_, false><<<(unsigned)p.n_poses, 32, 0, st>>>(p, tie_count, pivot, med_tan);
-                          return cudaGetLastError())
+#define DIFFUS_GN_LEVERS(...)                                                                      \
+    switch (lever) {                                                                                \
+        case GN_LEVER_SOURCE: { constexpr int V_ = GN_LEVER_SOURCE; DIFFUS_GN_LAYOUTS(__VA_ARGS__) break; } \
+        case GN_LEVER_POSE: { constexpr int V_ = GN_LEVER_POSE; DIFFUS_GN_LAYOUTS(__VA_ARGS__) break; }     \
+        case GN_LEVER_SWEEP: { constexpr int V_ = GN_LEVER_SWEEP; DIFFUS_GN_LAYOUTS(__VA_ARGS__) break; }   \
     }
+
+cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, int lever, const int32_t* tie_count, const double* pivot,
+                                     float* med_tan, cudaStream_t st) {
+    DIFFUS_GN_LEVERS(gn_median_tangent_kernel<L_, V_><<<(unsigned)p.n_poses, 32, 0, st>>>(p, tie_count, pivot, med_tan);
+                     return cudaGetLastError())
+    return cudaErrorInvalidValue;
+}
+
+// the march: one 32-float partial per ray
+static cudaError_t launch_gn_march(const RenderParams& p, int layout, int lever, const float* med_tan, const double* pivot,
+                                   float* partial, cudaStream_t st) {
+    const int wpb = gn_warps_per_block(p.total_rays);
+    const size_t smem = (size_t)wpb * GN_SMEM_PER_WARP * sizeof(float);
+    const unsigned grid = (unsigned)((p.total_rays + wpb - 1) / wpb);
+    DIFFUS_GN_LEVERS(auto k = render_gn_kernel<L_, V_>; cudaError_t e = ensure_smem(k, smem); if (e != cudaSuccess) return e;
+                     k<<<grid, wpb * 32, smem, st>>>(p, med_tan, pivot, partial); return cudaGetLastError())
     return cudaErrorInvalidValue;
 }
 
 cudaError_t launch_render_gn(const RenderParams& p, int layout, const float* med_tan, const double* pivot, float* partial, float* loss,
                              float* jtr, float* jtj, cudaStream_t st) {
-    const int wpb = gn_warps_per_block(p.total_rays);
-    const size_t smem = (size_t)wpb * GN_SMEM_PER_WARP * sizeof(float);
-    const unsigned grid = (unsigned)((p.total_rays + wpb - 1) / wpb);
-    cudaError_t e = cudaErrorInvalidValue;
-    if (pivot) {
-        DIFFUS_GN_LAYOUTS(auto k = render_gn_kernel<L_, true>; e = ensure_smem(k, smem); if (e != cudaSuccess) return e;
-                          k<<<grid, wpb * 32, smem, st>>>(p, med_tan, pivot, partial); e = cudaGetLastError(); break)
-    } else {
-        DIFFUS_GN_LAYOUTS(auto k = render_gn_kernel<L_, false>; e = ensure_smem(k, smem); if (e != cudaSuccess) return e;
-                          k<<<grid, wpb * 32, smem, st>>>(p, med_tan, pivot, partial); e = cudaGetLastError(); break)
-    }
+    cudaError_t e = launch_gn_march(p, layout, pivot ? GN_LEVER_POSE : GN_LEVER_SOURCE, med_tan, pivot, partial, st);
     if (e != cudaSuccess) return e;
     gn_reduce_kernel<<<(unsigned)p.n_poses, 128, 0, st>>>(partial, p.n_rays, loss, jtr, jtj);
     return cudaGetLastError();
 }
 
+cudaError_t launch_render_gn_sweep(const RenderParams& p, int layout, const float* med_tan, const double* pivot, float* partial,
+                                   double* range_ws, double* loss, double* jtr, double* jtj, cudaStream_t st) {
+    cudaError_t e = launch_gn_march(p, layout, GN_LEVER_SWEEP, med_tan, pivot, partial, st);
+    if (e != cudaSuccess) return e;
+    const int64_t len = gn_sweep_range_rows(p.total_rays), g = (p.total_rays + len - 1) / len;
+    gn_sweep_range_kernel<<<(unsigned)g, SWEEP_THREADS, 0, st>>>(partial, p.total_rays, len, range_ws);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    gn_sweep_sum_kernel<<<1, SWEEP_THREADS, 0, st>>>(range_ws, g, loss, jtr, jtj);
+    return cudaGetLastError();
+}
+
+#undef DIFFUS_GN_LEVERS
 #undef DIFFUS_GN_LAYOUTS
 
 }  // namespace diffus

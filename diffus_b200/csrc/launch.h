@@ -135,11 +135,20 @@ cudaError_t launch_gather_probe(const float* buf, int64_t n_floats, int reads, i
 // gn_kernels.cu: the Gauss-Newton system of each pose (trilinear sampler, float32 poses); partial holds 32 floats per ray,
 // med_tan 6 floats per pose (start > 0 only).  pivot (3 doubles per pose, from launch_gn_pivot) is given for per-ray origins
 // only, and selects the instantiations that rotate about it; NULL = one source per pose.
+// The lever of the twist: about each pose's source, about each pose's pivot (per-ray origins), about one pivot for the sweep.
+enum GnLever { GN_LEVER_SOURCE = 0, GN_LEVER_POSE = 1, GN_LEVER_SWEEP = 2 };
 cudaError_t launch_gn_pivot(const float* sources, int64_t n_poses, int64_t n_rays, double* pivot, cudaStream_t st);
-cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, const int32_t* tie_count, const double* pivot, float* med_tan,
-                                     cudaStream_t st);
+cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, int lever, const int32_t* tie_count, const double* pivot,
+                                     float* med_tan, cudaStream_t st);
 cudaError_t launch_render_gn(const RenderParams& p, int layout, const float* med_tan, const double* pivot, float* partial, float* loss,
                              float* jtr, float* jtj, cudaStream_t st);
+// Tracked sweeps: ONE system (double loss, jtr (6), jtj (6x6)) of a twist about the one pivot (3 doubles) shared by all poses.
+// range_ws holds gn_sweep_ranges(P*R) * 32 doubles; launch_gn_sweep_pivot writes the mean of n_rows origins (3 floats each) to
+// pivot, using the same workspace.
+int64_t gn_sweep_ranges(int64_t rows);
+cudaError_t launch_gn_sweep_pivot(const float* origins, int64_t n_rows, double* range_ws, double* pivot, cudaStream_t st);
+cudaError_t launch_render_gn_sweep(const RenderParams& p, int layout, const float* med_tan, const double* pivot, float* partial,
+                                   double* range_ws, double* loss, double* jtr, double* jtj, cudaStream_t st);
 
 // smooth_kernels.cu: scipy.ndimage.gaussian_filter(mode='nearest') of a (D,H,W) float32 volume in three separable passes,
 // radius r = int(truncate sigma + 0.5) <= BLUR_MAX_RADIUS (r = 0: a copy); dst and scratch hold D*H*W floats each

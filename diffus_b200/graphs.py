@@ -262,3 +262,123 @@ class GraphedFanGaussNewtonStep:
         """One iteration; returns the static (P,) loss after it."""
         self.graph.replay()
         return self.loss
+
+
+class GraphedSweepGaussNewtonStep:
+    """One Levenberg-Marquardt iteration of tracked-sweep registration as one CUDA-graph replay (see
+    ``pose_recovery.register_sweep``).
+
+    Static state on the device: the start poses in float64 (``start``, (3,P,3)), their origin centroid ``c0``, the current
+    transform (``rot`` (3,3), ``trans`` (3,), float64), its ``pivot = rot c0 + trans``, the current poses (``sources``,
+    ``median``, ``hint``: the transform applied to the start poses, rounded once to float32), the sweep's float64 loss (), JtJ
+    (6,6) and Jtr (6,), and the damping ``lam``.  A replay solves the damped 6x6 system (``_solve_spd6`` with a batch of one),
+    composes the candidate transform with the twist about the pivot, applies it to the start poses, renders the candidate's
+    sweep system (``ops.render_gauss_newton_sweep_impl``, about the candidate's pivot) and accepts or rejects it on the total
+    loss.  Call :meth:`reset` before the first replay.  ``probe``, ``radius`` and ``width`` as for
+    :class:`GraphedFanGaussNewtonStep`.
+    """
+
+    LAM_DOWN, LAM_UP, LAM_MIN, LAM_MAX = GraphedFanGaussNewtonStep.LAM_DOWN, GraphedFanGaussNewtonStep.LAM_UP, \
+        GraphedFanGaussNewtonStep.LAM_MIN, GraphedFanGaussNewtonStep.LAM_MAX
+
+    def __init__(self, volume, targets: torch.Tensor, n_rays: int, num_samples: int, opening_angle: float,
+                 attenuation_coeff: float = 0.5, start=0, *, probe: str = "sector", radius=None, width=None):
+        from .pose_recovery import apply_rigid_transform, compose_sweep_twist, probe_keywords
+        probe, radius, width = probe_keywords(probe, radius, width)
+        array = probe != "sector"
+        if array:
+            kid, angle, rho, wid = ops.probe_args(probe, opening_angle, radius, width)
+        if isinstance(volume, PreparedVolume):
+            bricks, vol = volume.bricks, volume.volume
+        else:
+            bricks, vol = None, volume.float().contiguous()
+        dev = vol.device
+        tgt = targets.to(torch.float32).contiguous()
+        P = tgt.shape[0]
+        start_i = _resolve_start(start, num_samples)
+        f64 = dict(dtype=torch.float64, device=dev)
+        self.P = P
+        self.start = torch.zeros((3, P, 3), **f64)                                  # [sources | median | hint] of the start
+        self.start[1, :, 1] = 1.0
+        self.start[2, :, 0] = 1.0
+        self.c0 = torch.zeros((3,), **f64)
+        self.poses = self.start.float()
+        self.sources, self.median, self.hint = self.poses[0], self.poses[1], self.poses[2]
+        self.cand = torch.zeros_like(self.poses)
+        self.rot, self.trans, self.pivot = torch.eye(3, **f64), torch.zeros((3,), **f64), torch.zeros((3,), **f64)
+        self.loss, self.jtj, self.jtr = torch.zeros((), **f64), torch.zeros((6, 6), **f64), torch.zeros((6,), **f64)
+        self.c_rot, self.c_trans, self.c_pivot = torch.zeros_like(self.rot), torch.zeros_like(self.trans), torch.zeros_like(self.pivot)
+        self.c_loss, self.c_jtj, self.c_jtr = torch.zeros_like(self.loss), torch.zeros_like(self.jtj), torch.zeros_like(self.jtr)
+        self.lam = torch.ones((1,), **f64)
+
+        def rays(poses):
+            if array:
+                return ops.probe_rays_fwd(kid, poses[0], poses[1], poses[2], n_rays, angle, rho, wid)
+            return poses[0], ops.fan_directions_fwd(poses[1], poses[2], opening_angle, n_rays)
+
+        def system(poses, pivot, loss, jtj, jtr):
+            src, dirs = rays(poses)
+            ops.render_gauss_newton_sweep_impl(vol, bricks, list(vol.shape), src, dirs, tgt, int(num_samples), start_i,
+                                               float(attenuation_coeff), pivot, loss_out=loss, jtj_out=jtj, jtr_out=jtr)
+
+        def step():
+            a = self.jtj.unsqueeze(0)
+            d = a.diagonal(dim1=-2, dim2=-1)
+            eps = 1e-12 * d.amax(-1, keepdim=True) + 1e-30
+            a = a + torch.diag_embed(self.lam[:, None] * d + eps)
+            delta, ok = _solve_spd6(a, -self.jtr.unsqueeze(0))
+            ok = ok & torch.isfinite(delta).all(-1)
+            delta = torch.where(ok[:, None], delta, torch.zeros_like(delta))[0]
+            r, t = compose_sweep_twist(self.rot, self.trans, delta, self.pivot)
+            self.c_rot.copy_(r)
+            self.c_trans.copy_(t)
+            self.c_pivot.copy_((self.c_rot * self.c0).sum(-1) + self.c_trans)
+            s, m, h = apply_rigid_transform(self.c_rot, self.c_trans, self.start[0], self.start[1], self.start[2])
+            self.cand[0].copy_(s)
+            self.cand[1].copy_(m)
+            self.cand[2].copy_(h)
+            system(self.cand, self.c_pivot, self.c_loss, self.c_jtj, self.c_jtr)
+            acc = self.c_loss < self.loss                                   # (NaN: rejected)
+            self.poses.copy_(torch.where(acc, self.cand, self.poses))
+            self.rot.copy_(torch.where(acc, self.c_rot, self.rot))
+            self.trans.copy_(torch.where(acc, self.c_trans, self.trans))
+            self.pivot.copy_(torch.where(acc, self.c_pivot, self.pivot))
+            self.loss.copy_(torch.where(acc, self.c_loss, self.loss))
+            self.jtj.copy_(torch.where(acc, self.c_jtj, self.jtj))
+            self.jtr.copy_(torch.where(acc, self.c_jtr, self.jtr))
+            self.lam.copy_(torch.where(acc, self.lam * self.LAM_DOWN, self.lam * self.LAM_UP).clamp(self.LAM_MIN, self.LAM_MAX))
+
+        def centroid(poses):
+            """The float64 mean of all P*R ray origins of ``poses`` (a sector fan's R rays share its source)."""
+            return (rays(poses)[0] if array else poses[0]).reshape(-1, 3).double().mean(0)
+
+        self._system, self._centroid = system, centroid
+        side = torch.cuda.Stream(device=dev)
+        side.wait_stream(torch.cuda.current_stream(dev))
+        with torch.cuda.stream(side):                      # warm up outside capture (lazy module loads, library handles)
+            system(self.poses, self.pivot, self.loss, self.jtj, self.jtr)
+            for _ in range(2):
+                step()
+        torch.cuda.current_stream(dev).wait_stream(side)
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            step()
+        self._keep = (vol, bricks, tgt)
+
+    def reset(self, sources: torch.Tensor, median: torch.Tensor, hint: torch.Tensor, damping: float = 1e-3) -> None:
+        """The start sweep (P,3 each), the identity transform and the initial damping; evaluates the start's system (eagerly, on
+        the device) about the start's origin centroid."""
+        for i, x in enumerate((sources, median, hint)):
+            self.start[i].copy_(x, non_blocking=True)
+            self.poses[i].copy_(x, non_blocking=True)
+        self.rot.copy_(torch.eye(3, dtype=torch.float64))
+        self.trans.zero_()
+        self.c0.copy_(self._centroid(self.poses))
+        self.pivot.copy_(self.c0)
+        self.lam.fill_(float(damping))
+        self._system(self.poses, self.pivot, self.loss, self.jtj, self.jtr)
+
+    def __call__(self) -> torch.Tensor:
+        """One iteration; returns the static float64 () total loss after it."""
+        self.graph.replay()
+        return self.loss

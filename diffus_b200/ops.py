@@ -540,6 +540,45 @@ def render_gauss_newton_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor
     return loss.view(P), jtj.view(P, 6, 6), jtr.view(P, 6)
 
 
+def render_gauss_newton_sweep_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: List[int], sources: torch.Tensor,
+                                   directions: torch.Tensor, target: torch.Tensor, n_samples: int, start: int, alpha: float,
+                                   pivot: Optional[torch.Tensor] = None, loss_out: Optional[torch.Tensor] = None,
+                                   jtj_out: Optional[torch.Tensor] = None,
+                                   jtr_out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """ONE system for all poses of a tracked sweep, with res = frame - target and J = d frame / d xi for one rigid twist
+    xi = (v, w) about ``pivot`` c shared by every pose: ``p_k = c + v + Rot(w) (s_i - c + k d_i)`` (s_i the pose's source or the
+    ray's own origin).  Returns float64 ``loss () = sum res^2``, ``JtJ (6,6)``, ``Jtr (6,)`` over all P x R x (S-start) elements.
+    ``pivot``: a (3,) float64 CUDA tensor (read on the device, so a graph replay sees its current value), or None for the mean of
+    all ray origins.  Trilinear sampler, float32 poses.
+
+    Four launches (+ two for the pivot when none is given, + two for the median when ``start > 0``).  ``*_out``: caller-provided
+    float64 output buffers (static tensors of a CUDA graph), else fresh tensors."""
+    dev = _require_cuda(volume, bricks, sources, directions, target)
+    _check_inputs(volume, bricks, dims, sources, directions)
+    if pivot is not None and (tuple(pivot.shape) != (3,) or pivot.dtype != torch.float64 or not pivot.is_contiguous()
+                              or pivot.device != dev):
+        raise _lib.DiffusError(f"pivot must be a contiguous float64 (3,) tensor on {dev}")
+    lib = _lib.load()
+    g = _lib.DiffusGaussNewtonSweepArgs()
+    with _on_device(dev):
+        P, R = _fill_render_args(g.fwd, volume, bricks, dims, sources, directions, n_samples, start, alpha, SAMPLER_TRILINEAR,
+                                 False)
+        sout = n_samples - start
+        if tuple(target.shape) != (P, R, sout) or target.dtype != torch.float32 or not target.is_contiguous():
+            raise _lib.DiffusError(f"target must be contiguous float32 {(P, R, sout)}")
+        loss = _out_buffer(loss_out, (), dev, "loss_out", torch.float64)
+        jtj = _out_buffer(jtj_out, (6, 6), dev, "jtj_out", torch.float64)
+        jtr = _out_buffer(jtr_out, (6,), dev, "jtr_out", torch.float64)
+        g.target, g.loss, g.jtr, g.jtj = target.data_ptr(), loss.data_ptr(), jtr.data_ptr(), jtj.data_ptr()
+        g.pivot = None if pivot is None else pivot.data_ptr()
+        wbytes = lib.diffus_render_gauss_newton_sweep_workspace_bytes(C.byref(g))
+        ws = torch.empty((max(wbytes, 1),), dtype=torch.uint8, device=dev)
+        g.workspace, g.workspace_bytes = ws.data_ptr(), wbytes
+        _lib.check(lib.diffus_render_gauss_newton_sweep(C.byref(g), _stream(dev)), "diffus_render_gauss_newton_sweep")
+        _count(3 + (2 if start > 0 else 0) + (2 if pivot is None else 0))
+    return loss.view(()), jtj.view(6, 6), jtr.view(6)
+
+
 @torch.library.custom_op("diffus::render_gn", mutates_args=())
 def render_gn(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: List[int], sources: torch.Tensor,
               directions: torch.Tensor, target: torch.Tensor, n_samples: int, start: int,
@@ -753,16 +792,16 @@ def fan_directions_fwd(median: torch.Tensor, hint: torch.Tensor, opening_angle: 
     return out
 
 
-def _out_buffer(out: Optional[torch.Tensor], shape, dev, what: str) -> torch.Tensor:
-    """A caller-provided contiguous float32 output of the right size (e.g. a slice of a static block inside a CUDA graph), or a
+def _out_buffer(out: Optional[torch.Tensor], shape, dev, what: str, dtype=torch.float32) -> torch.Tensor:
+    """A caller-provided contiguous output of the right size and dtype (e.g. a slice of a static block inside a CUDA graph), or a
     fresh tensor."""
     if out is None:
-        return torch.empty(shape, dtype=torch.float32, device=dev)
+        return torch.empty(shape, dtype=dtype, device=dev)
     n = 1
     for d in shape:
         n *= d
-    if out.dtype != torch.float32 or not out.is_contiguous() or out.numel() != n or out.device != dev:
-        raise _lib.DiffusError(f"{what} must be a contiguous float32 CUDA tensor of {n} elements on {dev}")
+    if out.dtype != dtype or not out.is_contiguous() or out.numel() != n or out.device != dev:
+        raise _lib.DiffusError(f"{what} must be a contiguous {str(dtype).replace('torch.', '')} CUDA tensor of {n} elements on {dev}")
     return out
 
 

@@ -7,6 +7,11 @@ turns back into the rotated fan.  Array probes (one origin per ray, :func:`diffu
 ``c``, the float64 mean of a pose's origins: ``p_k(xi) = c + v + Rot(w) (s_i - c + k d_i)``; :func:`apply_pose_twist` takes their
 (P,R,3) origins and :func:`apply_probe_twist` their parameters.  The functions are plain torch and run on any device (the test
 oracle differentiates them on the CPU).
+
+A tracked sweep knows the relative poses of its frames; what is unknown is one rigid transform ``x' = R x + t`` between the
+tracker and the volume.  :func:`register_sweep` fits it by Levenberg-Marquardt on ONE Gauss-Newton system of all frames
+(:func:`diffus_b200.render_gauss_newton_sweep`), with the twist taken about the image of the start sweep's origin centroid
+(:func:`compose_sweep_twist`, :func:`apply_rigid_transform`).
 """
 from __future__ import annotations
 
@@ -15,7 +20,7 @@ import numbers
 
 import torch
 
-from .renderer import PreparedVolume, smooth_volume
+from .renderer import PreparedVolume, _resolve_start, smooth_volume
 
 
 def _rotate(x: torch.Tensor, w: torch.Tensor) -> torch.Tensor:
@@ -66,6 +71,34 @@ def apply_probe_twist(centre: torch.Tensor, median: torch.Tensor, hint: torch.Te
     c = pivot.to(torch.float64)
     centre2 = (c + v.to(torch.float64) + _rotate(centre.to(torch.float64) - c, w.to(torch.float64))).to(centre.dtype)
     return centre2, _rotate(median, w), _rotate(hint, w)
+
+
+def rotation_matrix(w: torch.Tensor) -> torch.Tensor:
+    """``Rot(w)`` (3,3) of one rotation vector ``w`` (3,), by :func:`_rotate` on the unit vectors (elementwise only, so it records
+    into a CUDA graph)."""
+    eye = torch.eye(3, dtype=w.dtype, device=w.device)
+    return _rotate(eye, w.reshape(1, 3)).transpose(0, 1)
+
+
+def _mat_vec(m: torch.Tensor, x: torch.Tensor) -> torch.Tensor:
+    """``m @ x`` for a (3,3) matrix and (..., 3) vectors, elementwise (no library GEMM inside the graphed step)."""
+    return (m * x.unsqueeze(-2)).sum(-1)
+
+
+def compose_sweep_twist(rot: torch.Tensor, trans: torch.Tensor, delta: torch.Tensor, pivot: torch.Tensor):
+    """The transform ``x -> c + v + Rot(w) (R x + t - c)`` of the twist ``delta`` (6,) = (v, w) about ``pivot`` c (3,) after
+    ``x -> R x + t``: returns ``(Rot(w) R, c + v + Rot(w) (t - c))``, in the dtype of ``rot``."""
+    delta = delta.to(rot.dtype)
+    c = pivot.to(rot.dtype)
+    w = rotation_matrix(delta[3:])
+    return (w.unsqueeze(-1) * rot.unsqueeze(0)).sum(1), c + delta[:3] + _mat_vec(w, trans - c)
+
+
+def apply_rigid_transform(rot: torch.Tensor, trans: torch.Tensor, sources: torch.Tensor, median: torch.Tensor, hint: torch.Tensor):
+    """``(R s + t, R m, R h)`` on pose parameters (P,3) each, in the dtype of ``rot``: the points move, the two orientation
+    vectors turn."""
+    f = rot.dtype
+    return _mat_vec(rot, sources.to(f)) + trans, _mat_vec(rot, median.to(f)), _mat_vec(rot, hint.to(f))
 
 
 PROBES = ("sector", "convex", "linear")
@@ -188,3 +221,42 @@ def recover_poses_coarse_to_fine(volume, targets: torch.Tensor, sources: torch.T
             level.close()
         del level
     return poses, histories
+
+
+def register_sweep(volume, targets: torch.Tensor, sources: torch.Tensor, median: torch.Tensor, hint: torch.Tensor,
+                   opening_angle: float, n_rays: int, num_samples: int, attenuation_coeff: float = 0.5, start=0,
+                   iterations: int = 10, damping: float = 1e-3, *, probe: str = "sector", radius=None, width=None):
+    """Levenberg-Marquardt registration of a whole tracked sweep: ONE rigid transform for every frame.
+
+    The relative poses of the frames (``sources``, ``median``, ``hint``, (P,3) float32: the start sweep) are kept; the transform
+    ``x' = R x + t`` applied to all of them is fitted to the target frames ``targets`` (P, n_rays, S-start).  Each iteration solves
+    ``(JtJ + lam diag(JtJ) + eps I) delta = -Jtr`` (float64, Marquardt scaling) on the sweep's one system
+    (:func:`diffus_b200.render_gauss_newton_sweep`), with the twist about the image of the start sweep's origin centroid under
+    the current transform; composes the candidate transform in float64 (:func:`compose_sweep_twist`); applies it to the START
+    poses in float64, rounded to float32 once (:func:`apply_rigid_transform`: no rounding accumulates from step to step); renders
+    the candidate's system and keeps it only if the total loss went down (``lam`` shrinks), else stays and raises ``lam``.  One
+    iteration is one CUDA-graph replay (:class:`diffus_b200.graphs.GraphedSweepGaussNewtonStep`).
+
+    ``probe``, ``radius`` and ``width`` select the probe as in :func:`recover_poses`.  Returns ``((R (3,3), t (3,)),
+    (sources, median, hint), history)``: the float64 transform mapping the start sweep onto the registered one, the registered
+    poses, and the float64 (iterations + 1,) total loss ``sum (frame - target)^2`` before the first and after every iteration.
+    """
+    probe, radius, width = probe_keywords(probe, radius, width)
+    poses = (sources, median, hint)
+    if any(not isinstance(x, torch.Tensor) or x.dim() != 2 or x.shape[-1] != 3 or x.shape[0] != sources.shape[0] for x in poses):
+        raise ValueError("sources, median and hint must all be (P,3) tensors")
+    if any(x.dtype != torch.float32 for x in poses):
+        raise ValueError("register_sweep takes float32 poses (the transform itself is float64)")
+    want = (sources.shape[0], int(n_rays), int(num_samples) - _resolve_start(start, num_samples))
+    if tuple(targets.shape) != want:
+        raise ValueError(f"targets must be {want} (poses, rays, samples after the crop), got {tuple(targets.shape)}")
+    from .graphs import GraphedSweepGaussNewtonStep
+    step = GraphedSweepGaussNewtonStep(volume, targets, n_rays, num_samples, opening_angle, attenuation_coeff, start, probe=probe,
+                                       radius=radius, width=width)
+    step.reset(sources, median, hint, damping)
+    history = torch.empty((iterations + 1,), dtype=torch.float64, device=step.loss.device)
+    history[0].copy_(step.loss)
+    for i in range(iterations):
+        step()
+        history[i + 1].copy_(step.loss)
+    return (step.rot.clone(), step.trans.clone()), (step.sources.clone(), step.median.clone(), step.hint.clone()), history

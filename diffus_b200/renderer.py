@@ -204,6 +204,47 @@ def render_gauss_newton(volume, sources: torch.Tensor, directions: torch.Tensor,
                                         tgt, int(num_samples), _resolve_start(start, num_samples), float(attenuation_coeff))
 
 
+def render_gauss_newton_sweep(volume, sources: torch.Tensor, directions: torch.Tensor, target: torch.Tensor, num_samples: int,
+                              attenuation_coeff: float = 0.5, start=0, *, pivot=None):
+    """Gauss-Newton system of a whole tracked sweep: ONE rigid twist ``xi = (v, w)`` about ONE pivot ``c`` moves every pose,
+    ``p_k = c + v + Rot(w) (s_i - c + k d_i)`` with ``s_i`` the pose's source or, for per-ray sources (P,R,3), the ray's own
+    origin.  With ``res = frame - target`` over all P poses and ``J = d frame / d xi`` at ``xi = 0``, returns float64
+    ``loss () = sum res^2``, ``JtJ (6,6) = J^T J`` and ``Jtr (6,) = J^T res``; ``2 Jtr / n`` is the gradient of
+    :func:`render_mse_loss` (mean over n elements) w.r.t. the shared twist.  It equals ``sum_p A_p^T JtJ_p A_p`` and
+    ``sum_p A_p^T Jtr_p`` of :func:`render_gauss_newton` with ``A_p = [[I, -[c_p - c]x], [0, I]]``, ``c_p`` the point pose p
+    turns about there.
+
+    ``pivot`` is a (3,) float64 tensor on the volume's device, or None for the float64 mean of all ray origins.  Sources and
+    directions are as for :func:`render_gauss_newton` (float32, trilinear sampler).  The outputs are not differentiable: they are
+    what :func:`diffus_b200.pose_recovery.register_sweep` consumes.
+    """
+    bricks = None
+    if isinstance(volume, PreparedVolume):
+        bricks, volume = volume.bricks, volume.volume
+    src = torch.as_tensor(sources, device=volume.device)
+    dirs = torch.as_tensor(directions, device=volume.device)
+    if src.dtype != torch.float32 or dirs.dtype != torch.float32:
+        raise DiffusError("render_gauss_newton_sweep takes float32 sources and directions")
+    if src.dim() == 1:
+        src = src.unsqueeze(0)
+    if pivot is not None:
+        pivot = torch.as_tensor(pivot)
+        if tuple(pivot.shape) != (3,) or pivot.dtype != torch.float64:
+            raise DiffusError(f"pivot must be a float64 (3,) tensor, got {pivot.dtype} {tuple(pivot.shape)}")
+        pivot = pivot.to(volume.device).contiguous()
+    vol32 = (volume if volume.dtype == torch.float32 else volume.float()).detach().contiguous()
+    tgt = target.detach().to(torch.float32).contiguous()
+    if tgt.dim() == 2:
+        tgt = tgt.unsqueeze(0)
+    start_i = _resolve_start(start, num_samples)
+    want = (src.shape[0], dirs.shape[-2], int(num_samples) - start_i)
+    if tuple(tgt.shape) != want:
+        raise DiffusError(f"target must be {want} (poses, rays, samples after the crop), got {tuple(tgt.shape)}")
+    return ops.render_gauss_newton_sweep_impl(vol32, bricks, list(volume.shape), src.detach().contiguous(),
+                                              dirs.detach().contiguous(), tgt, int(num_samples), start_i,
+                                              float(attenuation_coeff), pivot)
+
+
 def smooth_volume(volume, sigma: float, truncate: float = 4.0) -> torch.Tensor:
     """Isotropic Gaussian smoothing of a (D,H,W) volume on the device: ``scipy.ndimage.gaussian_filter(volume, sigma,
     mode='nearest', truncate=truncate)`` computed in float32, radius ``int(truncate * sigma + 0.5)`` <= 64.  Beyond a face the

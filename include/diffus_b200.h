@@ -165,6 +165,27 @@ typedef struct DiffusGaussNewtonArgs {
 int64_t diffus_render_gauss_newton_workspace_bytes(const DiffusGaussNewtonArgs* args);
 int32_t diffus_render_gauss_newton(const DiffusGaussNewtonArgs* args, void* stream);
 
+/* Gauss-Newton system of a whole tracked sweep: ONE rigid twist xi = (v, w) about ONE pivot c moves every sample of every pose,
+ *   p_k = c + v + Rot(w) (s_i - c + k d_i),  s_i = the pose's source, or the ray's own origin for DIFFUS_POSE_F32_PER_RAY,
+ * and the residuals of all P x R x (S-start) elements go into one system:
+ *   loss[0] = sum res^2,   jtr (6) = J^T res,   jtj (6x6, full symmetric) = J^T J,   all float64.
+ * With A_p = [[I, -[c_p - c]x], [0, I]] it is sum_p A_p^T (system of pose p about its own source / pivot c_p) A_p.  pivot: 3
+ * doubles on the device, or NULL for the float64 mean of all P*R ray origins.  Validation, the median and NaN rules are those of
+ * diffus_render_gauss_newton; the sums over rays run in a fixed order (bit-identical from run to run). */
+typedef struct DiffusGaussNewtonSweepArgs {
+    DiffusRenderArgs fwd;       /* the render; fwd.frame, fwd.seg_prefix and fwd.workspace are unused */
+    const float* target;        /* (P,R,S-start)                                             */
+    const double* pivot;        /* 3, device; NULL = mean of all ray origins                 */
+    double* loss;               /* 1                                                         */
+    double* jtr;                /* 6                                                         */
+    double* jtj;                /* 6x6                                                       */
+    void* workspace;            /* diffus_render_gauss_newton_sweep_workspace_bytes() bytes  */
+    int64_t workspace_bytes;
+} DiffusGaussNewtonSweepArgs;
+
+int64_t diffus_render_gauss_newton_sweep_workspace_bytes(const DiffusGaussNewtonSweepArgs* args);
+int32_t diffus_render_gauss_newton_sweep(const DiffusGaussNewtonSweepArgs* args, void* stream);
+
 /* Clamped nearest-voxel indices of every ray point: the x, y, z int64 outputs of
  * custom_nearest_sampler (src/renderer.py:754-756, :816-819), cropped like
  * plot_beam_frame's return (:275).  Outputs are (P,R,S-start) int64. */
