@@ -92,6 +92,7 @@ _vp, _i32, _i64, _f32, _f64 = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_d
 SIGNATURES = {
     "diffus_abi_version": (_i32, []),
     "diffus_error_string": (C.c_char_p, [_i32]),
+    "diffus_launch_count": (_i64, []),
     "diffus_render_workspace_bytes": (_i64, [_P(DiffusRenderArgs)]),
     "diffus_render_forward": (_i32, [_P(DiffusRenderArgs), _vp]),
     "diffus_render_bwd_workspace_bytes": (_i64, [_P(DiffusRenderBwdArgs)]),

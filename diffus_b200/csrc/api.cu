@@ -251,9 +251,13 @@ GnSweepWorkspace gn_sweep_workspace(const DiffusGaussNewtonSweepArgs* g, void* b
 
 }  // namespace
 
+std::atomic<int64_t> diffus::launch_counter{0};
+
 extern "C" {
 
 int32_t diffus_abi_version(void) { return DIFFUS_ABI_VERSION; }
+
+int64_t diffus_launch_count(void) { return diffus::launch_counter.load(std::memory_order_relaxed); }
 
 const char* diffus_error_string(int32_t code) {
     switch (code) {

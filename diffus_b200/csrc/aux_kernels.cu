@@ -82,8 +82,7 @@ cudaError_t launch_first_refl_median(const RenderParams& p, int sampler, int lay
     size_t smem = (size_t)p.n_rays * sizeof(float);
     DIFFUS_DISPATCH(auto k = first_refl_median_kernel<S_, L_, P64_>;
                     if (smem > 40 * 1024) { cudaError_t e = ensure_smem(k, smem); if (e != cudaSuccess) return e; }
-                    k<<<(unsigned)p.n_poses, threads, smem, st>>>(p, median, tie_count);
-                    return cudaGetLastError())
+                    return launch_kernel(k, (unsigned)p.n_poses, threads, smem, st, p, median, tie_count))
     return cudaErrorInvalidValue;
 }
 
@@ -151,9 +150,9 @@ cudaError_t launch_median_backward(const RenderParams& p, int sampler, int layou
                                    const int32_t* tie_count, bool pose_grad, bool vol_grad, cudaStream_t st) {
     if (sampler == DIFFUS_SAMPLER_NEAREST) pose_grad = false;
     if (!pose_grad && !vol_grad) return cudaSuccess;      // loss / frame only: no gradient flows through the median
-#define DIFFUS_MB(PG, VG) median_backward_kernel<S_, L_, P64_, PG, VG><<<(unsigned)p.n_poses, 32, 0, st>>>(p, tie_count)
-    DIFFUS_DISPATCH(if (pose_grad && vol_grad) DIFFUS_MB(true, true); else if (pose_grad) DIFFUS_MB(true, false);
-                    else if (vol_grad) DIFFUS_MB(false, true); return cudaGetLastError())
+#define DIFFUS_MB(PG, VG) launch_kernel(median_backward_kernel<S_, L_, P64_, PG, VG>, (unsigned)p.n_poses, 32, 0, st, p, tie_count)
+    DIFFUS_DISPATCH(if (pose_grad && vol_grad) return DIFFUS_MB(true, true); if (pose_grad) return DIFFUS_MB(true, false);
+                    return DIFFUS_MB(false, true))
 #undef DIFFUS_MB
     return cudaErrorInvalidValue;
 }
@@ -180,9 +179,8 @@ __global__ void ray_indices_kernel(const RenderParams p, int64_t* __restrict__ x
 cudaError_t launch_ray_indices(const RenderParams& p, int pose64, int64_t* x, int64_t* y, int64_t* z, cudaStream_t st) {
     int64_t n = p.total_rays * p.Sout;
     unsigned grid = (unsigned)min((int64_t)148 * 16, (n + 255) / 256);
-    if (pose64) ray_indices_kernel<true><<<grid, 256, 0, st>>>(p, x, y, z);
-    else ray_indices_kernel<false><<<grid, 256, 0, st>>>(p, x, y, z);
-    return cudaGetLastError();
+    if (pose64) return launch_kernel(ray_indices_kernel<true>, grid, 256, 0, st, p, x, y, z);
+    return launch_kernel(ray_indices_kernel<false>, grid, 256, 0, st, p, x, y, z);
 }
 
 template <int SAMPLER, int LAYOUT, bool POSE64>
@@ -202,7 +200,7 @@ __global__ void trace_values_kernel(const RenderParams p, float* __restrict__ ou
 cudaError_t launch_trace_values(const RenderParams& p, int sampler, int layout, int pose64, float* out, cudaStream_t st) {
     int64_t n = p.total_rays * p.S;
     unsigned grid = (unsigned)min((int64_t)148 * 16, (n + 255) / 256);
-    DIFFUS_DISPATCH(trace_values_kernel<S_, L_, P64_><<<grid, 256, 0, st>>>(p, out); return cudaGetLastError())
+    DIFFUS_DISPATCH(return launch_kernel(trace_values_kernel<S_, L_, P64_>, grid, 256, 0, st, p, out))
     return cudaErrorInvalidValue;
 }
 
@@ -227,8 +225,7 @@ cudaError_t launch_sample_points(const RenderParams& p, int sampler, int layout,
                                  int64_t* x, int64_t* y, int64_t* z, cudaStream_t st) {
     unsigned grid = (unsigned)max((int64_t)1, min((int64_t)148 * 16, (n + 255) / 256));
     const int pose64 = 0;
-    DIFFUS_DISPATCH(sample_points_kernel<S_, L_><<<grid, 256, 0, st>>>(p.vol, pts, n, val, x, y, z); (void)P64_;
-                    return cudaGetLastError())
+    DIFFUS_DISPATCH((void)P64_; return launch_kernel(sample_points_kernel<S_, L_>, grid, 256, 0, st, p.vol, pts, n, val, x, y, z))
     return cudaErrorInvalidValue;
 }
 
@@ -288,9 +285,9 @@ cudaError_t launch_trace_values_bwd(const RenderParams& p, int sampler, int layo
     if (sampler == DIFFUS_SAMPLER_NEAREST) pose_grad = false;
     if (!pose_grad && !vol_grad) return cudaSuccess;      // nothing requested: nothing to write
     unsigned grid = (unsigned)((p.total_rays + 3) / 4);
-#define DIFFUS_TB(PG, VG) trace_values_bwd_kernel<S_, L_, P64_, PG, VG><<<grid, 128, 0, st>>>(p, gval)
-    DIFFUS_DISPATCH(if (pose_grad && vol_grad) DIFFUS_TB(true, true); else if (pose_grad) DIFFUS_TB(true, false);
-                    else if (vol_grad) DIFFUS_TB(false, true); return cudaGetLastError())
+#define DIFFUS_TB(PG, VG) launch_kernel(trace_values_bwd_kernel<S_, L_, P64_, PG, VG>, grid, 128, 0, st, p, gval)
+    DIFFUS_DISPATCH(if (pose_grad && vol_grad) return DIFFUS_TB(true, true); if (pose_grad) return DIFFUS_TB(true, false);
+                    return DIFFUS_TB(false, true))
 #undef DIFFUS_TB
     return cudaErrorInvalidValue;
 }
@@ -311,8 +308,7 @@ __global__ void reduce_rays_kernel(const float* __restrict__ partial, int64_t n_
 
 cudaError_t launch_reduce_rays(const float* partial, int64_t n_poses, int64_t n_rays, float* out, cudaStream_t st) {
     unsigned grid = (unsigned)((n_poses + 3) / 4);
-    reduce_rays_kernel<<<grid, 128, 0, st>>>(partial, n_poses, n_rays, out);
-    return cudaGetLastError();
+    return launch_kernel(reduce_rays_kernel, grid, 128, 0, st, partial, n_poses, n_rays, out);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -343,8 +339,7 @@ cudaError_t launch_cone_directions(const double* median, int64_t n_poses, int64_
                                    float* out, cudaStream_t st) {
     int64_t n = n_poses * n_rays;
     unsigned grid = (unsigned)min((int64_t)148 * 8, (n + 127) / 128);
-    cone_directions_kernel<<<grid, 128, 0, st>>>(median, n_poses, n_rays, opening_angle, out);
-    return cudaGetLastError();
+    return launch_kernel(cone_directions_kernel, grid, 128, 0, st, median, n_poses, n_rays, opening_angle, out);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -379,8 +374,7 @@ cudaError_t launch_to_bricks(const float* linear, const int32_t dim[3], float* b
     brick_counts(dim, nbi, nbj, nbk);
     int64_t n = (int64_t)nbi * nbj * nbk * 32;
     unsigned grid = (unsigned)min((int64_t)148 * 32, (n + 255) / 256);
-    brick_copy_kernel<true><<<grid, 256, 0, st>>>(linear, bricks, dim[0], dim[1], dim[2], nbi, nbj, nbk);
-    return cudaGetLastError();
+    return launch_kernel(brick_copy_kernel<true>, grid, 256, 0, st, linear, bricks, dim[0], dim[1], dim[2], nbi, nbj, nbk);
 }
 
 cudaError_t launch_from_bricks(const float* bricks, const int32_t dim[3], float* linear, cudaStream_t st) {
@@ -388,8 +382,7 @@ cudaError_t launch_from_bricks(const float* bricks, const int32_t dim[3], float*
     brick_counts(dim, nbi, nbj, nbk);
     int64_t n = (int64_t)nbi * nbj * nbk * 32;
     unsigned grid = (unsigned)min((int64_t)148 * 32, (n + 255) / 256);
-    brick_copy_kernel<false><<<grid, 256, 0, st>>>(bricks, linear, dim[0], dim[1], dim[2], nbi, nbj, nbk);
-    return cudaGetLastError();
+    return launch_kernel(brick_copy_kernel<false>, grid, 256, 0, st, bricks, linear, dim[0], dim[1], dim[2], nbi, nbj, nbk);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -420,8 +413,7 @@ cudaError_t launch_to_quads(const float* linear, const int32_t dim[3], float* qu
     int nqi = (dim[0] + QUAD_B - 1) / QUAD_B, nqj = (dim[1] + QUAD_B - 1) / QUAD_B, nqk = (dim[2] + QUAD_B - 1) / QUAD_B;
     int64_t n = (int64_t)nqi * nqj * nqk * 8;
     unsigned grid = (unsigned)min((int64_t)148 * 32, (n + 255) / 256);
-    quad_copy_kernel<<<grid, 256, 0, st>>>(linear, (float4*)quads, dim[0], dim[1], dim[2], nqi, nqj, nqk);
-    return cudaGetLastError();
+    return launch_kernel(quad_copy_kernel, grid, 256, 0, st, linear, (float4*)quads, dim[0], dim[1], dim[2], nqi, nqj, nqk);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -445,8 +437,7 @@ __global__ void __launch_bounds__(256) gather_probe_kernel(const float* __restri
 
 cudaError_t launch_gather_probe(const float* buf, int64_t n_floats, int reads, int64_t n_threads, uint32_t seed, float* sink,
                                 cudaStream_t st) {
-    gather_probe_kernel<<<(unsigned)(n_threads / 256), 256, 0, st>>>(buf, (uint32_t)(n_floats / 8), reads, seed, sink);
-    return cudaGetLastError();
+    return launch_kernel(gather_probe_kernel, (unsigned)(n_threads / 256), 256, 0, st, buf, (uint32_t)(n_floats / 8), reads, seed, sink);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -539,15 +530,13 @@ __global__ void fan_directions_bwd_kernel(const float* __restrict__ median, cons
 
 cudaError_t launch_fan_directions(const float* median, const float* hint, int64_t n_poses, int64_t n_rays, double angle,
                                   float* out, cudaStream_t st) {
-    fan_directions_kernel<<<(unsigned)n_poses, 128, 0, st>>>(median, hint, n_poses, n_rays, angle, out);
-    return cudaGetLastError();
+    return launch_kernel(fan_directions_kernel, (unsigned)n_poses, 128, 0, st, median, hint, n_poses, n_rays, angle, out);
 }
 
 cudaError_t launch_fan_directions_bwd(const float* median, const float* hint, const float* grad_dirs, int64_t n_poses,
                                       int64_t n_rays, double angle, float* grad_median, float* grad_hint, cudaStream_t st) {
-    fan_directions_bwd_kernel<<<(unsigned)n_poses, 32, 0, st>>>(median, hint, grad_dirs, n_poses, n_rays, angle, grad_median,
+    return launch_kernel(fan_directions_bwd_kernel, (unsigned)n_poses, 32, 0, st, median, hint, grad_dirs, n_poses, n_rays, angle, grad_median,
                                                                 grad_hint);
-    return cudaGetLastError();
 }
 
 
@@ -633,17 +622,15 @@ __global__ void probe_rays_bwd_kernel(int kind, const float* __restrict__ median
 
 cudaError_t launch_probe_rays(int kind, const float* centre, const float* median, const float* hint, int64_t n_poses, int64_t n_rays,
                               double angle, double radius, double width, float* origins, float* dirs, cudaStream_t st) {
-    probe_rays_kernel<<<(unsigned)n_poses, 128, 0, st>>>(kind, centre, median, hint, n_rays, angle, radius, width, origins, dirs);
-    return cudaGetLastError();
+    return launch_kernel(probe_rays_kernel, (unsigned)n_poses, 128, 0, st, kind, centre, median, hint, n_rays, angle, radius, width, origins, dirs);
 }
 
 cudaError_t launch_probe_rays_bwd(int kind, const float* centre, const float* median, const float* hint, const float* grad_origins,
                                   const float* grad_dirs, int64_t n_poses, int64_t n_rays, double angle, double radius, double width,
                                   float* grad_centre, float* grad_median, float* grad_hint, cudaStream_t st) {
     (void)centre;                                          // the centre enters the origins linearly
-    probe_rays_bwd_kernel<<<(unsigned)n_poses, 32, 0, st>>>(kind, median, hint, grad_origins, grad_dirs, n_rays, angle, radius, width,
+    return launch_kernel(probe_rays_bwd_kernel, (unsigned)n_poses, 32, 0, st, kind, median, hint, grad_origins, grad_dirs, n_rays, angle, radius, width,
                                                             grad_centre, grad_median, grad_hint);
-    return cudaGetLastError();
 }
 
 }  // namespace diffus

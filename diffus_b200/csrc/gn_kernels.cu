@@ -461,16 +461,14 @@ __global__ void __launch_bounds__(SWEEP_THREADS) gn_sweep_pivot_kernel(const T* 
 
 cudaError_t launch_gn_sweep_pivot(const float* origins, int64_t n_rows, double* range_ws, double* pivot, cudaStream_t st) {
     const int64_t len = gn_sweep_range_rows(n_rows), g = (n_rows + len - 1) / len;
-    gn_sweep_pivot_kernel<float, false><<<(unsigned)g, SWEEP_THREADS, 0, st>>>(origins, n_rows, len, n_rows, range_ws);
-    cudaError_t e = cudaGetLastError();
+    cudaError_t e = launch_kernel(gn_sweep_pivot_kernel<float, false>, (unsigned)g, SWEEP_THREADS, 0, st, origins, n_rows, len, n_rows,
+                                  range_ws);
     if (e != cudaSuccess) return e;
-    gn_sweep_pivot_kernel<double, true><<<1, SWEEP_THREADS, 0, st>>>(range_ws, g, g, n_rows, pivot);
-    return cudaGetLastError();
+    return launch_kernel(gn_sweep_pivot_kernel<double, true>, 1, SWEEP_THREADS, 0, st, range_ws, g, g, n_rows, pivot);
 }
 
 cudaError_t launch_gn_pivot(const float* sources, int64_t n_poses, int64_t n_rays, double* pivot, cudaStream_t st) {
-    gn_pivot_kernel<<<(unsigned)((n_poses + 3) / 4), 128, 0, st>>>(sources, n_poses, n_rays, pivot);
-    return cudaGetLastError();
+    return launch_kernel(gn_pivot_kernel, (unsigned)((n_poses + 3) / 4), 128, 0, st, sources, n_poses, n_rays, pivot);
 }
 
 static int gn_warps_per_block(int64_t total_rays) {
@@ -496,8 +494,7 @@ static int gn_warps_per_block(int64_t total_rays) {
 
 cudaError_t launch_gn_median_tangent(const RenderParams& p, int layout, int lever, const int32_t* tie_count, const double* pivot,
                                      float* med_tan, cudaStream_t st) {
-    DIFFUS_GN_LEVERS(gn_median_tangent_kernel<L_, V_><<<(unsigned)p.n_poses, 32, 0, st>>>(p, tie_count, pivot, med_tan);
-                     return cudaGetLastError())
+    DIFFUS_GN_LEVERS(return launch_kernel(gn_median_tangent_kernel<L_, V_>, (unsigned)p.n_poses, 32, 0, st, p, tie_count, pivot, med_tan))
     return cudaErrorInvalidValue;
 }
 
@@ -508,7 +505,7 @@ static cudaError_t launch_gn_march(const RenderParams& p, int layout, int lever,
     const size_t smem = (size_t)wpb * GN_SMEM_PER_WARP * sizeof(float);
     const unsigned grid = (unsigned)((p.total_rays + wpb - 1) / wpb);
     DIFFUS_GN_LEVERS(auto k = render_gn_kernel<L_, V_>; cudaError_t e = ensure_smem(k, smem); if (e != cudaSuccess) return e;
-                     k<<<grid, wpb * 32, smem, st>>>(p, med_tan, pivot, partial); return cudaGetLastError())
+                     return launch_kernel(k, grid, wpb * 32, smem, st, p, med_tan, pivot, partial))
     return cudaErrorInvalidValue;
 }
 
@@ -516,8 +513,7 @@ cudaError_t launch_render_gn(const RenderParams& p, int layout, const float* med
                              float* jtr, float* jtj, cudaStream_t st) {
     cudaError_t e = launch_gn_march(p, layout, pivot ? GN_LEVER_POSE : GN_LEVER_SOURCE, med_tan, pivot, partial, st);
     if (e != cudaSuccess) return e;
-    gn_reduce_kernel<<<(unsigned)p.n_poses, 128, 0, st>>>(partial, p.n_rays, loss, jtr, jtj);
-    return cudaGetLastError();
+    return launch_kernel(gn_reduce_kernel, (unsigned)p.n_poses, 128, 0, st, partial, p.n_rays, loss, jtr, jtj);
 }
 
 cudaError_t launch_render_gn_sweep(const RenderParams& p, int layout, const float* med_tan, const double* pivot, float* partial,
@@ -525,11 +521,9 @@ cudaError_t launch_render_gn_sweep(const RenderParams& p, int layout, const floa
     cudaError_t e = launch_gn_march(p, layout, GN_LEVER_SWEEP, med_tan, pivot, partial, st);
     if (e != cudaSuccess) return e;
     const int64_t len = gn_sweep_range_rows(p.total_rays), g = (p.total_rays + len - 1) / len;
-    gn_sweep_range_kernel<<<(unsigned)g, SWEEP_THREADS, 0, st>>>(partial, p.total_rays, len, range_ws);
-    e = cudaGetLastError();
+    e = launch_kernel(gn_sweep_range_kernel, (unsigned)g, SWEEP_THREADS, 0, st, partial, p.total_rays, len, range_ws);
     if (e != cudaSuccess) return e;
-    gn_sweep_sum_kernel<<<1, SWEEP_THREADS, 0, st>>>(range_ws, g, loss, jtr, jtj);
-    return cudaGetLastError();
+    return launch_kernel(gn_sweep_sum_kernel, 1, SWEEP_THREADS, 0, st, range_ws, g, loss, jtr, jtj);
 }
 
 #undef DIFFUS_GN_LEVERS

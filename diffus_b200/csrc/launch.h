@@ -3,9 +3,21 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <atomic>
+
 #include "common.cuh"
 
 namespace diffus {
+
+// Every kernel the library enqueues goes through launch_kernel, so that diffus_launch_count() (api.cu) states how many
+// kernels the library launched: memsets and copies are not counted.
+extern std::atomic<int64_t> launch_counter;
+template <typename K, typename... Args>
+static inline cudaError_t launch_kernel(K kernel, dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
+    kernel<<<grid, block, smem, st>>>(args...);
+    launch_counter.fetch_add(1, std::memory_order_relaxed);
+    return cudaGetLastError();
+}
 
 // 8-way template dispatch on (sampler, layout, pose dtype); the body sees S_, L_, P64_.
 #define DIFFUS_DISPATCH_CASE(Sv, Lv, Pv, ...)                              \

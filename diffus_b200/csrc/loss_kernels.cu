@@ -86,15 +86,13 @@ __global__ void masked_mse_edge_bwd_kernel(const float* __restrict__ a, const fl
 
 cudaError_t launch_masked_mse_edge_fwd(const float* a, const float* b, const uint8_t* mask, int H, int W, float edge_weight,
                                        float* stats, cudaStream_t st) {
-    masked_mse_edge_fwd_kernel<<<1, 1024, 0, st>>>(a, b, mask, H, W, edge_weight, stats);
-    return cudaGetLastError();
+    return launch_kernel(masked_mse_edge_fwd_kernel, 1, 1024, 0, st, a, b, mask, H, W, edge_weight, stats);
 }
 cudaError_t launch_masked_mse_edge_bwd(const float* a, const float* b, const uint8_t* mask, int H, int W, float edge_weight,
                                        const float* stats, const float* grad_loss, float* ga, cudaStream_t st) {
     const int64_t n = (int64_t)H * W;
-    masked_mse_edge_bwd_kernel<<<(unsigned)max((int64_t)1, min((int64_t)148 * 4, (n + 255) / 256)), 256, 0, st>>>(
+    return launch_kernel(masked_mse_edge_bwd_kernel, (unsigned)max((int64_t)1, min((int64_t)148 * 4, (n + 255) / 256)), 256, 0, st, 
         a, b, mask, H, W, edge_weight, stats, grad_loss, ga);
-    return cudaGetLastError();
 }
 
 // ---------------------------------------------------------------------------------------
@@ -326,12 +324,13 @@ __global__ void ssim_bwd_final_kernel(const float* __restrict__ s, int64_t n, in
 cudaError_t launch_ssim_fwd(const float* s, const float* y, int H, int W, int K, float sigma, float k1, float k2, int normalize,
                             float* loss, void* workspace, cudaStream_t st) {
     SsimLayout L = ssim_layout(workspace, H, W, K);
-    ssim_minmax_kernel<<<1, 1024, 0, st>>>(s, (int64_t)H * W, normalize, L.header);
+    cudaError_t e = launch_kernel(ssim_minmax_kernel, 1, 1024, 0, st, s, (int64_t)H * W, normalize, L.header);
+    if (e != cudaSuccess) return e;
     const int IN = SSIM_TILE + K - 1;
     const size_t smem = (size_t)(2 * IN * IN + 5 * IN * SSIM_TILE + SSIM_MAXK + 3) * sizeof(float);
-    ssim_fwd_kernel<<<L.tiles_fwd, SSIM_TILE * SSIM_TILE, smem, st>>>(s, y, H, W, K, sigma, k1 * k1, k2 * k2, L);
-    ssim_loss_final_kernel<<<1, 32, 0, st>>>(L, loss);
-    return cudaGetLastError();
+    e = launch_kernel(ssim_fwd_kernel, L.tiles_fwd, SSIM_TILE * SSIM_TILE, smem, st, s, y, H, W, K, sigma, k1 * k1, k2 * k2, L);
+    if (e != cudaSuccess) return e;
+    return launch_kernel(ssim_loss_final_kernel, 1, 32, 0, st, L, loss);
 }
 
 cudaError_t launch_ssim_bwd(const float* s, const float* y, int H, int W, int K, float sigma, int normalize, const float* grad_loss,
@@ -339,10 +338,10 @@ cudaError_t launch_ssim_bwd(const float* s, const float* y, int H, int W, int K,
     SsimLayout L = ssim_layout(workspace, H, W, K);
     const int IN = SSIM_TILE + K - 1;
     const size_t smem = (size_t)(3 * IN * IN + 3 * IN * SSIM_TILE + SSIM_MAXK + 3) * sizeof(float);
-    ssim_bwd_kernel<<<L.tiles_bwd, SSIM_TILE * SSIM_TILE, smem, st>>>(s, y, H, W, K, sigma, L);
+    cudaError_t e = launch_kernel(ssim_bwd_kernel, L.tiles_bwd, SSIM_TILE * SSIM_TILE, smem, st, s, y, H, W, K, sigma, L);
+    if (e != cudaSuccess) return e;
     const int64_t n = (int64_t)H * W;
-    ssim_bwd_final_kernel<<<(unsigned)max((int64_t)1, min((int64_t)148 * 4, (n + 255) / 256)), 256, 0, st>>>(s, n, normalize, L, grad_loss, grad_s);
-    return cudaGetLastError();
+    return launch_kernel(ssim_bwd_final_kernel, (unsigned)max((int64_t)1, min((int64_t)148 * 4, (n + 255) / 256)), 256, 0, st, s, n, normalize, L, grad_loss, grad_s);
 }
 
 }  // namespace diffus

@@ -79,8 +79,7 @@ cudaError_t launch_mlp_fwd(const float* params, const float* x, const uint8_t* m
                            float fill, float* out, cudaStream_t st) {
     int64_t want = (n + 256 * FWD_VPT - 1) / (256 * FWD_VPT);
     unsigned grid = (unsigned)max((int64_t)1, min(want, (int64_t)148 * 8));
-    mlp_fwd_kernel<<<grid, 256, 0, st>>>(params, x, mask, n, out_scale, fill, out);
-    return cudaGetLastError();
+    return launch_kernel(mlp_fwd_kernel, grid, 256, 0, st, params, x, mask, n, out_scale, fill, out);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -245,11 +244,10 @@ int64_t mlp_bwd_workspace_bytes(int64_t n) {
 cudaError_t launch_mlp_bwd(const float* params, const float* x, const uint8_t* mask, const float* grad_out, int64_t n,
                            float out_scale, float* grad_params, void* workspace, const int* gate, cudaStream_t st) {
     const int blocks = mlp_bwd_blocks(n);
-    mlp_bwd_kernel<<<blocks, BWD_WARPS * 32, 0, st>>>(params, x, mask, grad_out, n, out_scale, (float*)workspace, gate);
-    cudaError_t e = cudaGetLastError();
+    cudaError_t e = launch_kernel(mlp_bwd_kernel, blocks, BWD_WARPS * 32, 0, st, params, x, mask, grad_out, n, out_scale,
+                                  (float*)workspace, gate);
     if (e != cudaSuccess) return e;
-    mlp_bwd_reduce_kernel<<<(DIFFUS_MLP_NPARAMS + 127) / 128, 128, 0, st>>>((const float*)workspace, blocks, grad_params, gate);
-    return cudaGetLastError();
+    return launch_kernel(mlp_bwd_reduce_kernel, (DIFFUS_MLP_NPARAMS + 127) / 128, 128, 0, st, (const float*)workspace, blocks, grad_params, gate);
 }
 
 }  // namespace diffus

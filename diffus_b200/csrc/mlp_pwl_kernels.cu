@@ -526,8 +526,7 @@ cudaError_t launch_mlp_pwl_fwd(const float* params, const float* x, const uint8_
     const size_t smem = pwl_fwd_smem();
     cudaError_t e = cudaFuncSetAttribute(mlp_pwl_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    mlp_pwl_fwd_kernel<<<pwl_blocks(n), PWL_THREADS, smem, st>>>(params, x, mask, n, out_scale, fill, out);
-    return cudaGetLastError();
+    return launch_kernel(mlp_pwl_fwd_kernel, pwl_blocks(n), PWL_THREADS, smem, st, params, x, mask, n, out_scale, fill, out);
 }
 
 cudaError_t launch_mlp_pwl_dx(const float* params, const float* x, const uint8_t* mask, const float* grad_out, int64_t n,
@@ -536,9 +535,8 @@ cudaError_t launch_mlp_pwl_dx(const float* params, const float* x, const uint8_t
     cudaError_t e = cudaFuncSetAttribute(mlp_pwl_dx_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     const int64_t want = (n + PWL_THREADS - 1) / PWL_THREADS;
-    mlp_pwl_dx_kernel<<<(unsigned)max((int64_t)1, min(want, (int64_t)148 * 4)), PWL_THREADS, smem, st>>>(params, x, mask, grad_out, n,
+    return launch_kernel(mlp_pwl_dx_kernel, (unsigned)max((int64_t)1, min(want, (int64_t)148 * 4)), PWL_THREADS, smem, st, params, x, mask, grad_out, n,
                                                                                                       out_scale, grad_x);
-    return cudaGetLastError();
 }
 
 // `workspace` holds mlp_pwl_bwd_workspace_bytes(n) bytes followed by the dense fallback's block partials
@@ -552,10 +550,11 @@ cudaError_t launch_mlp_pwl_bwd(const float* params, const float* x, const uint8_
     double* ws_xm = (double*)((char*)workspace + PWL_HDR_BYTES);
     double* partial = ws_xm + PWL_MAXR;
     double* scratch = partial + (int64_t)blocks * PWL_MAXR * 2;
-    mlp_pwl_bwd_kernel<<<blocks, PWL_THREADS, smem, st>>>(params, x, mask, grad_out, n, out_scale, hdr, ws_xm, partial);
-    mlp_pwl_assemble_kernel<<<PWL_MAXR, 128, 0, st>>>(params, hdr, ws_xm, partial, blocks, scratch);
-    mlp_pwl_finish_kernel<<<(NP + 127) / 128, 128, 0, st>>>(hdr, scratch, grad_params);
-    e = cudaGetLastError();
+    e = launch_kernel(mlp_pwl_bwd_kernel, blocks, PWL_THREADS, smem, st, params, x, mask, grad_out, n, out_scale, hdr, ws_xm, partial);
+    if (e != cudaSuccess) return e;
+    e = launch_kernel(mlp_pwl_assemble_kernel, PWL_MAXR, 128, 0, st, params, hdr, ws_xm, partial, blocks, scratch);
+    if (e != cudaSuccess) return e;
+    e = launch_kernel(mlp_pwl_finish_kernel, (NP + 127) / 128, 128, 0, st, hdr, scratch, grad_params);
     if (e != cudaSuccess) return e;
     // more than PWL_MAXR regions: the layered CUDA-core kernels run instead (they return at once when hdr[1] == 0)
     void* dense_ws = (char*)workspace + mlp_pwl_bwd_workspace_bytes(n);

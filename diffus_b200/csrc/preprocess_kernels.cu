@@ -69,22 +69,22 @@ cudaError_t launch_brain_mask(const float* volume, const int32_t dim[3], float t
     const int64_t n = (int64_t)dim[0] * dim[1] * dim[2];
     uint8_t* a = mask;
     uint8_t* b = scratch;
-    threshold_kernel<<<grid_for(n), 256, 0, st>>>(volume, n, threshold, a);
-    for (int it = 0; it < 2 * iterations; ++it) {
-        if (it < iterations) morph_kernel<true><<<grid_for(n), 256, 0, st>>>(a, b, dim[0], dim[1], dim[2]);
-        else morph_kernel<false><<<grid_for(n), 256, 0, st>>>(a, b, dim[0], dim[1], dim[2]);
+    cudaError_t e = launch_kernel(threshold_kernel, grid_for(n), 256, 0, st, volume, n, threshold, a);
+    for (int it = 0; it < 2 * iterations && e == cudaSuccess; ++it) {
+        if (it < iterations) e = launch_kernel(morph_kernel<true>, grid_for(n), 256, 0, st, a, b, dim[0], dim[1], dim[2]);
+        else e = launch_kernel(morph_kernel<false>, grid_for(n), 256, 0, st, a, b, dim[0], dim[1], dim[2]);
         uint8_t* t = a; a = b; b = t;
     }
     // an even number of passes ends in `mask`
-    return cudaGetLastError();
+    return e;
 }
 
 cudaError_t launch_masked_zscore(const float* volume, const uint8_t* mask, int64_t n, float* out, void* ws, cudaStream_t st) {
     cudaError_t e = cudaMemsetAsync(ws, 0, sizeof(ZStats), st);
     if (e != cudaSuccess) return e;
-    masked_stats_kernel<<<grid_for(n), 256, 0, st>>>(volume, mask, n, (ZStats*)ws);
-    zscore_kernel<<<grid_for(n), 256, 0, st>>>(volume, n, (const ZStats*)ws, out);
-    return cudaGetLastError();
+    e = launch_kernel(masked_stats_kernel, grid_for(n), 256, 0, st, volume, mask, n, (ZStats*)ws);
+    if (e != cudaSuccess) return e;
+    return launch_kernel(zscore_kernel, grid_for(n), 256, 0, st, volume, n, (const ZStats*)ws, out);
 }
 
 }  // namespace diffus

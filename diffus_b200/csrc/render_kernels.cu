@@ -1082,8 +1082,7 @@ bool reduce_rays_and_sum_fits(int64_t n) { return n <= ((int64_t)1 << 18); }    
 cudaError_t launch_reduce_rays_and_sum(const float* src_partial, int64_t n_poses, int64_t n_rays, float* grad_src,
                                        const float* loss_partial, int64_t n, float scale, float* loss_out, cudaStream_t st) {
     const unsigned grid = (unsigned)((n_poses + 31) / 32) + 1u;
-    reduce_rays_and_sum_kernel<<<grid, 1024, 0, st>>>(src_partial, n_poses, n_rays, grad_src, loss_partial, n, scale, loss_out);
-    return cudaGetLastError();
+    return launch_kernel(reduce_rays_and_sum_kernel, grid, 1024, 0, st, src_partial, n_poses, n_rays, grad_src, loss_partial, n, scale, loss_out);
 }
 
 constexpr int REDUCE_BLOCKS = 64;
@@ -1091,13 +1090,12 @@ int64_t reduce_sum_workspace_bytes() { return REDUCE_BLOCKS * sizeof(double); }
 
 cudaError_t launch_reduce_sum(const float* partial, int64_t n, float scale, float* out, void* workspace, cudaStream_t st) {
     if (n <= ((int64_t)1 << 18)) {        // (one SM sums 1 MB in ~10 us; the 2 MB of a 4096-pose batch took 79 us under ncu)
-        reduce_sum_kernel<<<1, 1024, 0, st>>>(partial, n, scale, out, nullptr);
-        return cudaGetLastError();
+        return launch_kernel(reduce_sum_kernel, 1, 1024, 0, st, partial, n, scale, out, nullptr);
     }
     double* sums = (double*)workspace;
-    reduce_sum_kernel<<<REDUCE_BLOCKS, 1024, 0, st>>>(partial, n, scale, out, sums);
-    reduce_final_kernel<<<1, 32, 0, st>>>(sums, REDUCE_BLOCKS, scale, out);
-    return cudaGetLastError();
+    cudaError_t e = launch_kernel(reduce_sum_kernel, REDUCE_BLOCKS, 1024, 0, st, partial, n, scale, out, sums);
+    if (e != cudaSuccess) return e;
+    return launch_kernel(reduce_final_kernel, 1, 32, 0, st, sums, REDUCE_BLOCKS, scale, out);
 }
 
 #endif  // !DIFFUS_LAYOUT_SLICE
@@ -1125,7 +1123,7 @@ cudaError_t DIFFUS_FWD_NAME(const RenderParams& p_in, int sampler, int layout, i
     size_t smem = ((size_t)p.att_slots + (size_t)wpb * FWD_SMEM_PER_WARP) * sizeof(float);
     unsigned grid = (unsigned)((p.total_rays + wpb - 1) / wpb);
     DIFFUS_DISPATCH(auto k = render_fwd_kernel<S_, L_, P64_>; cudaError_t e = ensure_smem(k, smem, 28 / wpb);
-                    if (e != cudaSuccess) return e; k<<<grid, wpb * 32, smem, st>>>(p); return cudaGetLastError())
+                    if (e != cudaSuccess) return e; return launch_kernel(k, grid, wpb * 32, smem, st, p))
     return cudaErrorInvalidValue;
 }
 
@@ -1143,15 +1141,13 @@ static cudaError_t launch_bwd_g(const RenderParams& p, bool pg, bool vg, unsigne
             auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, true, WIDE_>;                                     \
             cudaError_t e = ensure_smem(k, smem, WIDE_CTAS * 4 / (threads / 32));                                     \
             if (e != cudaSuccess) return e;                                                                           \
-            k<<<grid, threads, smem, st>>>(p);                                                                        \
-            return cudaGetLastError();                                                                                \
+            return launch_kernel(k, grid, threads, smem, st, p);                                                      \
         }                                                                                                             \
         if (!P64_ && p.Sout <= PREFIX_STRIDE) {                                                                       \
             auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, true>;                                            \
             cudaError_t e = ensure_smem(k, smem, ((VG) ? 16 : 20) / (threads / 32));                                  \
             if (e != cudaSuccess) return e;                                                                           \
-            k<<<grid, threads, smem, st>>>(p);                                                                        \
-            return cudaGetLastError();                                                                                \
+            return launch_kernel(k, grid, threads, smem, st, p);                                                      \
         }                                                                                                             \
         if (render_bwd_is_coop(p.Sout, p.total_rays, S_, P64_, PG, VG)) { /* rays of 2..4 passes (config 5: 4): one ray per CTA, no pre-pass */ \
             auto k = render_bwd_kernel<S_, L_, false, PG, VG, LOSS, false, COOP_, COOP_>;                             \
@@ -1159,14 +1155,12 @@ static cudaError_t launch_bwd_g(const RenderParams& p, bool pg, bool vg, unsigne
             const size_t smem_ = ((size_t)p.att_slots_padded + (size_t)nw_ * BWD_SMEM_PER_WARP + CoopXch::FLOATS) * sizeof(float); \
             cudaError_t e = ensure_smem(k, smem_, 16 / nw_);                                                          \
             if (e != cudaSuccess) return e;                                                                           \
-            k<<<(unsigned)p.total_rays, nw_ * 32, smem_, st>>>(p);                                                    \
-            return cudaGetLastError();                                                                                \
+            return launch_kernel(k, (unsigned)p.total_rays, nw_ * 32, smem_, st, p);                                  \
         }                                                                                                             \
         auto k = render_bwd_kernel<S_, L_, P64_, PG, VG, LOSS, false>;                                                \
         cudaError_t e = ensure_smem(k, smem, 16 / (threads / 32));                                                    \
         if (e != cudaSuccess) return e;                                                                               \
-        k<<<grid, threads, smem, st>>>(p);                                                                            \
-        return cudaGetLastError();                                                                                    \
+        return launch_kernel(k, grid, threads, smem, st, p);                                                          \
     }
     if (!TRI) pg = false;                      // no pose gradient exists (round+long cuts the graph)
     if (pg && vg) DIFFUS_BWD_GO(TRI, true)
@@ -1216,8 +1210,7 @@ cudaError_t launch_render_bwd(const RenderParams& p, int sampler, int layout, in
 cudaError_t launch_echo_fwd(const float* refl, int64_t n_rays, int N, float* echo, cudaStream_t st) {
     int wpb = warps_per_block(n_rays);
     size_t smem = (size_t)wpb * 2 * FwdGeo::OBUF * sizeof(float);
-    echo_fwd_kernel<<<(unsigned)((n_rays + wpb - 1) / wpb), wpb * 32, smem, st>>>(refl, n_rays, N, echo);
-    return cudaGetLastError();
+    return launch_kernel(echo_fwd_kernel, (unsigned)((n_rays + wpb - 1) / wpb), wpb * 32, smem, st, refl, n_rays, N, echo);
 }
 
 cudaError_t launch_echo_bwd(const float* refl, const float* grad_echo, int64_t n_rays, int N, float* grad_refl,
@@ -1227,8 +1220,7 @@ cudaError_t launch_echo_bwd(const float* refl, const float* grad_echo, int64_t n
     size_t smem = (size_t)wpb * (2 * BwdGeo::OBUF + 4 * nseg) * sizeof(float);
     cudaError_t e = ensure_smem(echo_bwd_kernel, smem);
     if (e != cudaSuccess) return e;
-    echo_bwd_kernel<<<(unsigned)((n_rays + wpb - 1) / wpb), wpb * 32, smem, st>>>(refl, grad_echo, n_rays, N, grad_refl);
-    return cudaGetLastError();
+    return launch_kernel(echo_bwd_kernel, (unsigned)((n_rays + wpb - 1) / wpb), wpb * 32, smem, st, refl, grad_echo, n_rays, N, grad_refl);
 }
 #endif  // DIFFUS_LAYOUT_SLICE
 

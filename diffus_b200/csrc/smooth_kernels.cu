@@ -111,14 +111,15 @@ cudaError_t launch_gaussian_blur(const float* src, const int32_t dim[3], float s
     const BlurTaps taps = gaussian_taps((double)sigma, r);
     const int64_t max_ctas = (int64_t)148 * 32;
     const int64_t t2 = D * H * ((W + P2_SEG - 1) / P2_SEG);
-    blur_p2_kernel<<<(unsigned)min(t2, max_ctas), P2_THREADS, (P2_SEG + 2 * r) * sizeof(float), st>>>(src, dst, D * H, (int)W, r,
-                                                                                                         taps);
+    cudaError_t e = launch_kernel(blur_p2_kernel, (unsigned)min(t2, max_ctas), P2_THREADS, (P2_SEG + 2 * r) * sizeof(float), st, src, dst,
+                                  D * H, (int)W, r, taps);
+    if (e != cudaSuccess) return e;
     const size_t smem = (size_t)(SR_SEG + 2 * r) * SR_LANES * sizeof(float);
     const int64_t t1 = D * ((H + SR_SEG - 1) / SR_SEG) * ((W + SR_LANES - 1) / SR_LANES);
-    blur_strided_kernel<<<(unsigned)min(t1, max_ctas), SR_LANES * SR_WARPS, smem, st>>>(dst, scratch, D, (int)H, W, r, taps);
+    e = launch_kernel(blur_strided_kernel, (unsigned)min(t1, max_ctas), SR_LANES * SR_WARPS, smem, st, dst, scratch, D, (int)H, W, r, taps);
+    if (e != cudaSuccess) return e;
     const int64_t t0 = ((D + SR_SEG - 1) / SR_SEG) * ((H * W + SR_LANES - 1) / SR_LANES);
-    blur_strided_kernel<<<(unsigned)min(t0, max_ctas), SR_LANES * SR_WARPS, smem, st>>>(scratch, dst, 1, (int)D, H * W, r, taps);
-    return cudaGetLastError();
+    return launch_kernel(blur_strided_kernel, (unsigned)min(t0, max_ctas), SR_LANES * SR_WARPS, smem, st, scratch, dst, 1, (int)D, H * W, r, taps);
 }
 
 }  // namespace diffus

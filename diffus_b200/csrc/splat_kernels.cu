@@ -143,10 +143,11 @@ static cudaError_t splat_prepare(const float* c0, const float* c1, const float* 
     unsigned long long* keys = (unsigned long long*)((char*)ws + 256);
     cudaError_t e = cudaMemsetAsync(ws, 0, 256 + (size_t)H * W * 8, st);
     if (e != cudaSuccess) return e;
-    splat_stats_kernel<<<grid_for(n), 256, 0, st>>>(c0, c1, c2, n, stats);
-    splat_axes_kernel<<<1, 1, 0, st>>>(stats, n);
-    splat_scatter_kernel<<<grid_for(n), 256, 0, st>>>(c0, c1, c2, val, n, H, W, stats, keys);
-    return cudaGetLastError();
+    e = launch_kernel(splat_stats_kernel, grid_for(n), 256, 0, st, c0, c1, c2, n, stats);
+    if (e != cudaSuccess) return e;
+    e = launch_kernel(splat_axes_kernel, 1, 1, 0, st, stats, n);
+    if (e != cudaSuccess) return e;
+    return launch_kernel(splat_scatter_kernel, grid_for(n), 256, 0, st, c0, c1, c2, val, n, H, W, stats, keys);
 }
 
 cudaError_t launch_splat_fwd(const float* c0, const float* c1, const float* c2, const float* val, int64_t n, int H, int W,
@@ -156,8 +157,7 @@ cudaError_t launch_splat_fwd(const float* c0, const float* c1, const float* c2, 
     cudaError_t e = splat_prepare(c0, c1, c2, val, n, H, W, ws, st);
     if (e != cudaSuccess) return e;
     const unsigned long long* keys = (const unsigned long long*)((char*)ws + 256);
-    splat_blur_kernel<0><<<grid_for((int64_t)H * W), 256, 0, st>>>(keys, nullptr, H, W, K, sigma, out);
-    return cudaGetLastError();
+    return launch_kernel(splat_blur_kernel<0>, grid_for((int64_t)H * W), 256, 0, st, keys, nullptr, H, W, K, sigma, out);
 }
 
 cudaError_t launch_splat_bwd(const float* c0, const float* c1, const float* c2, const float* val, int64_t n, int H, int W,
@@ -170,10 +170,11 @@ cudaError_t launch_splat_bwd(const float* c0, const float* c1, const float* c2, 
     const unsigned long long* keys = (const unsigned long long*)((char*)ws + 256);
     float* g2 = (float*)((char*)ws + 256 + (size_t)H * W * 8);
     float* gimg = g2 + (size_t)H * W;
-    splat_blur_kernel<1><<<grid_for((int64_t)H * W), 256, 0, st>>>(keys, grad_out, H, W, K, sigma, g2);
-    splat_blur_kernel<2><<<grid_for((int64_t)H * W), 256, 0, st>>>(keys, g2, H, W, K, sigma, gimg);
-    splat_gather_grad_kernel<<<grid_for(n), 256, 0, st>>>(c0, c1, c2, n, H, W, stats, gimg, grad_val);
-    return cudaGetLastError();
+    e = launch_kernel(splat_blur_kernel<1>, grid_for((int64_t)H * W), 256, 0, st, keys, grad_out, H, W, K, sigma, g2);
+    if (e != cudaSuccess) return e;
+    e = launch_kernel(splat_blur_kernel<2>, grid_for((int64_t)H * W), 256, 0, st, keys, g2, H, W, K, sigma, gimg);
+    if (e != cudaSuccess) return e;
+    return launch_kernel(splat_gather_grad_kernel, grid_for(n), 256, 0, st, c0, c1, c2, n, H, W, stats, gimg, grad_val);
 }
 
 }  // namespace diffus

@@ -43,8 +43,7 @@ __global__ void __launch_bounds__(1024) adam_step_kernel(float* __restrict__ par
 
 cudaError_t launch_adam_step(float* params, const float* grads, float* state, int64_t n, float lr, float beta1, float beta2,
                              float eps, float weight_decay, float grad_scale, cudaStream_t st) {
-    adam_step_kernel<<<1, 1024, 0, st>>>(params, grads, state, (int)n, lr, beta1, beta2, eps, weight_decay, grad_scale);
-    return cudaGetLastError();
+    return launch_kernel(adam_step_kernel, 1, 1024, 0, st, params, grads, state, (int)n, lr, beta1, beta2, eps, weight_decay, grad_scale);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -82,13 +81,11 @@ cudaError_t launch_volume_slice(float* vol, const int32_t dim[3], int layout, in
     const int64_t n = (int64_t)nb * nc;
     const unsigned grid = (unsigned)max((int64_t)1, min((int64_t)148 * 8, (n + 255) / 256));
     if (layout == DIFFUS_LAYOUT_BRICK) {
-        if (scatter) volume_slice_kernel<DIFFUS_LAYOUT_BRICK, true><<<grid, 256, 0, st>>>(vol, v, axis, index, slice, nb, nc);
-        else volume_slice_kernel<DIFFUS_LAYOUT_BRICK, false><<<grid, 256, 0, st>>>(vol, v, axis, index, slice, nb, nc);
-    } else {
-        if (scatter) volume_slice_kernel<DIFFUS_LAYOUT_LINEAR, true><<<grid, 256, 0, st>>>(vol, v, axis, index, slice, nb, nc);
-        else volume_slice_kernel<DIFFUS_LAYOUT_LINEAR, false><<<grid, 256, 0, st>>>(vol, v, axis, index, slice, nb, nc);
+        if (scatter) return launch_kernel(volume_slice_kernel<DIFFUS_LAYOUT_BRICK, true>, grid, 256, 0, st, vol, v, axis, index, slice, nb, nc);
+        return launch_kernel(volume_slice_kernel<DIFFUS_LAYOUT_BRICK, false>, grid, 256, 0, st, vol, v, axis, index, slice, nb, nc);
     }
-    return cudaGetLastError();
+    if (scatter) return launch_kernel(volume_slice_kernel<DIFFUS_LAYOUT_LINEAR, true>, grid, 256, 0, st, vol, v, axis, index, slice, nb, nc);
+    return launch_kernel(volume_slice_kernel<DIFFUS_LAYOUT_LINEAR, false>, grid, 256, 0, st, vol, v, axis, index, slice, nb, nc);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -107,8 +104,7 @@ __global__ void rotate_apex_kernel(const float* __restrict__ x, const float* __r
 cudaError_t launch_rotate_apex(const float* x, const float* z, int64_t n, float cos_a, float sin_a, float shift, float apex0,
                                float apex1, float* xr, float* zr, cudaStream_t st) {
     const unsigned grid = (unsigned)max((int64_t)1, min((int64_t)148 * 8, (n + 255) / 256));
-    rotate_apex_kernel<<<grid, 256, 0, st>>>(x, z, n, cos_a, sin_a, shift, apex0, apex1, xr, zr);
-    return cudaGetLastError();
+    return launch_kernel(rotate_apex_kernel, grid, 256, 0, st, x, z, n, cos_a, sin_a, shift, apex0, apex1, xr, zr);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -170,12 +166,10 @@ __global__ void __launch_bounds__(1024) log_compress_bwd_kernel(const float* __r
 }
 
 cudaError_t launch_log_compress_fwd(const float* x, int64_t n, float* out, float* max_out, cudaStream_t st) {
-    log_compress_fwd_kernel<<<1, 1024, 0, st>>>(x, n, out, max_out);
-    return cudaGetLastError();
+    return launch_kernel(log_compress_fwd_kernel, 1, 1024, 0, st, x, n, out, max_out);
 }
 cudaError_t launch_log_compress_bwd(const float* x, const float* gout, int64_t n, float* gx, cudaStream_t st) {
-    log_compress_bwd_kernel<<<1, 1024, 0, st>>>(x, gout, n, gx);
-    return cudaGetLastError();
+    return launch_kernel(log_compress_bwd_kernel, 1, 1024, 0, st, x, gout, n, gx);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -244,24 +238,24 @@ cudaError_t launch_conv1d_rows(const float* in, int64_t rows, int n_in, const fl
                                int n_out, cudaStream_t st) {
     const int64_t total = rows * n_out;
     const unsigned grid = (unsigned)max((int64_t)1, min((total + 255) / 256, (int64_t)148 * 8));
-    conv1d_rows_kernel<<<grid, 256, 0, st>>>(in, rows, n_in, w, taps, pad, flip, out, n_out);
-    return cudaGetLastError();
+    return launch_kernel(conv1d_rows_kernel, grid, 256, 0, st, in, rows, n_in, w, taps, pad, flip, out, n_out);
 }
 
 __global__ void zero_word_kernel(unsigned* w) { *w = 0u; }
 
 cudaError_t launch_rf_to_bmode(const float* rf, int64_t n_rays, int S, const float* g, float* out, void* workspace, cudaStream_t st) {
     unsigned* max_bits = (unsigned*)workspace;
-    zero_word_kernel<<<1, 1, 0, st>>>(max_bits);
+    cudaError_t e = launch_kernel(zero_word_kernel, 1, 1, 0, st, max_bits);
+    if (e != cudaSuccess) return e;
     const size_t smem = (size_t)2 * S * sizeof(float);
     if (smem > 48 * 1024) {
-        cudaError_t e = ensure_smem(rf_envelope_kernel, smem);
+        e = ensure_smem(rf_envelope_kernel, smem);
         if (e != cudaSuccess) return e;
     }
-    rf_envelope_kernel<<<(unsigned)n_rays, 256, smem, st>>>(rf, S, g, out, max_bits);
+    e = launch_kernel(rf_envelope_kernel, (unsigned)n_rays, 256, smem, st, rf, S, g, out, max_bits);
+    if (e != cudaSuccess) return e;
     const int64_t n = n_rays * S;
-    rf_normalise_kernel<<<(unsigned)max((int64_t)1, min((int64_t)148 * 8, (n + 255) / 256)), 256, 0, st>>>(out, n, max_bits);
-    return cudaGetLastError();
+    return launch_kernel(rf_normalise_kernel, (unsigned)max((int64_t)1, min((int64_t)148 * 8, (n + 255) / 256)), 256, 0, st, out, n, max_bits);
 }
 
 }  // namespace diffus

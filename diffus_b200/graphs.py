@@ -11,7 +11,35 @@ import torch
 
 from . import ops
 from ._lib import SAMPLER_TRILINEAR
-from .renderer import PreparedVolume, _resolve_start, _sampler_id
+from .renderer import _resolve_start, _sampler_id, _target, _unwrap
+
+
+def _capture(dev, step, prime=None):
+    """Run ``prime`` and then ``step`` twice on a side stream (lazy module loads, kernel attributes, library handles), then
+    capture ``step`` into a CUDA graph.  Returns the graph and what the captured ``step`` returned."""
+    side = torch.cuda.Stream(device=dev)
+    side.wait_stream(torch.cuda.current_stream(dev))
+    with torch.cuda.stream(side):
+        if prime is not None:
+            prime()
+        for _ in range(2):
+            step()
+    torch.cuda.current_stream(dev).wait_stream(side)
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        out = step()
+    return graph, out
+
+
+def _ray_fn(probe: str, opening_angle, radius, width, n_rays: int):
+    """``(rays, args)``: ``rays(poses)`` gives the (origins, directions) of (3,P,3) pose parameters [sources | median | hint]
+    -- a sector fan's origins are its (P,3) sources, an array probe has one origin per ray (P,R,3) -- and ``args`` the
+    ``(kind id, angle, radius, width)`` of an array probe for ``ops.probe_rays_*`` (None for a sector fan)."""
+    if probe == "sector":
+        return (lambda poses: (poses[0], ops.fan_directions_fwd(poses[1], poses[2], opening_angle, n_rays))), None
+    args = ops.probe_args(probe, opening_angle, radius, width)
+    kid, angle, rho, wid = args
+    return (lambda poses: ops.probe_rays_fwd(kid, poses[0], poses[1], poses[2], n_rays, angle, rho, wid)), args
 
 
 class GraphedPoseStep:
@@ -23,14 +51,9 @@ class GraphedPoseStep:
 
     def __init__(self, volume, targets: torch.Tensor, n_rays: int, num_samples: int, attenuation_coeff: float = 0.5,
                  start=0, sampler: str = "trilinear", shared_directions: bool = False):
-        if isinstance(volume, PreparedVolume):
-            bricks, vol = volume.bricks, volume.volume
-        else:
-            bricks, vol = None, volume.float().contiguous()
+        vol, bricks = _unwrap(volume)
         dev = vol.device
-        tgt = targets.to(torch.float32).contiguous()
-        if tgt.dim() == 2:
-            tgt = tgt.unsqueeze(0)
+        tgt = _target(targets)
         P = tgt.shape[0]
         self.sources = torch.zeros((P, 3), dtype=torch.float32, device=dev)
         self.directions = torch.zeros((n_rays, 3) if shared_directions else (P, n_rays, 3), dtype=torch.float32, device=dev)
@@ -38,15 +61,7 @@ class GraphedPoseStep:
         args = (vol, bricks, list(vol.shape), self.sources, self.directions, tgt, int(num_samples),
                 _resolve_start(start, num_samples), float(attenuation_coeff), _sampler_id(sampler), False, False,
                 _sampler_id(sampler) == SAMPLER_TRILINEAR, False)
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):                      # warm up outside capture (lazy module loads, attributes)
-            for _ in range(2):
-                ops.render_mse_impl(*args)
-        torch.cuda.current_stream(dev).wait_stream(side)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            self.loss, _, _, self.grad_sources, self.grad_directions = ops.render_mse_impl(*args)
+        self.graph, (self.loss, _, _, self.grad_sources, self.grad_directions) = _capture(dev, lambda: ops.render_mse_impl(*args))
         self._keep = args
 
     def __call__(self, sources: torch.Tensor, directions: torch.Tensor):
@@ -73,10 +88,8 @@ class GraphedFanPoseStep:
                  attenuation_coeff: float = 0.5, start=0, *, probe: str = "sector", radius=None, width=None):
         from .pose_recovery import probe_keywords
         probe, radius, width = probe_keywords(probe, radius, width)
-        if isinstance(volume, PreparedVolume):
-            bricks, vol = volume.bricks, volume.volume
-        else:
-            bricks, vol = None, volume.float().contiguous()
+        rays, probe_args = _ray_fn(probe, opening_angle, radius, width, n_rays)
+        vol, bricks = _unwrap(volume)
         dev = vol.device
         tgt = targets.to(torch.float32).contiguous()
         P = tgt.shape[0]
@@ -94,30 +107,17 @@ class GraphedFanPoseStep:
         o_gs, o_gm, o_gh, o_loss = self.out[:3 * P], self.out[3 * P:6 * P], self.out[6 * P:9 * P], self.out[9 * P:]
 
         def step():
-            if probe != "sector":
-                kid, angle, rho, w = ops.probe_args(probe, opening_angle, radius, width)
-                org, dirs = ops.probe_rays_fwd(kid, self.sources, self.median, self.hint, n_rays, angle, rho, w)
-                _, _, _, go, gd = ops.render_mse_impl(vol, bricks, list(vol.shape), org, dirs, tgt, int(num_samples), start_i,
-                                                      float(attenuation_coeff), SAMPLER_TRILINEAR, False, False, True, False,
-                                                      loss_out=o_loss)
-                ops.probe_rays_bwd(kid, self.sources, self.median, self.hint, go, gd, n_rays, angle, rho, w, grad_centre_out=o_gs,
-                                   grad_median_out=o_gm, grad_hint_out=o_gh)
-                return
-            dirs = ops.fan_directions_fwd(self.median, self.hint, opening_angle, n_rays)
-            _, _, _, _, gd = ops.render_mse_impl(vol, bricks, list(vol.shape), self.sources, dirs, tgt, int(num_samples),
-                                                 start_i, float(attenuation_coeff), SAMPLER_TRILINEAR, False, False, True,
-                                                 False, loss_out=o_loss, grad_sources_out=o_gs)
-            ops.fan_directions_bwd(self.median, self.hint, gd, opening_angle, n_rays, grad_median_out=o_gm, grad_hint_out=o_gh)
+            org, dirs = rays(self.poses)
+            _, _, _, go, gd = ops.render_mse_impl(vol, bricks, list(vol.shape), org, dirs, tgt, int(num_samples), start_i,
+                                                  float(attenuation_coeff), SAMPLER_TRILINEAR, False, False, True, False,
+                                                  loss_out=o_loss, grad_sources_out=None if probe_args else o_gs)
+            if probe_args:
+                ops.probe_rays_bwd(probe_args[0], self.sources, self.median, self.hint, go, gd, n_rays, *probe_args[1:],
+                                   grad_centre_out=o_gs, grad_median_out=o_gm, grad_hint_out=o_gh)
+            else:
+                ops.fan_directions_bwd(self.median, self.hint, gd, opening_angle, n_rays, grad_median_out=o_gm, grad_hint_out=o_gh)
 
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):                      # warm up outside capture
-            for _ in range(2):
-                step()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            step()
+        self.graph, _ = _capture(dev, step)
         self.P = P
         self.loss = self.out[9 * P]
         self.grad_sources = self.out[:3 * P].view(P, 3)
@@ -162,7 +162,36 @@ def _solve_spd6(a: torch.Tensor, b: torch.Tensor):
     return x, ok
 
 
-class GraphedFanGaussNewtonStep:
+class _LevenbergMarquardt:
+    """The Marquardt-damped solve and the accept / reject of the graphed Gauss-Newton steps, on the static ``jtj``, ``jtr``,
+    ``loss``, ``lam`` and candidate ``c_loss`` of a subclass."""
+
+    LAM_DOWN, LAM_UP, LAM_MIN, LAM_MAX = 1.0 / 3.0, 4.0, 1e-9, 1e9
+
+    def _delta(self, jtj: torch.Tensor, jtr: torch.Tensor) -> torch.Tensor:
+        """The float64 step of the batched systems (P,6,6), (P,6): ``(JtJ + lam diag(JtJ) + eps I) delta = -Jtr``; zero where the
+        damped system is not positive definite or the step is not finite."""
+        a = jtj.double()
+        d = a.diagonal(dim1=-2, dim2=-1)
+        eps = 1e-12 * d.amax(-1, keepdim=True) + 1e-30
+        a = a + torch.diag_embed(self.lam[:, None] * d + eps)
+        delta, ok = _solve_spd6(a, -jtr.double())
+        ok = ok & torch.isfinite(delta).all(-1)
+        return torch.where(ok[:, None], delta, torch.zeros_like(delta))
+
+    def _accept(self, *pairs) -> None:
+        """Where the candidate's loss went down, copy each ``(candidate, state[, pose dim])`` over the state and shrink ``lam``;
+        else keep the state and grow ``lam``.  (NaN: rejected.)  ``pose dim``: the dimension of the state that runs over the
+        poses of the (P,) loss, 0 if not given."""
+        acc = self.c_loss < self.loss
+        for cand, cur, *dim in pairs:
+            d = dim[0] if dim else 0
+            mask = acc.reshape((1,) * d + acc.shape + (1,) * (cur.dim() - d - acc.dim()))
+            cur.copy_(torch.where(mask, cand, cur))
+        self.lam.copy_(torch.where(acc, self.lam * self.LAM_DOWN, self.lam * self.LAM_UP).clamp(self.LAM_MIN, self.LAM_MAX))
+
+
+class GraphedFanGaussNewtonStep(_LevenbergMarquardt):
     """One Levenberg-Marquardt iteration of fan pose recovery as one CUDA-graph replay (see ``pose_recovery.recover_poses``).
 
     Static state on the device: the current poses (``sources``, ``median``, ``hint``, (P,3) each), their loss (P,), JtJ
@@ -176,19 +205,12 @@ class GraphedFanGaussNewtonStep:
     ``apply_probe_twist`` about the pivot of the current origins -- the point the kernel's twist turns about.
     """
 
-    LAM_DOWN, LAM_UP, LAM_MIN, LAM_MAX = 1.0 / 3.0, 4.0, 1e-9, 1e9
-
     def __init__(self, volume, targets: torch.Tensor, n_rays: int, num_samples: int, opening_angle: float,
                  attenuation_coeff: float = 0.5, start=0, *, probe: str = "sector", radius=None, width=None):
         from .pose_recovery import apply_fan_twist, apply_probe_twist, probe_keywords, probe_pivot
         probe, radius, width = probe_keywords(probe, radius, width)
-        array = probe != "sector"
-        if array:
-            kid, angle, rho, wid = ops.probe_args(probe, opening_angle, radius, width)
-        if isinstance(volume, PreparedVolume):
-            bricks, vol = volume.bricks, volume.volume
-        else:
-            bricks, vol = None, volume.float().contiguous()
+        rays, array = _ray_fn(probe, opening_angle, radius, width, n_rays)
+        vol, bricks = _unwrap(volume)
         dev = vol.device
         tgt = targets.to(torch.float32).contiguous()
         P = tgt.shape[0]
@@ -206,48 +228,24 @@ class GraphedFanGaussNewtonStep:
         self.lam = torch.ones((P,), dtype=torch.float64, device=dev)
 
         def system(poses, loss, jtj, jtr):
-            if array:
-                src, dirs = ops.probe_rays_fwd(kid, poses[0], poses[1], poses[2], n_rays, angle, rho, wid)
-            else:
-                src, dirs = poses[0], ops.fan_directions_fwd(poses[1], poses[2], opening_angle, n_rays)
+            src, dirs = rays(poses)
             ops.render_gauss_newton_impl(vol, bricks, list(vol.shape), src, dirs, tgt, int(num_samples), start_i,
                                          float(attenuation_coeff), loss_out=loss, jtj_out=jtj, jtr_out=jtr)
 
         def step():
-            a = self.jtj.double()
-            d = a.diagonal(dim1=-2, dim2=-1)
-            eps = 1e-12 * d.amax(-1, keepdim=True) + 1e-30
-            a = a + torch.diag_embed(self.lam[:, None] * d + eps)
-            delta, ok = _solve_spd6(a, -self.jtr.double())
-            ok = ok & torch.isfinite(delta).all(-1)
-            delta = torch.where(ok[:, None], delta, torch.zeros_like(delta)).float()
+            delta = self._delta(self.jtj, self.jtr).float()
             if array:
-                org, _ = ops.probe_rays_fwd(kid, self.sources, self.median, self.hint, n_rays, angle, rho, wid)
-                s, m, h = apply_probe_twist(self.sources, self.median, self.hint, delta, probe_pivot(org))
+                s, m, h = apply_probe_twist(self.sources, self.median, self.hint, delta, probe_pivot(rays(self.poses)[0]))
             else:
                 s, m, h = apply_fan_twist(self.sources, self.median, self.hint, delta)
             self.cand[0].copy_(s)
             self.cand[1].copy_(m)
             self.cand[2].copy_(h)
             system(self.cand, self.c_loss, self.c_jtj, self.c_jtr)
-            acc = self.c_loss < self.loss                                   # (NaN: rejected)
-            self.poses.copy_(torch.where(acc[None, :, None], self.cand, self.poses))
-            self.loss.copy_(torch.where(acc, self.c_loss, self.loss))
-            self.jtj.copy_(torch.where(acc[:, None, None], self.c_jtj, self.jtj))
-            self.jtr.copy_(torch.where(acc[:, None], self.c_jtr, self.jtr))
-            self.lam.copy_(torch.where(acc, self.lam * self.LAM_DOWN, self.lam * self.LAM_UP).clamp(self.LAM_MIN, self.LAM_MAX))
+            self._accept((self.cand, self.poses, 1), (self.c_loss, self.loss), (self.c_jtj, self.jtj), (self.c_jtr, self.jtr))
 
         self._system = system
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):                      # warm up outside capture (lazy module loads, library handles)
-            system(self.poses, self.loss, self.jtj, self.jtr)
-            for _ in range(2):
-                step()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            step()
+        self.graph, _ = _capture(dev, step, lambda: system(self.poses, self.loss, self.jtj, self.jtr))
         self._keep = (vol, bricks, tgt)
 
     def reset(self, sources: torch.Tensor, median: torch.Tensor, hint: torch.Tensor, damping: float = 1e-3) -> None:
@@ -264,7 +262,7 @@ class GraphedFanGaussNewtonStep:
         return self.loss
 
 
-class GraphedSweepGaussNewtonStep:
+class GraphedSweepGaussNewtonStep(_LevenbergMarquardt):
     """One Levenberg-Marquardt iteration of tracked-sweep registration as one CUDA-graph replay (see
     ``pose_recovery.register_sweep``).
 
@@ -278,20 +276,12 @@ class GraphedSweepGaussNewtonStep:
     :class:`GraphedFanGaussNewtonStep`.
     """
 
-    LAM_DOWN, LAM_UP, LAM_MIN, LAM_MAX = GraphedFanGaussNewtonStep.LAM_DOWN, GraphedFanGaussNewtonStep.LAM_UP, \
-        GraphedFanGaussNewtonStep.LAM_MIN, GraphedFanGaussNewtonStep.LAM_MAX
-
     def __init__(self, volume, targets: torch.Tensor, n_rays: int, num_samples: int, opening_angle: float,
                  attenuation_coeff: float = 0.5, start=0, *, probe: str = "sector", radius=None, width=None):
         from .pose_recovery import apply_rigid_transform, compose_sweep_twist, probe_keywords
         probe, radius, width = probe_keywords(probe, radius, width)
-        array = probe != "sector"
-        if array:
-            kid, angle, rho, wid = ops.probe_args(probe, opening_angle, radius, width)
-        if isinstance(volume, PreparedVolume):
-            bricks, vol = volume.bricks, volume.volume
-        else:
-            bricks, vol = None, volume.float().contiguous()
+        rays, array = _ray_fn(probe, opening_angle, radius, width, n_rays)
+        vol, bricks = _unwrap(volume)
         dev = vol.device
         tgt = targets.to(torch.float32).contiguous()
         P = tgt.shape[0]
@@ -311,24 +301,13 @@ class GraphedSweepGaussNewtonStep:
         self.c_loss, self.c_jtj, self.c_jtr = torch.zeros_like(self.loss), torch.zeros_like(self.jtj), torch.zeros_like(self.jtr)
         self.lam = torch.ones((1,), **f64)
 
-        def rays(poses):
-            if array:
-                return ops.probe_rays_fwd(kid, poses[0], poses[1], poses[2], n_rays, angle, rho, wid)
-            return poses[0], ops.fan_directions_fwd(poses[1], poses[2], opening_angle, n_rays)
-
         def system(poses, pivot, loss, jtj, jtr):
             src, dirs = rays(poses)
             ops.render_gauss_newton_sweep_impl(vol, bricks, list(vol.shape), src, dirs, tgt, int(num_samples), start_i,
                                                float(attenuation_coeff), pivot, loss_out=loss, jtj_out=jtj, jtr_out=jtr)
 
         def step():
-            a = self.jtj.unsqueeze(0)
-            d = a.diagonal(dim1=-2, dim2=-1)
-            eps = 1e-12 * d.amax(-1, keepdim=True) + 1e-30
-            a = a + torch.diag_embed(self.lam[:, None] * d + eps)
-            delta, ok = _solve_spd6(a, -self.jtr.unsqueeze(0))
-            ok = ok & torch.isfinite(delta).all(-1)
-            delta = torch.where(ok[:, None], delta, torch.zeros_like(delta))[0]
+            delta = self._delta(self.jtj.unsqueeze(0), self.jtr.unsqueeze(0))[0]
             r, t = compose_sweep_twist(self.rot, self.trans, delta, self.pivot)
             self.c_rot.copy_(r)
             self.c_trans.copy_(t)
@@ -338,31 +317,15 @@ class GraphedSweepGaussNewtonStep:
             self.cand[1].copy_(m)
             self.cand[2].copy_(h)
             system(self.cand, self.c_pivot, self.c_loss, self.c_jtj, self.c_jtr)
-            acc = self.c_loss < self.loss                                   # (NaN: rejected)
-            self.poses.copy_(torch.where(acc, self.cand, self.poses))
-            self.rot.copy_(torch.where(acc, self.c_rot, self.rot))
-            self.trans.copy_(torch.where(acc, self.c_trans, self.trans))
-            self.pivot.copy_(torch.where(acc, self.c_pivot, self.pivot))
-            self.loss.copy_(torch.where(acc, self.c_loss, self.loss))
-            self.jtj.copy_(torch.where(acc, self.c_jtj, self.jtj))
-            self.jtr.copy_(torch.where(acc, self.c_jtr, self.jtr))
-            self.lam.copy_(torch.where(acc, self.lam * self.LAM_DOWN, self.lam * self.LAM_UP).clamp(self.LAM_MIN, self.LAM_MAX))
+            self._accept((self.cand, self.poses), (self.c_rot, self.rot), (self.c_trans, self.trans), (self.c_pivot, self.pivot),
+                         (self.c_loss, self.loss), (self.c_jtj, self.jtj), (self.c_jtr, self.jtr))
 
         def centroid(poses):
             """The float64 mean of all P*R ray origins of ``poses`` (a sector fan's R rays share its source)."""
             return (rays(poses)[0] if array else poses[0]).reshape(-1, 3).double().mean(0)
 
         self._system, self._centroid = system, centroid
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):                      # warm up outside capture (lazy module loads, library handles)
-            system(self.poses, self.pivot, self.loss, self.jtj, self.jtr)
-            for _ in range(2):
-                step()
-        torch.cuda.current_stream(dev).wait_stream(side)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            step()
+        self.graph, _ = _capture(dev, step, lambda: system(self.poses, self.pivot, self.loss, self.jtj, self.jtr))
         self._keep = (vol, bricks, tgt)
 
     def reset(self, sources: torch.Tensor, median: torch.Tensor, hint: torch.Tensor, damping: float = 1e-3) -> None:

@@ -19,16 +19,10 @@ from ._lib import (LAYOUT_BRICK, LAYOUT_LINEAR, LAYOUT_QUAD, LAYOUT_TEXTURE, MLP
 
 SEG = 512  # PREFIX_STRIDE of csrc/common.cuh: the forward saves a 2x2 prefix every SEG columns
 
-_LAUNCHES = 0  # kernels enqueued through this module (bench.py reports it as gpu_launches)
-
 
 def launch_count() -> int:
-    return _LAUNCHES
-
-
-def _count(n: int) -> None:
-    global _LAUNCHES
-    _LAUNCHES += n
+    """Kernels this process has enqueued through the library (bench.py reports it as gpu_launches)."""
+    return _lib.load().diffus_launch_count()
 
 
 def _require_cuda(*tensors: torch.Tensor) -> torch.device:
@@ -105,7 +99,6 @@ class VolumeTexture:
             self.token = torch.zeros((1,), dtype=torch.int64, device=dev)
         self.texture, self.array = tex.value, arr.value
         _TEXTURES[self.token.data_ptr()] = self
-        _count(1)
 
     def update(self, volume: torch.Tensor) -> None:
         v = volume.detach().contiguous().float()
@@ -114,7 +107,6 @@ class VolumeTexture:
         with torch.cuda.device(self.device):
             _lib.check(_lib.load().diffus_volume_texture_update(self.array, v.data_ptr(), C.byref((C.c_int32 * 3)(*self.dims)),
                                                                 _stream(self.device)), "diffus_volume_texture_update")
-        _count(1)
 
     def close(self) -> None:
         if self.texture:
@@ -158,6 +150,34 @@ def _grad_volume_shape(bricks: Optional[torch.Tensor], dims) -> Tuple[int, ...]:
     if layout == LAYOUT_BRICK:
         return (bricks.numel(),)
     return (_lib.load().diffus_brick_elems(C.byref((C.c_int32 * 3)(*dims))),)
+
+
+def _zero_grad_volume(bricks: Optional[torch.Tensor], dims, dev) -> torch.Tensor:
+    """The zero-filled buffer d loss / d volume is accumulated into, in the layout of :func:`_grad_volume_shape`."""
+    return torch.zeros(_grad_volume_shape(bricks, dims), dtype=torch.float32, device=dev)
+
+
+def _linear_grad_volume(gvol: torch.Tensor, bricks: Optional[torch.Tensor], dims) -> torch.Tensor:
+    """The gradient of a packed volume comes back in bricks: convert it to the (D,H,W) layout of the volume tensor."""
+    return from_bricks(gvol, dims) if bricks is not None and bricks.numel() > 0 else gvol
+
+
+def _pose_grad(need_pose: bool, sampler: int) -> bool:
+    """Only the trilinear sampler has a pose derivative."""
+    return bool(need_pose) and sampler == SAMPLER_TRILINEAR
+
+
+def _check_target(target: torch.Tensor, P: int, R: int, sout: int) -> None:
+    if tuple(target.shape) != (P, R, sout) or target.dtype != torch.float32 or not target.is_contiguous():
+        raise _lib.DiffusError(f"target must be contiguous float32 {(P, R, sout)}")
+
+
+def _workspace(args, nbytes: int, dev) -> torch.Tensor:
+    """Scratch of ``nbytes`` (from the entry point's ``*_workspace_bytes``) set in ``args``; the caller keeps the tensor alive
+    until the call is enqueued."""
+    ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=dev)
+    args.workspace, args.workspace_bytes = ws.data_ptr(), nbytes
+    return ws
 
 
 def _fill_render_args(a: DiffusRenderArgs, volume, bricks, dims, sources, directions, n_samples, start, alpha,
@@ -232,13 +252,8 @@ def render_fwd_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: 
         a.frame = frame.data_ptr() if frame.numel() else None
         a.seg_prefix = _ptr(prefix)
         wbytes = lib.diffus_render_workspace_bytes(C.byref(a)) if start > 0 else 0      # only the median needs scratch
-        if wbytes:
-            ws = torch.empty((wbytes,), dtype=torch.uint8, device=dev)
-            a.workspace, a.workspace_bytes = ws.data_ptr(), wbytes
-        else:
-            a.workspace, a.workspace_bytes = None, 0
+        ws = _workspace(a, wbytes, dev) if wbytes else None
         _lib.check(lib.diffus_render_forward(C.byref(a), _stream(dev)), "diffus_render_forward")
-        _count(2 if start > 0 else 1)
     return frame, prefix
 
 
@@ -271,26 +286,19 @@ def render_bwd_impl(grad_frame: torch.Tensor, volume: torch.Tensor, bricks: Opti
         P, R = _fill_render_args(b.fwd, volume, bricks, dims, sources, directions, n_samples, start, alpha,
                                  sampler, product_f32)
         grad_frame = grad_frame.contiguous().float()
-        need_pose = need_pose and sampler == SAMPLER_TRILINEAR
-        use_bricks = bricks is not None and bricks.numel() > 0
-        gshape = _grad_volume_shape(bricks, dims)
-        gvol = torch.zeros(gshape, dtype=torch.float32, device=dev) if need_volume else \
-            torch.empty((0,), dtype=torch.float32, device=dev)
+        need_pose = _pose_grad(need_pose, sampler)
+        gvol = _zero_grad_volume(bricks, dims, dev) if need_volume else torch.empty((0,), dtype=torch.float32, device=dev)
         gsrc = torch.empty(tuple(sources.shape) if need_pose else (0,), dtype=torch.float32, device=dev)
         gdir = torch.empty((P, R, 3) if need_pose else (0,), dtype=torch.float32, device=dev)
         b.fwd.seg_prefix = _ptr(prefix)
         b.grad_frame = grad_frame.data_ptr()
         b.grad_volume, b.grad_sources, b.grad_directions = _ptr(gvol), _ptr(gsrc), _ptr(gdir)
         b.target, b.loss, b.fwd.frame = None, None, None
-        wbytes = lib.diffus_render_bwd_workspace_bytes(C.byref(b))
-        ws = torch.empty((max(wbytes, 1),), dtype=torch.uint8, device=dev)
-        b.workspace, b.workspace_bytes = ws.data_ptr(), wbytes
+        ws = _workspace(b, lib.diffus_render_bwd_workspace_bytes(C.byref(b)), dev)
         b.fwd.workspace, b.fwd.workspace_bytes = None, 0
         _lib.check(lib.diffus_render_backward(C.byref(b), _stream(dev)), "diffus_render_backward")
-        fold = need_pose and sources.dim() == 2           # per-ray origins: no reduction over the rays
-        _count((1 if (need_volume or need_pose) else 0) + (2 if start > 0 else 0) + (1 if fold else 0))
-        if need_volume and use_bricks:
-            gvol = from_bricks(gvol, dims)
+        if need_volume:
+            gvol = _linear_grad_volume(gvol, bricks, dims)
     return gvol, gsrc, gdir
 
 
@@ -306,7 +314,7 @@ def render_bwd(grad_frame: torch.Tensor, volume: torch.Tensor, bricks: Optional[
 def _(grad_frame, volume, bricks, dims, sources, directions, prefix, n_samples, start, alpha, sampler, product_f32,
       need_volume, need_pose):
     P, R = sources.shape[0], directions.shape[-2]
-    need_pose = need_pose and sampler == SAMPLER_TRILINEAR
+    need_pose = _pose_grad(need_pose, sampler)
     gvol = volume.new_empty(tuple(dims) if need_volume else (0,), dtype=torch.float32)
     gsrc = volume.new_empty(tuple(sources.shape) if need_pose else (0,), dtype=torch.float32)
     gdir = volume.new_empty((P, R, 3) if need_pose else (0,), dtype=torch.float32)
@@ -321,26 +329,37 @@ def _render_setup(ctx, inputs, output):
     ctx.meta = (list(dims), n_samples, start, alpha, sampler, product_f32, save_prefix)
 
 
-def _render_backward(ctx, grad_frame, grad_prefix):
+def _pose_grads(ctx, need_pose, gs, gd, src_dtype, dir_dtype, dir_dim, scale=None):
+    """d/d sources and d/d directions (inputs 3 and 4) in their dtypes, or None where not requested: the (P,R,3) direction
+    gradient of a fan shared by all poses (R,3) is summed over the poses; ``scale`` multiplies both before the cast."""
+    gsrc = gdir = None
+    if need_pose and ctx.needs_input_grad[3]:
+        gsrc = (gs if scale is None else gs * scale).to(src_dtype)
+    if need_pose and ctx.needs_input_grad[4]:
+        d = gd if dir_dim == 3 else gd.sum(0)
+        gdir = (d if scale is None else d * scale).to(dir_dtype)
+    return gsrc, gdir
+
+
+def _render_grads(ctx, grad_frame, bwd):
+    """The backward of a render: ``(d volume, None, None, d sources, d directions)`` through ``bwd`` (the registered op or its
+    impl) from what :func:`_render_setup` saved."""
     volume, bricks, sources, directions, prefix = ctx.saved_tensors
     dims, n_samples, start, alpha, sampler, product_f32, save_prefix = ctx.meta
     need_volume = ctx.needs_input_grad[0]
-    need_pose = (ctx.needs_input_grad[3] or ctx.needs_input_grad[4]) and sampler == SAMPLER_TRILINEAR
-    sout = n_samples - start
-    if _nseg(sout) > 1 and not save_prefix:
+    need_pose = _pose_grad(ctx.needs_input_grad[3] or ctx.needs_input_grad[4], sampler)
+    if _nseg(n_samples - start) > 1 and not save_prefix:
         raise _lib.DiffusError("render_fwd was called with save_prefix=False but a gradient was requested")
-    gvol = gsrc = gdir = None
-    if need_volume or need_pose:
-        gv, gs, gd = render_bwd(grad_frame, volume, bricks if ctx.has_bricks else None, dims, sources, directions,
-                                prefix, n_samples, start, alpha, sampler, product_f32, need_volume, need_pose)
-        if need_volume:
-            gvol = gv
-        if need_pose and ctx.needs_input_grad[3]:
-            gsrc = gs.to(sources.dtype)
-        if need_pose and ctx.needs_input_grad[4]:
-            gdir = gd if directions.dim() == 3 else gd.sum(0)
-            gdir = gdir.to(directions.dtype)
-    return gvol, None, None, gsrc, gdir, None, None, None, None, None, None
+    if not (need_volume or need_pose):
+        return None, None, None, None, None
+    gv, gs, gd = bwd(grad_frame, volume, bricks if ctx.has_bricks else None, dims, sources, directions, prefix, n_samples,
+                     start, alpha, sampler, product_f32, need_volume, need_pose)
+    gsrc, gdir = _pose_grads(ctx, need_pose, gs, gd, sources.dtype, directions.dtype, directions.dim())
+    return gv if need_volume else None, None, None, gsrc, gdir
+
+
+def _render_backward(ctx, grad_frame, grad_prefix):
+    return _render_grads(ctx, grad_frame, render_bwd) + (None,) * 6
 
 
 torch.library.register_autograd("diffus::render_fwd", _render_backward, setup_context=_render_setup)
@@ -352,30 +371,13 @@ class RenderFunction(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, volume, bricks, dims, sources, directions, n_samples, start, alpha, sampler, product_f32):
-        frame, prefix = render_fwd_impl(volume, bricks, dims, sources, directions, n_samples, start, alpha, sampler,
-                                        product_f32, True)
-        ctx.save_for_backward(volume, sources, directions, prefix)
-        ctx.bricks = bricks
-        ctx.meta = (list(dims), n_samples, start, alpha, sampler, product_f32)
-        return frame
+        out = render_fwd_impl(volume, bricks, dims, sources, directions, n_samples, start, alpha, sampler, product_f32, True)
+        _render_setup(ctx, (volume, bricks, dims, sources, directions, n_samples, start, alpha, sampler, product_f32, True), out)
+        return out[0]
 
     @staticmethod
     def backward(ctx, grad_frame):
-        volume, sources, directions, prefix = ctx.saved_tensors
-        dims, n_samples, start, alpha, sampler, product_f32 = ctx.meta
-        need_volume = ctx.needs_input_grad[0]
-        need_pose = (ctx.needs_input_grad[3] or ctx.needs_input_grad[4]) and sampler == SAMPLER_TRILINEAR
-        gvol = gsrc = gdir = None
-        if need_volume or need_pose:
-            gv, gs, gd = render_bwd_impl(grad_frame, volume, ctx.bricks, dims, sources, directions, prefix, n_samples,
-                                         start, alpha, sampler, product_f32, need_volume, need_pose)
-            if need_volume:
-                gvol = gv
-            if need_pose and ctx.needs_input_grad[3]:
-                gsrc = gs.to(sources.dtype)
-            if need_pose and ctx.needs_input_grad[4]:
-                gdir = (gd if directions.dim() == 3 else gd.sum(0)).to(directions.dtype)
-        return gvol, None, None, gsrc, gdir, None, None, None, None, None
+        return _render_grads(ctx, grad_frame, render_bwd_impl) + (None,) * 5
 
 
 # ---------------------------------------------------------------------------------------
@@ -410,22 +412,20 @@ def render_mse_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: 
         P, R = _fill_render_args(b.fwd, volume, bricks, dims, sources, directions, n_samples, start, alpha,
                                  sampler, product_f32)
         sout = n_samples - start
-        if tuple(target.shape) != (P, R, sout) or target.dtype != torch.float32 or not target.is_contiguous():
-            raise _lib.DiffusError(f"target must be contiguous float32 {(P, R, sout)}")
-        need_pose = need_pose and sampler == SAMPLER_TRILINEAR
+        _check_target(target, P, R, sout)
+        need_pose = _pose_grad(need_pose, sampler)
         n = P * R * sout if n_total is None else int(n_total)
         def empty():                      # outputs of a custom op must not alias each other
             return torch.empty((0,), dtype=torch.float32, device=dev)
         loss = torch.empty((1,), dtype=torch.float32, device=dev) if loss_out is None else loss_out
         frame = torch.empty((P, R, sout), dtype=torch.float32, device=dev) if want_frame else empty()
-        use_bricks = bricks is not None and bricks.numel() > 0
-        gshape = _grad_volume_shape(bricks, dims)
         if need_volume and grad_volume_out is not None:
+            gshape = _grad_volume_shape(bricks, dims)
             if tuple(grad_volume_out.shape) != tuple(gshape) or grad_volume_out.dtype != torch.float32:
                 raise _lib.DiffusError(f"grad_volume_out must be float32 {tuple(gshape)}")
             gvol = grad_volume_out
         else:
-            gvol = torch.zeros(gshape, dtype=torch.float32, device=dev) if need_volume else empty()
+            gvol = _zero_grad_volume(bricks, dims, dev) if need_volume else empty()
         gsrc = _out_buffer(grad_sources_out, tuple(sources.shape), dev, "grad_sources_out") if need_pose else empty()
         gdir = torch.empty((P, R, 3), dtype=torch.float32, device=dev) if need_pose else empty()
         b.grad_frame = None
@@ -440,16 +440,10 @@ def render_mse_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: 
         b.fwd.frame = _ptr(frame)
         b.fwd.seg_prefix = _ptr(prefix)
         b.target, b.grad_scale, b.loss_scale, b.loss = target.data_ptr(), 2.0 / n, 1.0 / n, loss.data_ptr()
-        wbytes = lib.diffus_render_bwd_workspace_bytes(C.byref(b))
-        ws = torch.empty((max(wbytes, 1),), dtype=torch.uint8, device=dev)
-        b.workspace, b.workspace_bytes = ws.data_ptr(), wbytes
+        ws = _workspace(b, lib.diffus_render_bwd_workspace_bytes(C.byref(b)), dev)
         _lib.check(lib.diffus_render_backward(C.byref(b), _stream(dev)), "diffus_render_backward (fused MSE)")
-        # fused kernel + loss reduction (+ the d/dsources reduction: the same launch as the loss up to 2^18 rays) (+ median,
-        # and its backward when a gradient is requested)
-        n_median = (2 if need_volume or need_pose else 1) if start > 0 else 0
-        _count(2 + n_median + (1 if need_pose and sources.dim() == 2 and P * R > (1 << 18) else 0))
-        if need_volume and use_bricks and not keep_brick_grad:
-            gvol = from_bricks(gvol, dims)
+        if need_volume and not keep_brick_grad:
+            gvol = _linear_grad_volume(gvol, bricks, dims)
     return loss, frame, gvol, gsrc, gdir
 
 
@@ -465,7 +459,7 @@ def render_mse(volume: torch.Tensor, bricks: Optional[torch.Tensor], dims: List[
 def _(volume, bricks, dims, sources, directions, target, n_samples, start, alpha, sampler, product_f32, need_volume,
       need_pose, want_frame):
     P, R = sources.shape[0], directions.shape[-2]
-    need_pose = need_pose and sampler == SAMPLER_TRILINEAR
+    need_pose = _pose_grad(need_pose, sampler)
     def e():
         return volume.new_empty((0,), dtype=torch.float32)
     return (volume.new_empty((1,), dtype=torch.float32),
@@ -482,7 +476,7 @@ class RenderMSELoss(torch.autograd.Function):
     def forward(ctx, volume, bricks, dims, sources, directions, target, n_samples, start, alpha, sampler,
                 product_f32, want_frame):
         need_volume = ctx.needs_input_grad[0]
-        need_pose = (ctx.needs_input_grad[3] or ctx.needs_input_grad[4]) and sampler == SAMPLER_TRILINEAR
+        need_pose = _pose_grad(ctx.needs_input_grad[3] or ctx.needs_input_grad[4], sampler)
         loss, frame, gvol, gsrc, gdir = render_mse_impl(volume.detach(), bricks, dims, sources.detach(),
                                                         directions.detach(), target, n_samples, start, alpha, sampler,
                                                         product_f32, need_volume, need_pose, want_frame)
@@ -496,12 +490,7 @@ class RenderMSELoss(torch.autograd.Function):
         gvol, gsrc, gdir = ctx.saved_tensors
         need_volume, need_pose, sdt, ddt, ddim = ctx.flags
         out_v = gvol * gloss if need_volume and ctx.needs_input_grad[0] else None
-        out_s = out_d = None
-        if need_pose and ctx.needs_input_grad[3]:
-            out_s = (gsrc * gloss).to(sdt)
-        if need_pose and ctx.needs_input_grad[4]:
-            d = gdir if ddim == 3 else gdir.sum(0)
-            out_d = (d * gloss).to(ddt)
+        out_s, out_d = _pose_grads(ctx, need_pose, gsrc, gdir, sdt, ddt, ddim, scale=gloss)
         return out_v, None, None, out_s, out_d, None, None, None, None, None, None, None
 
 
@@ -525,18 +514,13 @@ def render_gauss_newton_impl(volume: torch.Tensor, bricks: Optional[torch.Tensor
     with _on_device(dev):
         P, R = _fill_render_args(g.fwd, volume, bricks, dims, sources, directions, n_samples, start, alpha, SAMPLER_TRILINEAR,
                                  False)
-        sout = n_samples - start
-        if tuple(target.shape) != (P, R, sout) or target.dtype != torch.float32 or not target.is_contiguous():
-            raise _lib.DiffusError(f"target must be contiguous float32 {(P, R, sout)}")
+        _check_target(target, P, R, n_samples - start)
         loss = _out_buffer(loss_out, (P,), dev, "loss_out")
         jtj = _out_buffer(jtj_out, (P, 6, 6), dev, "jtj_out")
         jtr = _out_buffer(jtr_out, (P, 6), dev, "jtr_out")
         g.target, g.loss, g.jtr, g.jtj = target.data_ptr(), loss.data_ptr(), jtr.data_ptr(), jtj.data_ptr()
-        wbytes = lib.diffus_render_gauss_newton_workspace_bytes(C.byref(g))
-        ws = torch.empty((max(wbytes, 1),), dtype=torch.uint8, device=dev)
-        g.workspace, g.workspace_bytes = ws.data_ptr(), wbytes
+        ws = _workspace(g, lib.diffus_render_gauss_newton_workspace_bytes(C.byref(g)), dev)
         _lib.check(lib.diffus_render_gauss_newton(C.byref(g), _stream(dev)), "diffus_render_gauss_newton")
-        _count(2 + (2 if start > 0 else 0) + (1 if sources.dim() == 3 else 0))
     return loss.view(P), jtj.view(P, 6, 6), jtr.view(P, 6)
 
 
@@ -563,19 +547,14 @@ def render_gauss_newton_sweep_impl(volume: torch.Tensor, bricks: Optional[torch.
     with _on_device(dev):
         P, R = _fill_render_args(g.fwd, volume, bricks, dims, sources, directions, n_samples, start, alpha, SAMPLER_TRILINEAR,
                                  False)
-        sout = n_samples - start
-        if tuple(target.shape) != (P, R, sout) or target.dtype != torch.float32 or not target.is_contiguous():
-            raise _lib.DiffusError(f"target must be contiguous float32 {(P, R, sout)}")
+        _check_target(target, P, R, n_samples - start)
         loss = _out_buffer(loss_out, (), dev, "loss_out", torch.float64)
         jtj = _out_buffer(jtj_out, (6, 6), dev, "jtj_out", torch.float64)
         jtr = _out_buffer(jtr_out, (6,), dev, "jtr_out", torch.float64)
         g.target, g.loss, g.jtr, g.jtj = target.data_ptr(), loss.data_ptr(), jtr.data_ptr(), jtj.data_ptr()
         g.pivot = None if pivot is None else pivot.data_ptr()
-        wbytes = lib.diffus_render_gauss_newton_sweep_workspace_bytes(C.byref(g))
-        ws = torch.empty((max(wbytes, 1),), dtype=torch.uint8, device=dev)
-        g.workspace, g.workspace_bytes = ws.data_ptr(), wbytes
+        ws = _workspace(g, lib.diffus_render_gauss_newton_sweep_workspace_bytes(C.byref(g)), dev)
         _lib.check(lib.diffus_render_gauss_newton_sweep(C.byref(g), _stream(dev)), "diffus_render_gauss_newton_sweep")
-        _count(3 + (2 if start > 0 else 0) + (2 if pivot is None else 0))
     return loss.view(()), jtj.view(6, 6), jtr.view(6)
 
 
@@ -608,7 +587,6 @@ def ray_indices(dims, sources, directions, n_samples, start, product_f32=False):
         out = torch.empty((3, P, R, n_samples - start), dtype=torch.int64, device=dev)
         _lib.check(lib.diffus_ray_indices(C.byref(a), out[0].data_ptr(), out[1].data_ptr(), out[2].data_ptr(),
                                           _stream(dev)), "diffus_ray_indices")
-        _count(1)
     return out[0], out[1], out[2]
 
 
@@ -622,7 +600,6 @@ def trace_values(volume, bricks, dims, sources, directions, n_samples, sampler, 
         P, R = _fill_render_args(a, volume, bricks, dims, sources, directions, n_samples, 0, 0.0, sampler, product_f32)
         out = torch.empty((P, R, n_samples), dtype=torch.float32, device=dev)
         _lib.check(lib.diffus_trace_values(C.byref(a), out.data_ptr(), _stream(dev)), "diffus_trace_values")
-        _count(1)
     return out
 
 
@@ -643,7 +620,6 @@ def sample_points(volume: torch.Tensor, points: torch.Tensor, sampler: int):
         if n:
             _lib.check(lib.diffus_sample_points(C.byref(vol), pts.data_ptr(), n, sampler, val.data_ptr(), idx[0].data_ptr(),
                                                 idx[1].data_ptr(), idx[2].data_ptr(), _stream(dev)), "diffus_sample_points")
-            _count(1)
     shape = points.shape[:-1]
     return idx[0].reshape(shape), idx[1].reshape(shape), idx[2].reshape(shape), val.reshape(shape)
 
@@ -655,20 +631,17 @@ def trace_values_bwd(grad_values, volume, bricks, dims, sources, directions, n_s
     a = DiffusRenderArgs()
     with _on_device(dev):
         P, R = _fill_render_args(a, volume, bricks, dims, sources, directions, n_samples, 0, 0.0, sampler, product_f32)
-        need_pose = need_pose and sampler == SAMPLER_TRILINEAR
-        use_bricks = bricks is not None and bricks.numel() > 0
+        need_pose = _pose_grad(need_pose, sampler)
         g = grad_values.contiguous().float()
-        gvol = torch.zeros(_grad_volume_shape(bricks, dims), dtype=torch.float32, device=dev) \
-            if need_volume else None
+        gvol = _zero_grad_volume(bricks, dims, dev) if need_volume else None
         gsrc = torch.empty(tuple(sources.shape), dtype=torch.float32, device=dev) if need_pose else None
         gdir = torch.empty((P, R, 3), dtype=torch.float32, device=dev) if need_pose else None
         ws = torch.empty((max(P * R * 12 + 256, 256),), dtype=torch.uint8, device=dev)
         _lib.check(lib.diffus_trace_values_backward(C.byref(a), g.data_ptr(), _ptr(gvol), _ptr(gsrc), _ptr(gdir),
                                                     ws.data_ptr(), ws.numel(), _stream(dev)),
                    "diffus_trace_values_backward")
-        _count(1 + (1 if need_pose and sources.dim() == 2 else 0))
-        if need_volume and use_bricks:
-            gvol = from_bricks(gvol, dims)
+        if need_volume:
+            gvol = _linear_grad_volume(gvol, bricks, dims)
     return gvol, gsrc, gdir
 
 
@@ -687,15 +660,12 @@ class TraceValuesFunction(torch.autograd.Function):
         volume, sources, directions = ctx.saved_tensors
         dims, n_samples, sampler, product_f32 = ctx.meta
         need_volume = ctx.needs_input_grad[0]
-        need_pose = (ctx.needs_input_grad[3] or ctx.needs_input_grad[4]) and sampler == SAMPLER_TRILINEAR
+        need_pose = _pose_grad(ctx.needs_input_grad[3] or ctx.needs_input_grad[4], sampler)
         gvol = gsrc = gdir = None
         if need_volume or need_pose:
             gvol, gs, gd = trace_values_bwd(grad, volume, ctx.bricks, dims, sources, directions, n_samples, sampler,
                                             product_f32, need_volume, need_pose)
-            if need_pose and ctx.needs_input_grad[3]:
-                gsrc = gs.to(sources.dtype)
-            if need_pose and ctx.needs_input_grad[4]:
-                gdir = (gd if directions.dim() == 3 else gd.sum(0)).to(directions.dtype)
+            gsrc, gdir = _pose_grads(ctx, need_pose, gs, gd, sources.dtype, directions.dtype, directions.dim())
         return gvol, None, None, gsrc, gdir, None, None, None
 
 
@@ -710,7 +680,6 @@ def echo_fwd_impl(refl: torch.Tensor) -> torch.Tensor:
     with _on_device(dev):
         out = torch.empty((B, N + 1), dtype=torch.float32, device=dev)
         _lib.check(lib.diffus_echo_forward(r.data_ptr(), B, N, out.data_ptr(), _stream(dev)), "diffus_echo_forward")
-        _count(1)
     return out
 
 
@@ -734,7 +703,6 @@ def echo_bwd_impl(refl: torch.Tensor, grad_echo: torch.Tensor) -> torch.Tensor:
         out = torch.empty((B, N), dtype=torch.float32, device=dev)
         _lib.check(lib.diffus_echo_backward(r.data_ptr(), g.data_ptr(), B, N, out.data_ptr(), _stream(dev)),
                    "diffus_echo_backward")
-        _count(1)
     return out
 
 
@@ -773,7 +741,6 @@ def cone_directions(median: torch.Tensor, opening_angle: float, n_rays: int) -> 
         out = torch.empty((P, n_rays, 3), dtype=torch.float32, device=dev)
         _lib.check(lib.diffus_cone_directions(m.data_ptr(), P, n_rays, float(opening_angle), out.data_ptr(),
                                               _stream(dev)), "diffus_cone_directions")
-        _count(1)
     return out
 
 
@@ -788,7 +755,6 @@ def fan_directions_fwd(median: torch.Tensor, hint: torch.Tensor, opening_angle: 
         out = torch.empty((P, n_rays, 3), dtype=torch.float32, device=dev)
         _lib.check(lib.diffus_fan_directions(m.data_ptr(), h.data_ptr(), P, n_rays, float(opening_angle), out.data_ptr(),
                                              _stream(dev)), "diffus_fan_directions")
-        _count(1)
     return out
 
 
@@ -819,7 +785,6 @@ def fan_directions_bwd(median: torch.Tensor, hint: torch.Tensor, grad_dirs: torc
         _lib.check(lib.diffus_fan_directions_backward(m.data_ptr(), h.data_ptr(), g.data_ptr(), P, n_rays, float(opening_angle),
                                                       gm.data_ptr(), gh.data_ptr(), _stream(dev)),
                    "diffus_fan_directions_backward")
-        _count(1)
     return gm, gh
 
 
@@ -878,7 +843,6 @@ def probe_rays_fwd(kind: int, centre: torch.Tensor, median: torch.Tensor, hint: 
         _lib.check(lib.diffus_probe_rays(kind, c.data_ptr(), m.data_ptr(), h.data_ptr(), P, n_rays, float(opening_angle),
                                          float(radius), float(width), o.data_ptr(), d.data_ptr(), _stream(dev)),
                    "diffus_probe_rays")
-        _count(1)
     return o.view(P, n_rays, 3), d.view(P, n_rays, 3)
 
 
@@ -901,7 +865,6 @@ def probe_rays_bwd(kind: int, centre: torch.Tensor, median: torch.Tensor, hint: 
         _lib.check(lib.diffus_probe_rays_backward(kind, c.data_ptr(), m.data_ptr(), h.data_ptr(), go.data_ptr(), gd.data_ptr(), P,
                                                   n_rays, float(opening_angle), float(radius), float(width), gc.data_ptr(),
                                                   gm.data_ptr(), gh.data_ptr(), _stream(dev)), "diffus_probe_rays_backward")
-        _count(1)
     return gc, gm, gh
 
 
@@ -998,7 +961,6 @@ def to_bricks(volume: torch.Tensor) -> torch.Tensor:
         out = torch.empty((lib.diffus_brick_elems(C.byref(dim)),), dtype=torch.float32, device=dev)
         _lib.check(lib.diffus_volume_to_bricks(v.data_ptr(), C.byref(dim), out.data_ptr(), _stream(dev)),
                    "diffus_volume_to_bricks")
-        _count(1)
     return out
 
 
@@ -1012,7 +974,6 @@ def to_quads(volume: torch.Tensor) -> torch.Tensor:
         out = torch.empty((lib.diffus_quad_elems(C.byref(dim)) // 4, 4), dtype=torch.float32, device=dev)
         _lib.check(lib.diffus_volume_to_quads(v.data_ptr(), C.byref(dim), out.data_ptr(), _stream(dev)),
                    "diffus_volume_to_quads")
-        _count(1)
     return out
 
 
@@ -1029,7 +990,6 @@ def gaussian_blur_volume(volume: torch.Tensor, sigma: float, truncate: float = 4
         scratch = torch.empty_like(v)
         _lib.check(_lib.load().diffus_volume_gaussian_blur(v.data_ptr(), C.byref(dim), float(sigma), float(truncate), out.data_ptr(),
                                                            scratch.data_ptr(), _stream(dev)), "diffus_volume_gaussian_blur")
-        _count(3 if sigma > 0 else 0)
     return out
 
 
@@ -1041,7 +1001,6 @@ def from_bricks(bricks: torch.Tensor, dims) -> torch.Tensor:
         out = torch.empty(tuple(dims), dtype=torch.float32, device=dev)
         _lib.check(lib.diffus_bricks_to_volume(bricks.data_ptr(), C.byref(dim), out.data_ptr(), _stream(dev)),
                    "diffus_bricks_to_volume")
-        _count(1)
     return out
 
 
@@ -1062,14 +1021,12 @@ def _splat_call(fwd: bool, coords, val, H, W, sigma, grad_out=None):
             _lib.check(lib.diffus_splat_forward(c[0].data_ptr(), c[1].data_ptr(), c[2].data_ptr(), v.data_ptr(), n, H, W,
                                                 float(sigma), out.data_ptr(), ws.data_ptr(), wbytes, _stream(dev)),
                        "diffus_splat_forward")
-            _count(4)
         else:
             g = grad_out.to(torch.float32).contiguous()
             out = torch.empty((n,), dtype=torch.float32, device=dev)
             _lib.check(lib.diffus_splat_backward(c[0].data_ptr(), c[1].data_ptr(), c[2].data_ptr(), v.data_ptr(), n, H, W,
                                                  float(sigma), g.data_ptr(), out.data_ptr(), ws.data_ptr(), wbytes,
                                                  _stream(dev)), "diffus_splat_backward")
-            _count(6)
     return out
 
 
@@ -1125,7 +1082,6 @@ def mlp_fwd_impl(params: torch.Tensor, x: torch.Tensor, mask: Optional[torch.Ten
         if xc.numel():
             _lib.check(lib.diffus_mlp_forward_ex(p.data_ptr(), xc.data_ptr(), _ptr(m), xc.numel(), out_scale, fill,
                                                  out.data_ptr(), _MLP_PATH, _stream(dev)), "diffus_mlp_forward")
-            _count(1)
     return out
 
 
@@ -1161,7 +1117,6 @@ def mlp_bwd_impl(params: torch.Tensor, x: torch.Tensor, mask: Optional[torch.Ten
             _lib.check(lib.diffus_mlp_backward_ex(p.data_ptr(), xc.data_ptr(), _ptr(m), g.data_ptr(), n, out_scale,
                                                   gp.data_ptr(), ws.data_ptr(), wbytes, _MLP_PATH, _stream(dev)),
                        "diffus_mlp_backward")
-            _count(2)
     return gp
 
 
@@ -1193,7 +1148,6 @@ def mlp_input_grad_impl(params: torch.Tensor, x: torch.Tensor, mask: Optional[to
         if xc.numel():
             _lib.check(_lib.load().diffus_mlp_input_grad(p.data_ptr(), xc.data_ptr(), _ptr(m), g.data_ptr(), xc.numel(), out_scale,
                                                          gx.data_ptr(), _stream(dev)), "diffus_mlp_input_grad")
-            _count(1)
     return gx
 
 
@@ -1238,7 +1192,6 @@ def adam_step(params: torch.Tensor, grads: torch.Tensor, state: torch.Tensor, lr
     with _on_device(dev):
         _lib.check(_lib.load().diffus_adam_step(params.data_ptr(), grads.data_ptr(), state.data_ptr(), n, lr, betas[0], betas[1], eps,
                                                 weight_decay, grad_scale, _stream(dev)), "diffus_adam_step")
-        _count(1)
 
 
 class Conv1dRows(torch.autograd.Function):
@@ -1255,7 +1208,6 @@ class Conv1dRows(torch.autograd.Function):
             out = torch.empty((rows, max(n_out, 0)), dtype=torch.float32, device=dev)
             _lib.check(_lib.load().diffus_conv1d_rows_forward(xc.data_ptr(), rows, n_in, wc.data_ptr(), taps, pad, out.data_ptr(),
                                                               _stream(dev)), "diffus_conv1d_rows_forward")
-            _count(1)
         ctx.save_for_backward(wc)
         ctx.meta = (rows, n_in, taps, pad, x.dtype)
         return out.to(x.dtype)
@@ -1271,7 +1223,6 @@ class Conv1dRows(torch.autograd.Function):
             gin = torch.empty((rows, n_in), dtype=torch.float32, device=dev)
             _lib.check(_lib.load().diffus_conv1d_rows_backward(g.data_ptr(), rows, n_in, wc.data_ptr(), taps, pad, gin.data_ptr(),
                                                                _stream(dev)), "diffus_conv1d_rows_backward")
-            _count(1)
         return gin.to(dt), None, None
 
 
@@ -1287,7 +1238,6 @@ def volume_slice(volume: torch.Tensor, dims, layout: int, axis: int, index: int,
             raise _lib.DiffusError(f"slice must be contiguous float32 {tuple(rest)}")
         _lib.check(_lib.load().diffus_volume_slice(volume.data_ptr(), C.byref((C.c_int32 * 3)(*dims)), layout, axis, index,
                                                    slice_.data_ptr(), int(scatter), _stream(dev)), "diffus_volume_slice")
-        _count(1)
     return slice_
 
 
@@ -1323,7 +1273,6 @@ def rotate_apex(x: torch.Tensor, z: torch.Tensor, cos_a: float, sin_a: float, sh
         if xf.numel():
             _lib.check(_lib.load().diffus_rotate_around_apex(xf.data_ptr(), zf.data_ptr(), xf.numel(), cos_a, sin_a, shift, apex0, apex1,
                                                              xr.data_ptr(), zr.data_ptr(), _stream(dev)), "diffus_rotate_around_apex")
-            _count(1)
     return xr, zr
 
 
@@ -1336,7 +1285,6 @@ class LogCompressFunction(torch.autograd.Function):
             out = torch.empty_like(x)
             _lib.check(_lib.load().diffus_log_compress_forward(x.data_ptr(), x.numel(), out.data_ptr(), None, _stream(dev)),
                        "diffus_log_compress_forward")
-            _count(1)
         ctx.save_for_backward(x)
         return out
 
@@ -1349,7 +1297,6 @@ class LogCompressFunction(torch.autograd.Function):
             gx = torch.empty_like(x)
             _lib.check(_lib.load().diffus_log_compress_backward(x.data_ptr(), g.data_ptr(), x.numel(), gx.data_ptr(), _stream(x.device)),
                        "diffus_log_compress_backward")
-            _count(1)
         return gx
 
 
@@ -1363,7 +1310,6 @@ def rf_to_bmode(profiles: torch.Tensor, hilbert_kernel: torch.Tensor) -> torch.T
         ws = torch.empty((4,), dtype=torch.uint8, device=dev)
         _lib.check(_lib.load().diffus_rf_to_bmode(rf.data_ptr(), rf.shape[0], rf.shape[1], hilbert_kernel.contiguous().float().data_ptr(),
                                                   out.data_ptr(), ws.data_ptr(), 4, _stream(dev)), "diffus_rf_to_bmode")
-        _count(3)
     return out
 
 
@@ -1380,7 +1326,6 @@ class MaskedMSEEdgeFunction(torch.autograd.Function):
             stats = torch.empty((3,), dtype=torch.float32, device=dev)
             _lib.check(_lib.load().diffus_masked_mse_edge_forward(a.data_ptr(), b.data_ptr(), m.data_ptr(), H, W, edge_weight,
                                                                   stats.data_ptr(), _stream(dev)), "diffus_masked_mse_edge_forward")
-            _count(1)
         ctx.save_for_backward(a, b, m, stats)
         ctx.edge_weight = edge_weight
         return stats[0].clone()
@@ -1396,7 +1341,6 @@ class MaskedMSEEdgeFunction(torch.autograd.Function):
             _lib.check(_lib.load().diffus_masked_mse_edge_backward(a.data_ptr(), b.data_ptr(), m.data_ptr(), H, W, ctx.edge_weight,
                                                                    stats.data_ptr(), g.data_ptr(), ga.data_ptr(), _stream(a.device)),
                        "diffus_masked_mse_edge_backward")
-            _count(1)
         return ga, None, None, None
 
 
@@ -1417,7 +1361,6 @@ class SSIMLossFunction(torch.autograd.Function):
             loss = torch.empty((1,), dtype=torch.float32, device=dev)
             _lib.check(lib.diffus_ssim_loss_forward(a.data_ptr(), b.data_ptr(), H, W, ksize, sigma, k1, k2, int(normalize), loss.data_ptr(),
                                                     ws.data_ptr(), wbytes, _stream(dev)), "diffus_ssim_loss_forward")
-            _count(3)
         ctx.save_for_backward(a, b, ws)
         ctx.meta = (int(normalize), ksize, sigma)
         return loss.reshape(())
@@ -1434,5 +1377,4 @@ class SSIMLossFunction(torch.autograd.Function):
             _lib.check(_lib.load().diffus_ssim_loss_backward(a.data_ptr(), b.data_ptr(), H, W, ksize, sigma, normalize, g.data_ptr(),
                                                              ga.data_ptr(), ws.data_ptr(), ws.numel(), _stream(a.device)),
                        "diffus_ssim_loss_backward")
-            _count(2)
         return ga, None, None, None, None, None, None

@@ -162,8 +162,7 @@ def recover_poses(volume, targets: torch.Tensor, sources: torch.Tensor, median: 
     step = GraphedFanGaussNewtonStep(volume, targets, n_rays, num_samples, opening_angle, attenuation_coeff, start, probe=probe,
                                      radius=radius, width=width)
     step.reset(sources, median, hint, damping)
-    vol = volume.volume if isinstance(volume, PreparedVolume) else volume
-    history = torch.empty((iterations + 1, step.P), dtype=torch.float32, device=vol.device)
+    history = torch.empty((iterations + 1, step.P), dtype=torch.float32, device=step.loss.device)
     history[0].copy_(step.loss)
     for i in range(iterations):
         step()

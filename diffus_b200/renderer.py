@@ -110,6 +110,21 @@ class PreparedVolume:
         return self._bricks
 
 
+def _unwrap(volume) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+    """``(volume, packed copy or None)`` of a tensor or a :class:`PreparedVolume`, the volume as a contiguous float32 tensor.
+    Not detached: autograd still reaches the caller's tensor."""
+    bricks = None
+    if isinstance(volume, PreparedVolume):
+        bricks, volume = volume.bricks, volume.volume
+    return (volume if volume.dtype == torch.float32 else volume.float()).contiguous(), bricks
+
+
+def _target(target: torch.Tensor) -> torch.Tensor:
+    """Target frames as a contiguous float32 (P,R,S-start) tensor; one (R,S-start) frame is a batch of one."""
+    tgt = target.to(torch.float32).contiguous()
+    return tgt.unsqueeze(0) if tgt.dim() == 2 else tgt
+
+
 def render_frames(volume, sources: torch.Tensor, directions: torch.Tensor, num_samples: int,
                   attenuation_coeff: float = 0.5, start=0, *, sampler: str = "nearest") -> torch.Tensor:
     """Batched ``plot_beam_frame``: (P,3) sources, (P,R,3) or (R,3) directions -> (P,R,S-start) frames.  Float32 sources
@@ -118,25 +133,20 @@ def render_frames(volume, sources: torch.Tensor, directions: torch.Tensor, num_s
     Differentiable w.r.t. ``volume`` and, with ``sampler='trilinear'``, w.r.t. ``sources``
     and ``directions``.  ``volume`` is a (D,H,W) CUDA tensor or a :class:`PreparedVolume`.
     """
-    bricks = None
-    if isinstance(volume, PreparedVolume):
-        bricks, volume = volume.bricks, volume.volume
-    if volume.dim() != 3:
+    vol32, bricks = _unwrap(volume)
+    if vol32.dim() != 3:
         raise ValueError("volume must be (D,H,W)")
-    device = volume.device
     sid = _sampler_id(sampler)
-    src, dirs, product_f32 = _canon_pose(sources, directions, device)
+    src, dirs, product_f32 = _canon_pose(sources, directions, vol32.device)
     if src.dim() == 1:
         src = src.unsqueeze(0)
-    vol32 = volume if volume.dtype == torch.float32 else volume.float()
     start_i = _resolve_start(start, num_samples)
     need_grad = torch.is_grad_enabled() and (vol32.requires_grad or src.requires_grad or dirs.requires_grad)
     if need_grad:
-        return ops.RenderFunction.apply(vol32.contiguous(), bricks, list(volume.shape), src.contiguous(),
-                                        dirs.contiguous(), int(num_samples), int(start_i), float(attenuation_coeff),
-                                        sid, product_f32)
-    frame, _ = ops.render_fwd_impl(vol32.contiguous(), bricks, list(volume.shape), src.contiguous(), dirs.contiguous(),
-                                   int(num_samples), int(start_i), float(attenuation_coeff), sid, product_f32, False)
+        return ops.RenderFunction.apply(vol32, bricks, list(vol32.shape), src.contiguous(), dirs.contiguous(), int(num_samples),
+                                        int(start_i), float(attenuation_coeff), sid, product_f32)
+    frame, _ = ops.render_fwd_impl(vol32, bricks, list(vol32.shape), src.contiguous(), dirs.contiguous(), int(num_samples),
+                                   int(start_i), float(attenuation_coeff), sid, product_f32, False)
     return frame
 
 
@@ -152,20 +162,13 @@ def render_mse_loss(volume, sources: torch.Tensor, directions: torch.Tensor, tar
     the trilinear sampler, ``sources`` / ``directions``), plus the frames if asked.  Per-ray sources (P,R,3) get (P,R,3)
     gradients.
     """
-    bricks = None
-    if isinstance(volume, PreparedVolume):
-        bricks, volume = volume.bricks, volume.volume
-    device = volume.device
+    vol32, bricks = _unwrap(volume)
     sid = _sampler_id(sampler)
-    src, dirs, product_f32 = _canon_pose(sources, directions, device)
+    src, dirs, product_f32 = _canon_pose(sources, directions, vol32.device)
     if src.dim() == 1:
         src = src.unsqueeze(0)
-    vol32 = (volume if volume.dtype == torch.float32 else volume.float()).contiguous()
     start_i = _resolve_start(start, num_samples)
-    tgt = target.to(torch.float32).contiguous()
-    if tgt.dim() == 2:
-        tgt = tgt.unsqueeze(0)
-    loss, frame = ops.RenderMSELoss.apply(vol32, bricks, list(volume.shape), src.contiguous(), dirs.contiguous(), tgt,
+    loss, frame = ops.RenderMSELoss.apply(vol32, bricks, list(vol32.shape), src.contiguous(), dirs.contiguous(), _target(target),
                                           int(num_samples), int(start_i), float(attenuation_coeff), sid, product_f32,
                                           bool(return_frame))
     return (loss, frame) if return_frame else loss
@@ -187,21 +190,16 @@ def render_gauss_newton(volume, sources: torch.Tensor, directions: torch.Tensor,
     """
     if _sampler_id(sampler) != SAMPLER_TRILINEAR:
         raise DiffusError("render_gauss_newton needs sampler='trilinear' (the nearest sampler has no pose derivative)")
-    bricks = None
-    if isinstance(volume, PreparedVolume):
-        bricks, volume = volume.bricks, volume.volume
-    src = torch.as_tensor(sources, device=volume.device)
-    dirs = torch.as_tensor(directions, device=volume.device)
+    vol32, bricks = _unwrap(volume)
+    src = torch.as_tensor(sources, device=vol32.device)
+    dirs = torch.as_tensor(directions, device=vol32.device)
     if src.dtype != torch.float32 or dirs.dtype != torch.float32:
         raise DiffusError("render_gauss_newton takes float32 sources and directions")
     if src.dim() == 1:
         src = src.unsqueeze(0)
-    vol32 = (volume if volume.dtype == torch.float32 else volume.float()).detach().contiguous()
-    tgt = target.detach().to(torch.float32).contiguous()
-    if tgt.dim() == 2:
-        tgt = tgt.unsqueeze(0)
-    return ops.render_gauss_newton_impl(vol32, bricks, list(volume.shape), src.detach().contiguous(), dirs.detach().contiguous(),
-                                        tgt, int(num_samples), _resolve_start(start, num_samples), float(attenuation_coeff))
+    return ops.render_gauss_newton_impl(vol32.detach(), bricks, list(vol32.shape), src.detach().contiguous(), dirs.detach().contiguous(),
+                                        _target(target.detach()), int(num_samples), _resolve_start(start, num_samples),
+                                        float(attenuation_coeff))
 
 
 def render_gauss_newton_sweep(volume, sources: torch.Tensor, directions: torch.Tensor, target: torch.Tensor, num_samples: int,
@@ -218,11 +216,9 @@ def render_gauss_newton_sweep(volume, sources: torch.Tensor, directions: torch.T
     directions are as for :func:`render_gauss_newton` (float32, trilinear sampler).  The outputs are not differentiable: they are
     what :func:`diffus_b200.pose_recovery.register_sweep` consumes.
     """
-    bricks = None
-    if isinstance(volume, PreparedVolume):
-        bricks, volume = volume.bricks, volume.volume
-    src = torch.as_tensor(sources, device=volume.device)
-    dirs = torch.as_tensor(directions, device=volume.device)
+    vol32, bricks = _unwrap(volume)
+    src = torch.as_tensor(sources, device=vol32.device)
+    dirs = torch.as_tensor(directions, device=vol32.device)
     if src.dtype != torch.float32 or dirs.dtype != torch.float32:
         raise DiffusError("render_gauss_newton_sweep takes float32 sources and directions")
     if src.dim() == 1:
@@ -231,16 +227,13 @@ def render_gauss_newton_sweep(volume, sources: torch.Tensor, directions: torch.T
         pivot = torch.as_tensor(pivot)
         if tuple(pivot.shape) != (3,) or pivot.dtype != torch.float64:
             raise DiffusError(f"pivot must be a float64 (3,) tensor, got {pivot.dtype} {tuple(pivot.shape)}")
-        pivot = pivot.to(volume.device).contiguous()
-    vol32 = (volume if volume.dtype == torch.float32 else volume.float()).detach().contiguous()
-    tgt = target.detach().to(torch.float32).contiguous()
-    if tgt.dim() == 2:
-        tgt = tgt.unsqueeze(0)
+        pivot = pivot.to(vol32.device).contiguous()
+    tgt = _target(target.detach())
     start_i = _resolve_start(start, num_samples)
     want = (src.shape[0], dirs.shape[-2], int(num_samples) - start_i)
     if tuple(tgt.shape) != want:
         raise DiffusError(f"target must be {want} (poses, rays, samples after the crop), got {tuple(tgt.shape)}")
-    return ops.render_gauss_newton_sweep_impl(vol32, bricks, list(volume.shape), src.detach().contiguous(),
+    return ops.render_gauss_newton_sweep_impl(vol32.detach(), bricks, list(vol32.shape), src.detach().contiguous(),
                                               dirs.detach().contiguous(), tgt, int(num_samples), start_i,
                                               float(attenuation_coeff), pivot)
 
@@ -294,18 +287,14 @@ class UltrasoundRenderer:
         the (R, num_samples) impedances.  ``start`` is accepted for signature parity; as in
         the reference it only affected the debug plot.
         """
-        if isinstance(volume, PreparedVolume):
-            bricks, vol = volume.bricks, volume.volume
-        else:
-            bricks, vol = None, volume
+        vol32, bricks = _unwrap(volume)
         if directions.ndim == 1:
             directions = directions.unsqueeze(0)
-        src, dirs, product_f32 = _canon_pose(source, directions, vol.device)
+        src, dirs, product_f32 = _canon_pose(source, directions, vol32.device)
         src = src.reshape(1, 3).contiguous()
         dirs = dirs.contiguous()
-        dims = list(vol.shape)
+        dims = list(vol32.shape)
         x, y, z = ops.ray_indices(dims, src, dirs, int(num_samples), 0, product_f32)
-        vol32 = (vol if vol.dtype == torch.float32 else vol.float()).contiguous()
         if torch.is_grad_enabled() and (vol32.requires_grad or src.requires_grad or dirs.requires_grad):
             values = ops.TraceValuesFunction.apply(vol32, bricks, dims, src, dirs, int(num_samples), _sampler_id(sampler),
                                                    product_f32)

@@ -23,7 +23,6 @@ def create_brain_mask(volume: torch.Tensor, threshold=50, iterations: int = 2) -
         scratch = torch.empty(v.shape, dtype=torch.uint8, device=dev)
         _lib.check(lib.diffus_brain_mask(v.data_ptr(), C.byref(dim), float(threshold), int(iterations), mask.data_ptr(),
                                          scratch.data_ptr(), ops._stream(dev)), "diffus_brain_mask")
-        ops._count(1 + 2 * int(iterations))
     return mask.bool()
 
 
@@ -38,5 +37,4 @@ def zscore_normalize(volume: torch.Tensor, mask: torch.Tensor) -> torch.Tensor:
         ws = torch.empty((64,), dtype=torch.uint8, device=dev)
         _lib.check(lib.diffus_masked_zscore(v.data_ptr(), m.data_ptr(), v.numel(), out.data_ptr(), ws.data_ptr(), 64,
                                             ops._stream(dev)), "diffus_masked_zscore")
-        ops._count(2)
     return out

@@ -132,6 +132,8 @@ typedef struct DiffusRenderBwdArgs {
 
 int32_t diffus_abi_version(void);
 const char* diffus_error_string(int32_t code);
+/* Number of kernels this process has enqueued through the library so far (memsets and copies are not kernels). */
+int64_t diffus_launch_count(void);
 
 int64_t diffus_render_workspace_bytes(const DiffusRenderArgs* args);
 int32_t diffus_render_forward(const DiffusRenderArgs* args, void* stream);
